@@ -12,6 +12,7 @@ collective (weak scaling: 64 utterances per GPU; `--scaling strong` splits a fix
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the oracle (CPU port; the reference ships no code) on host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed inference's outputs to DIR/*.npy (seeded inputs)
 
 Prints ONE JSON line (rank 0).  `value` = device-resident throughput (inputs already in HBM, CUDA-event
 timed); `e2e` = the same through TransformerTTS.inference with HOST tensors (results land in the module's pinned
@@ -69,6 +70,26 @@ def synthetic_inputs(B: int, S: int, seed: int):
     g = torch.Generator().manual_seed(seed)
     ph = torch.randint(1, 128, (B, S), generator=g, dtype=torch.int64)
     return ph, torch.full((B,), S, dtype=torch.int32)
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir: str, utt0: int, mel_after, mel_lens, stop_logits):
+    """Writes what one inference() call returned as float32 DIR/<name>.npy, so that two builds can be compared output for
+    output.  Above DUMP_BYTES in all, a fixed seeded sample of utterances is written and their ids go to utterance_ids.npy."""
+    import numpy as np
+    B = mel_after.shape[0]
+    per_utt = 4 * (mel_after[0].numel() + 1 + stop_logits[0].numel())
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES - 4096                                         # the .npy headers
+    rows = torch.arange(B)
+    if B * per_utt > budget:
+        keep = budget // (per_utt + 8)                                 # 8 bytes per utterance id
+        rows = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        np.save(os.path.join(out_dir, "utterance_ids.npy"), (rows + utt0).numpy().astype(np.float64))
+    for name, t in (("mel_after", mel_after), ("mel_lens", mel_lens), ("stop_logits", stop_logits)):
+        np.save(os.path.join(out_dir, name + ".npy"), t[rows.to(t.device)].float().cpu().numpy())
 
 
 class ClockSampler:
@@ -262,6 +283,8 @@ def run_b200(args, rank, world, local_rank):
     dec_ms = max_over_ranks(statistics.mean(model.decode_ms))
     frames_total = world * B * T * args.steps
     value = frames_total / (dev_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, utt0, *out)
 
     # ---- end to end through the public API with HOST tensors -----------------------------------
     model.profile_events = False
@@ -465,7 +488,13 @@ def main():
     ap.add_argument("--train-batch", type=int, default=32)
     ap.add_argument("--no-extra", action="store_true", help="skip the strong-scaling / batch-1 latency / long-utterance lines")
     ap.add_argument("--nccl-timeout", type=int, default=180, help="seconds before a collective gives up (a dead rank must not stall the job)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed inference returned on "
+                    "rank 0 (mel_after, mel_lens, stop_logits) to DIR/<name>.npy as float32, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

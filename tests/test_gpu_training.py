@@ -9,7 +9,7 @@ import torch
 
 from tests.gpu_util import make_b200_model, rel_l2
 
-pytestmark = pytest.mark.gpu
+pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not torch.cuda.is_available(), reason="no GPU")]
 
 TOL_OUT = 2e-2        # rel-L2 of train-mode forward outputs
 TOL_LOSS = 5e-3       # relative error of the scalar loss

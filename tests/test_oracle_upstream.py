@@ -1,15 +1,36 @@
-"""T1: pin the oracle's sub-modules against the independent upstream implementations in the image
-(SURVEY.md 8(c)): torch.nn.Transformer{Encoder,Decoder}Layer [TT] and torchaudio Tacotron2 [TA].
+"""T1: pin the oracle's sub-modules against independent upstream implementations (SURVEY.md 8(c)):
+torch.nn.Transformer{Encoder,Decoder}Layer [TT], run live, and torchaudio Tacotron2 [TA], whose outputs on the canonical
+weights and the seeded inputs below are stored in tests/golden/upstream_torchaudio.npz (tests/golden/make_upstream_golden.py
+regenerates them), so the comparison runs without torchaudio.
 The reference repository has no tests or vectors of its own ("parity unpinned" at that boundary)."""
+import os
+
 import numpy as np
-import pytest
 import torch
 import torch.nn as nn
 
 from oracle import synthetic
 from oracle.transformer_tts import masked_batchnorm, length_mask, sinusoid_table
 
-ta = pytest.importorskip("torchaudio.models.tacotron2")
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def postnet_input():
+    return torch.randn(2, 23, 80, generator=torch.Generator().manual_seed(3))
+
+
+def encoder_convs_input():
+    return torch.randn(2, 512, 19, generator=torch.Generator().manual_seed(4))
+
+
+def prenet_input():
+    return torch.randn(4, 80, generator=torch.Generator().manual_seed(6))
+
+
+def _torchaudio_outputs(oracle_model):
+    g = np.load(os.path.join(GOLD, "upstream_torchaudio.npz"))
+    assert str(g["digest"]) == synthetic.state_dict_digest(oracle_model.state_dict())    # stored for these weights
+    return g
 
 
 def _copy_mha(dst: nn.MultiheadAttention, src):
@@ -68,32 +89,23 @@ def test_decoder_layer_matches_torch(oracle_model):
 
 
 def test_postnet_matches_torchaudio_eval(oracle_model):
-    ref = ta._Postnet(80, 512, 5, 5).eval()
-    for i, cb in enumerate(oracle_model.postnet.convs):
-        ref.convolutions[i][0].load_state_dict(cb.conv.state_dict())
-        ref.convolutions[i][1].load_state_dict(cb.bn.state_dict())
-    x = torch.randn(2, 23, 80, generator=torch.Generator().manual_seed(3))
+    x = postnet_input()
     lens = torch.tensor([23, 23])                      # [TA] has no per-layer masking; full lengths
     with torch.no_grad():
         got = oracle_model._postnet(x, lens, 0, np.arange(2))
-        want = ref(x.transpose(1, 2)).transpose(1, 2)
+    want = torch.from_numpy(_torchaudio_outputs(oracle_model)["postnet"])     # [TA] _Postnet(80, 512, 5, 5), eval
     assert torch.allclose(got, want, atol=2e-5, rtol=1e-5)
 
 
 def test_encoder_convs_match_torchaudio_eval(oracle_model):
-    ref = ta._Encoder(512, 3, 5).eval()
-    for i, cb in enumerate(oracle_model.enc_prenet.convs):
-        ref.convolutions[i][0].load_state_dict(cb.conv.state_dict())
-        ref.convolutions[i][1].load_state_dict(cb.bn.state_dict())
-    x = torch.randn(2, 512, 19, generator=torch.Generator().manual_seed(4))
+    x = encoder_convs_input()
     m = torch.ones(2, 1, 19)
     with torch.no_grad():
         got = x
         for cb in oracle_model.enc_prenet.convs:
             got = torch.relu(masked_batchnorm(cb.bn, cb.conv(got), m, False)) * m
-        want = x
-        for conv in ref.convolutions:                  # [TA]:407-408 (eval: dropout is identity)
-            want = torch.relu(conv(want))
+    # [TA] _Encoder(512, 3, 5).convolutions, each followed by ReLU ([TA]:407-408; eval: dropout is identity)
+    want = torch.from_numpy(_torchaudio_outputs(oracle_model)["encoder_convs"])
     assert torch.allclose(got, want, atol=2e-5, rtol=1e-5)
 
 
@@ -110,15 +122,10 @@ def test_masked_batchnorm_training_matches_torch_on_full_lengths():
 def test_prenet_matches_torchaudio_structure(oracle_model):
     """[TA] _Prenet: relu(linear) then dropout p=0.5 with training=True even in eval (line 284).
     [TA] has bias=False; with our biases zeroed and masks forced to keep-all the maths coincide."""
-    ref = ta._Prenet(80, [256, 256]).eval()
     p = oracle_model.dec_prenet
+    x = prenet_input()
+    out = torch.from_numpy(_torchaudio_outputs(oracle_model)["prenet"])   # [TA] _Prenet with fc1 / fc2 weights, torch.manual_seed(0)
     with torch.no_grad():
-        ref.layers[0].weight.copy_(p.fc1.weight)
-        ref.layers[1].weight.copy_(p.fc2.weight)
-    x = torch.randn(4, 80, generator=torch.Generator().manual_seed(6))
-    with torch.no_grad():
-        torch.manual_seed(0)
-        out = ref(x)
         h1 = torch.relu(x @ p.fc1.weight.T)
     # dropout was applied in eval mode: about half of the positive activations are zeroed
     torch.manual_seed(0)
