@@ -218,6 +218,46 @@ int tts_k_layernorm(const float* X, const float* gamma, const float* beta, void*
 /* Keep-bits of a p = 0.5 dropout site: out[t][b][c] (uint8) for t < T, b < B, c < C. */
 int tts_k_philox_bits(uint64_t seed, int site, int T, int B, int C, int utt_offset, uint8_t* out, void* stream);
 
+/* Training-step kernels (tests/test_gpu_train_kernels.py), launched exactly as tts_train_step launches them.  Rows are
+ * m = b * T + t, valid iff t < lens[b]; `seed` is a DEVICE pointer to the uint64 dropout seed; site < 0 disables dropout.
+ * Weight gradient (tcgen05): dW[n][k * taps + tap] += sum_{b,t} dY[b*T+t][n] X[b*T+t+tap-taps/2][k] (zero outside each
+ * utterance), dbias[n] += sum dY[.][n] when dbias is not null.  dY [nb*T][ldy], X [nb*T][ldx] bf16; taps 1 or 5. */
+int tts_k_wgrad(const void* dY_bf16, int ldy, int Cout, const void* X_bf16, int ldx, int Cin, int taps, int T, int nb,
+                float* dW, float* dbias, void* stream);
+/* Input gradient: packs the fp32 weight W [N][K][taps] (torch layout) into the transposed, tap-reversed bf16 layout
+ * [taps][round_up(K,128)][round_up(N,64)] in `scratch`, then out[m][k] = sum_tap sum_{n < Kdy} dY[m+taps/2-tap][n] W[n][k][tap]
+ * (conv1d input gradient; columns n >= N of dY meet zero weights).  Exactly one of out_f32 / out_bf16 (row stride ldo). */
+int tts_k_dgrad(const float* W, int N, int K, int taps, const void* dY_bf16, int ldy, int Kdy, int M, int T,
+                float* out_f32, void* out_bf16, int ldo, void* scratch_bf16, void* stream);
+/* Masked batch-statistics BatchNorm forward over x [B*T][C] fp32 (C % 4 == 0, C <= 512): stat [1024] <- (sums, centred
+ * squares) over valid rows; y = mask * dropout_0.5(act(BN(x))) (act 0 none / 1 relu / 2 tanh) -> out16 (bf16, row
+ * stride ldo) and / or out32 (fp32, stride C); running stats updated (momentum 0.1, unbiased) if run_mean / run_var given. */
+int tts_k_bn_train_fwd(const float* x, int B, int T, int C, const int32_t* lens, float* stat, const float* gamma,
+                       const float* beta, float eps, int act, int site, const uint64_t* seed, int utt_offset, void* out16,
+                       int ldo, float* out32, float* run_mean, float* run_var, void* stream);
+/* Its backward from dout (fp32, or bf16 if dout_bf16; row stride ldd): dgamma / dbeta (zero on entry) get the parameter
+ * gradients, dx (bf16, row stride ldx) the input gradient, zero on padded rows. */
+int tts_k_bn_train_bwd(const void* dout, int dout_bf16, int ldd, const float* x, int B, int T, int C, const int32_t* lens,
+                       const float* stat, const float* gamma, const float* beta, float eps, int act, int site,
+                       const uint64_t* seed, int utt_offset, float* dgamma, float* dbeta, void* dx_bf16, int ldx, void* stream);
+/* LayerNorm(512) backward from dx [M][512] at pre-norm input ypre: dy32 (fp32), dsub16 = bf16(dy * keep * dscale) with the
+ * word-dropout site's keep mask (keep iff word >= thresh; site < 0: plain copy); dgamma / dbeta += their sums. */
+int tts_k_ln_bwd(const float* dx, const float* ypre, const float* gamma, float eps, int M, int T, float* dy32, void* dsub16_bf16,
+                 int site, const uint64_t* seed, int utt_offset, uint32_t thresh, float dscale, float* dgamma, float* dbeta,
+                 void* stream);
+/* Loss P13 over [B][T][80] / [B][T]: loss[0], and its gradients wrt mel_before, mel_after, stop_logits; acc: 16 floats scratch. */
+int tts_k_loss(const float* before, const float* after, const float* stop, const float* target, const int32_t* lens, int B,
+               int T, float pos_weight, float* acc, float* dbefore, float* dafter, float* dstop, float* loss, void* stream);
+/* Head gradient dhead [B*T][128] bf16: [0, 80) = mask * (dbefore + dafter + dpost0), [80] = mask * dstop, rest 0. */
+int tts_k_head_grad(const float* dbefore, const float* dafter, const void* dpost0_bf16, int ldp, const float* dstop,
+                    const int32_t* lens, int B, int T, void* dhead_bf16, void* stream);
+/* Word-dropout backward of d [B*T][512] -> out (bf16) = d * keep * dscale, dalpha += sum out_fp32 * pe[t] (pe [T][512]);
+ * decoder != 0 uses the decoder's launch (1184 blocks), 0 the encoder's (592). */
+int tts_k_dropw_bwd(const float* d, void* out_bf16, int B, int T, int site, const uint64_t* seed, int utt_offset,
+                    uint32_t thresh, float dscale, const float* pe, float* dalpha, int decoder, void* stream);
+/* Embedding backward: dE[ph[m]][c] += d[m][c] over valid rows with 0 < ph[m] < V; d [B*S][512] bf16, dE [V][512]. */
+int tts_k_embed_bwd(const void* d_bf16, const int64_t* ph, const int32_t* lens, int B, int S, int V, float* dE, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

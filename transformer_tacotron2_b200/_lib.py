@@ -69,6 +69,15 @@ SIGNATURES = {
     "tts_k_attention_bwd": (_I, [_P] * 11 + [_I, _I, _I, _I, _I, _P]),
     "tts_k_layernorm": (_I, [_P, _P, _P, _P, _I, C.c_float, _P]),
     "tts_k_philox_bits": (_I, [_U64, _I, _I, _I, _I, _I, _P, _P]),
+    "tts_k_wgrad": (_I, [_P, _I, _I, _P, _I, _I, _I, _I, _I, _P, _P, _P]),
+    "tts_k_dgrad": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _I, _P, _P, _I, _P, _P]),
+    "tts_k_bn_train_fwd": (_I, [_P, _I, _I, _I, _P, _P, _P, _P, C.c_float, _I, _I, _P, _I, _P, _I, _P, _P, _P, _P]),
+    "tts_k_bn_train_bwd": (_I, [_P, _I, _I, _P, _I, _I, _I, _P, _P, _P, _P, C.c_float, _I, _I, _P, _I, _P, _P, _P, _I, _P]),
+    "tts_k_ln_bwd": (_I, [_P, _P, _P, C.c_float, _I, _I, _P, _P, _I, _P, _I, C.c_uint32, C.c_float, _P, _P, _P]),
+    "tts_k_loss": (_I, [_P, _P, _P, _P, _P, _I, _I, C.c_float, _P, _P, _P, _P, _P, _P]),
+    "tts_k_head_grad": (_I, [_P, _P, _P, _I, _P, _P, _I, _I, _P, _P]),
+    "tts_k_dropw_bwd": (_I, [_P, _P, _I, _I, _I, _P, _I, C.c_uint32, C.c_float, _P, _P, _I, _P]),
+    "tts_k_embed_bwd": (_I, [_P, _P, _P, _I, _I, _I, _P, _P]),
 }
 
 _lib = None

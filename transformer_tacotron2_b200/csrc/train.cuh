@@ -20,6 +20,28 @@ struct TrEnc { TrLin qkv, wo, w1, w2; size_t ln1g, ln1b, ln2g, ln2b; };
 struct TrDec { TrLin qkv, wo, q2, wo2, w1, w2; size_t ln1g, ln1b, ln2g, ln2b, ln3g, ln3b; };
 struct TrEntry { std::string name; size_t off, numel; };
 
+// padded shapes of the two bf16 operand copies of an [N][K][taps] fp32 matrix: forward [taps][Nw][Kp], input gradient [taps][Kw][Np]
+TrMat tr_mat_dims(int N, int K, int taps) {
+    TrMat m; memset(&m, 0, sizeof(m));
+    m.N = N; m.K = K; m.taps = taps;
+    m.Nw = round_up(N, 128); m.Kp = round_up(K, 32); m.Kw = round_up(K, 128); m.Np = round_up(N, 64);
+    return m;
+}
+// cast_pack_all_kernel descriptor of one copy (flip = 1: the transposed, tap-reversed input-gradient layout); *blocks = its grid share
+PackDesc tr_pack_desc(const TrMat& m, int flip, long src_off, long dst_off, int blk0, int* blocks) {
+    PackDesc d; memset(&d, 0, sizeof(d));
+    d.src_off = src_off; d.dst_off = dst_off; d.N = m.N; d.K = m.K; d.taps = m.taps;
+    d.R = flip ? m.Kw : m.Nw; d.Cc = flip ? m.Np : m.Kp; d.flip = flip; d.blk0 = blk0;
+    *blocks = (int)(((long)d.taps * d.R * d.Cc + 2047) / 2048);
+    return d;
+}
+// input-gradient GEMM dX[M][K] = sum_tap dY[m + tap - pad][:Kdy] . Wbwd[tap] over the packed layout [taps][Kw][Np] of m
+GemmParams tr_dgrad_params(const TrMat& m, const bf16* wbwd, const bf16* dY, int ldy, int Kdy, int M, int Trows) {
+    GemmParams p = gp(dY, ldy, wbwd, m.Np, M, m.K, Kdy);
+    p.Nw = m.Kw; p.taps = m.taps; p.T = Trows; p.B = M / Trows;
+    return p;
+}
+
 }  // namespace
 
 struct TtsTrain {
@@ -136,8 +158,7 @@ int train_build(TtsHandle* h) {
     auto pad4 = [&]() { t->n = (t->n + 3) / 4 * 4; };
     auto addbuf = [&](const std::string& name, size_t numel) { size_t off = t->nrs; t->buffers.push_back({name, off, numel}); t->nrs += numel; return off; };
     auto mat = [&](size_t off, int N, int K, int taps) {
-        TrMat m; m.off = off; m.N = N; m.K = K; m.taps = taps;
-        m.Nw = round_up(N, 128); m.Kp = round_up(K, 32); m.Kw = round_up(K, 128); m.Np = round_up(N, 64);
+        TrMat m = tr_mat_dims(N, K, taps); m.off = off;
         m.fwd_off = t->wpack_elems; t->wpack_elems += (size_t)taps * m.Nw * m.Kp;
         m.bwd_off = t->wpack_elems; t->wpack_elems += (size_t)taps * m.Kw * m.Np;
         m.fwd = m.bwd = nullptr;
@@ -226,11 +247,9 @@ int train_build(TtsHandle* h) {
     for (auto& m : t->mats) {
         m.fwd = t->wpack + m.fwd_off; m.bwd = t->wpack + m.bwd_off;
         for (int flip = 0; flip < 2; ++flip) {
-            PackDesc d; memset(&d, 0, sizeof(d));
-            d.src_off = (long)m.off; d.dst_off = (long)(flip ? m.bwd_off : m.fwd_off); d.N = m.N; d.K = m.K; d.taps = m.taps;
-            d.R = flip ? m.Kw : m.Nw; d.Cc = flip ? m.Np : m.Kp; d.flip = flip; d.blk0 = blk;
-            blk += (int)(((long)d.taps * d.R * d.Cc + 2047) / 2048);
-            descs.push_back(d);
+            int nblk = 0;
+            descs.push_back(tr_pack_desc(m, flip, (long)m.off, (long)(flip ? m.bwd_off : m.fwd_off), blk, &nblk));
+            blk += nblk;
         }
     }
     t->n_pack = (int)descs.size(); t->pack_blocks = blk;
@@ -271,9 +290,7 @@ void tr_dropw(TrCtx& c, GemmParams& p, int site) {
 // input-gradient GEMM: dX[M][K] = dY[M][N] . W[N][K]
 GemmParams tr_dgrad(TrCtx& c, const bf16* dY, int ldy, int Kdy, int M, int Trows, int mat) {
     const TrMat& m = c.t->mats[mat];
-    GemmParams p = gp(dY, ldy, m.bwd, m.Np, M, m.K, Kdy);
-    p.Nw = m.Kw; p.taps = m.taps; p.T = Trows; p.B = M / Trows;
-    return p;
+    return tr_dgrad_params(m, m.bwd, dY, ldy, Kdy, M, Trows);
 }
 // weight gradient dW[N][K * taps] += sum_m dY[m][n] X[m + tap - pad][k] (+ bias gradient), accumulated into G (wgrad_tc.cuh)
 int tr_wgrad(TrCtx& c, const bf16* dY, int ldy, const bf16* X, int ldx, int M, int Trows, int mat, size_t bias_off, bool has_bias = true) {
@@ -286,10 +303,8 @@ int tr_wgrad(TrCtx& c, const bf16* dY, int ldy, const bf16* X, int ldx, int M, i
     return 0;
 }
 int tr_ln_bwd(TrCtx& c, const float* dx, const float* ypre, size_t g_off, size_t b_off, int M, int Trows, int site, float* dy32, bf16* dsub) {
-    ln_bwd_kernel<<<std::min((M + 7) / 8, 592), 256, 0, c.st>>>(dx, ypre, c.P + g_off, c.h->cfg.ln_eps, M, Trows, dy32, dsub, c.thresh ? site : -1, c.seed,
-                                                                 c.utt0, c.thresh, c.dscale, c.G + g_off, c.G + b_off);
-    ++launch_counter();
-    TRL(cudaGetLastError());
+    TRL(launch_ln_bwd(dx, ypre, c.P + g_off, c.h->cfg.ln_eps, M, Trows, dy32, dsub, c.thresh ? site : -1, c.seed, c.utt0, c.thresh, c.dscale,
+                      c.G + g_off, c.G + b_off, c.st));
     return 0;
 }
 AttnBwdParams tr_abwd(const AttnParams& f, const bf16* dO, const float* lse, const float* dsum, float* dQ, bf16* dK, int lddk, bf16* dV, int lddv) {
@@ -332,15 +347,8 @@ int tr_conv_fwd(TrCtx& c, const TrConv& cv, const bf16* in, int ldin, int M, int
     GemmParams p = gp(in, ldin, m.fwd, m.Kp, M, m.N, m.Kp);
     p.taps = 5; p.T = Trows; p.B = M / Trows; p.bias = c.P + cv.b; p.out_f32 = pre; p.ldo = m.N;
     TRL(launch_gemm_tc(p, c.st));
-    TRL(cudaMemsetAsync(stat, 0, 1024 * 4, c.st));
-    const dim3 g((m.N + 127) / 128, 592);
-    bn_stats_kernel<<<g, 128, 0, c.st>>>(pre, M, m.N, Trows, c.B, lens, stat, 0);
-    bn_stats_kernel<<<g, 128, 0, c.st>>>(pre, M, m.N, Trows, c.B, lens, stat, 1);
-    const int bn_threads = (m.N / 4) * std::max(1, 256 / (m.N / 4));      // (C / 4) channel groups x row lanes
-    bn_act_fwd_kernel<<<1184, bn_threads, 0, c.st>>>(pre, M, m.N, Trows, c.B, lens, stat, c.P + cv.g, c.P + cv.be, c.h->cfg.bn_eps, act,
-                                                                                          site, c.seed, c.utt0, out16, ldo, out32, c.t->RS + cv.rm, c.t->RS + cv.rv, 0.1f);
-    launch_counter() += 3;
-    TRL(cudaGetLastError());
+    TRL(launch_bn_train_fwd(pre, M, m.N, Trows, c.B, lens, stat, c.P + cv.g, c.P + cv.be, c.h->cfg.bn_eps, act, site, c.seed, c.utt0, out16, ldo,
+                            out32, c.t->RS + cv.rm, c.t->RS + cv.rv, c.st));
     return 0;
 }
 // backward of the same block: dout (grad wrt the block output) -> dpre (bf16 [M][N]), parameter gradients, input gradient din16
@@ -348,14 +356,8 @@ template <typename TD>
 int tr_conv_bwd(TrCtx& c, const TrConv& cv, const TD* dout, int ldd, const float* pre, const float* stat, const bf16* in, int ldin, int M, int Trows,
                 const int* lens, int act, int site, bf16* dpre, bf16* din16, int ldi) {
     const TrMat& m = c.t->mats[cv.mat];
-    const dim3 g((m.N + 127) / 128, 592);
-    bn_bwd_reduce_kernel<TD><<<g, 128, 0, c.st>>>(dout, ldd, pre, M, m.N, Trows, c.B, lens, stat, c.P + cv.g, c.P + cv.be, c.h->cfg.bn_eps, act, site, c.seed,
-                                                  c.utt0, c.G + cv.be, c.G + cv.g);
-    const int bn_threads = (m.N / 4) * std::max(1, 256 / (m.N / 4));
-    bn_bwd_apply_kernel<TD><<<1184, bn_threads, 0, c.st>>>(dout, ldd, pre, M, m.N, Trows, c.B, lens, stat, c.P + cv.g, c.P + cv.be,
-                                                                                                 c.h->cfg.bn_eps, act, site, c.seed, c.utt0, c.G + cv.be, c.G + cv.g, dpre, m.N);
-    launch_counter() += 2;
-    TRL(cudaGetLastError());
+    TRL(launch_bn_train_bwd<TD>(dout, ldd, pre, M, m.N, Trows, c.B, lens, stat, c.P + cv.g, c.P + cv.be, c.h->cfg.bn_eps, act, site, c.seed, c.utt0,
+                                c.G + cv.be, c.G + cv.g, dpre, m.N, c.st));
     int r = tr_wgrad(c, dpre, m.N, in, ldin, M, Trows, cv.mat, cv.b);
     if (r) return r;
     if (din16) {
@@ -468,12 +470,8 @@ int train_loss(TrCtx& c, float* loss_out, float pos_weight) {
     const int64_t* ph = w.ph_in; const float* mels = w.mels_in;
     (void)h; (void)t; (void)S; (void)Me; (void)eps; (void)plens; (void)ph;
     // ================================================================ loss (P13) and its gradient
-    TRL(cudaMemsetAsync(w.acc, 0, 64, st));
-    loss_kernel<<<std::min<long>(((long)Md * 81 + 255) / 256, 2368), 256, 0, st>>>(w.mel_before, w.mel_after, w.stop, mels, mlens, B, T, pos_weight, w.acc, w.dbefore,
-                                                                                  w.dafter, w.dstop);
-    loss_finalize_kernel<<<1, 32, 0, st>>>(w.acc, mlens, B, loss_out);
-    launch_counter() += 2;
-    TRL(cudaGetLastError());
+    (void)Md;
+    TRL(launch_loss(w.mel_before, w.mel_after, w.stop, mels, mlens, B, T, pos_weight, w.acc, w.dbefore, w.dafter, w.dstop, loss_out, st));
 
     return 0;
 }
@@ -499,8 +497,7 @@ int train_backward(TrCtx& c) {
             std::swap(din, tmp);
         }
         // din now holds d(postnet input) as bf16 [Md][96]
-        head_grad_kernel<<<(unsigned)(((long)Md * 128 + 255) / 256), 256, 0, st>>>(w.dbefore, w.dafter, din, 96, w.dstop, mlens, Md, T, w.dhead);
-        ++launch_counter();
+        TRL(launch_head_grad(w.dbefore, w.dafter, din, 96, w.dstop, mlens, Md, T, w.dhead, st));
     }
     {   // heads
         int r = tr_wgrad(c, w.dhead, 128, w.xd[6], 512, Md, T, t->head.mat, t->head.b);
@@ -545,8 +542,7 @@ int train_backward(TrCtx& c) {
         TRL(launch_gemm_tc(p, st));
     }
     {   // decoder prenet
-        dropw_bwd_kernel<<<1184, 256, 0, st>>>(w.dx, w.dsub, Md, T, c.thresh ? (int)SITE_DEC_PE : -1, c.seed, c.utt0, c.thresh, c.dscale, h->pe, c.G + t->dec_alpha);
-        ++launch_counter();
+        TRL(launch_dropw_bwd(true, w.dx, w.dsub, Md, T, c.thresh ? (int)SITE_DEC_PE : -1, c.seed, c.utt0, c.thresh, c.dscale, h->pe, c.G + t->dec_alpha, st));
         int r;
         if ((r = tr_wgrad(c, w.dsub, 512, w.h2, 256, Md, T, t->dproj.mat, t->dproj.b))) return r;
         GemmParams p = tr_dgrad(c, w.dsub, 512, 512, Md, T, t->dproj.mat); p.out_bf16 = w.dctx; p.ldo = 256;
@@ -589,8 +585,7 @@ int train_backward(TrCtx& c) {
         TRL(launch_gemm_tc(p, st));
     }
     {   // encoder prenet
-        dropw_bwd_kernel<<<592, 256, 0, st>>>(w.dx, w.dsub, Me, S, c.thresh ? (int)SITE_ENC_PE : -1, c.seed, c.utt0, c.thresh, c.dscale, h->pe, c.G + t->enc_alpha);
-        ++launch_counter();
+        TRL(launch_dropw_bwd(false, w.dx, w.dsub, Me, S, c.thresh ? (int)SITE_ENC_PE : -1, c.seed, c.utt0, c.thresh, c.dscale, h->pe, c.G + t->enc_alpha, st));
         int r;
         if ((r = tr_wgrad(c, w.dsub, 512, w.e[3], 512, Me, S, t->enc_proj.mat, t->enc_proj.b))) return r;
         GemmParams p = tr_dgrad(c, w.dsub, 512, 512, Me, S, t->enc_proj.mat); p.out_bf16 = w.dctx; p.ldo = 512;
@@ -601,8 +596,7 @@ int train_backward(TrCtx& c) {
             if (r) return r;
             std::swap(din, tmp);
         }
-        embed_bwd_kernel<<<(unsigned)(((long)Me * 512 + 255) / 256), 256, 0, st>>>(din, ph, plens, Me, S, h->cfg.n_vocab, c.G + t->mats[t->embed].off);
-        ++launch_counter();
+        TRL(launch_embed_bwd(din, ph, plens, Me, S, h->cfg.n_vocab, c.G + t->mats[t->embed].off, st));
     }
     TRL(cudaGetLastError());
     return 0;

@@ -371,6 +371,80 @@ __global__ void head_grad_kernel(const float* __restrict__ dbefore32, const floa
     dhead16[i] = __float2bfloat16(v);
 }
 
+// ---------------------------------------------------------------------------------------------- launches
+// Launch geometry of the kernels above, shared by the training step (train.cuh) and the per-kernel test entry points, so
+// that the tests check the launches training runs.
+// Masked BatchNorm: the statistics / reduce kernels run one thread per channel over BN_ROW_CHUNKS row chunks, the
+// element-wise kernels (C / 4) channel groups x row lanes per block over BN_ELEM_BLOCKS blocks (grid-stride over rows).
+constexpr int BN_ROW_CHUNKS = 592, BN_ELEM_BLOCKS = 1184;
+constexpr int BN_STAT_FLOATS = 1024;             // stat buffer of one BN layer: [0, C) sums, [C, 2C) centred squares (C <= 512)
+inline int bn_threads(int C) { return (C / 4) * std::max(1, 256 / (C / 4)); }
+
+// stat <- batch statistics over the valid rows of x [B * T][C]; y = mask * dropout(act(BN(x))) -> out16 (row stride ldo) and / or
+// out32 (row stride C); running statistics updated with momentum 0.1 (unbiased variance) when run_mean is given
+inline cudaError_t launch_bn_train_fwd(const float* x, int M, int C, int T, int B, const int* lens, float* stat, const float* gamma,
+                                       const float* beta, float eps, int act, int site, const uint64_t* seedp, int utt_offset, bf16* out16,
+                                       int ldo, float* out32, float* run_mean, float* run_var, cudaStream_t st) {
+    cudaError_t e = cudaMemsetAsync(stat, 0, BN_STAT_FLOATS * 4, st);
+    if (e != cudaSuccess) return e;
+    const dim3 g((C + 127) / 128, BN_ROW_CHUNKS);
+    bn_stats_kernel<<<g, 128, 0, st>>>(x, M, C, T, B, lens, stat, 0);
+    bn_stats_kernel<<<g, 128, 0, st>>>(x, M, C, T, B, lens, stat, 1);
+    bn_act_fwd_kernel<<<BN_ELEM_BLOCKS, bn_threads(C), 0, st>>>(x, M, C, T, B, lens, stat, gamma, beta, eps, act, site, seedp, utt_offset, out16, ldo,
+                                                               out32, run_mean, run_var, 0.1f);
+    launch_counter() += 3;
+    return cudaGetLastError();
+}
+// backward of the same block from dout (row stride ldd): dbeta / dgamma (zero on entry) += their sums, dx (bf16, row stride ldx)
+template <typename TD>
+inline cudaError_t launch_bn_train_bwd(const TD* dout, int ldd, const float* x, int M, int C, int T, int B, const int* lens, const float* stat,
+                                       const float* gamma, const float* beta, float eps, int act, int site, const uint64_t* seedp, int utt_offset,
+                                       float* dbeta, float* dgamma, bf16* dx, int ldx, cudaStream_t st) {
+    const dim3 g((C + 127) / 128, BN_ROW_CHUNKS);
+    bn_bwd_reduce_kernel<TD><<<g, 128, 0, st>>>(dout, ldd, x, M, C, T, B, lens, stat, gamma, beta, eps, act, site, seedp, utt_offset, dbeta, dgamma);
+    bn_bwd_apply_kernel<TD><<<BN_ELEM_BLOCKS, bn_threads(C), 0, st>>>(dout, ldd, x, M, C, T, B, lens, stat, gamma, beta, eps, act, site, seedp,
+                                                                     utt_offset, dbeta, dgamma, dx, ldx);
+    launch_counter() += 2;
+    return cudaGetLastError();
+}
+inline cudaError_t launch_ln_bwd(const float* dx, const float* ypre, const float* gamma, float eps, int M, int T, float* dy32, bf16* dsub16, int site,
+                                 const uint64_t* seedp, int utt_offset, uint32_t thresh, float dscale, float* dgamma, float* dbeta, cudaStream_t st) {
+    ln_bwd_kernel<<<std::min((M + 7) / 8, 592), 256, 0, st>>>(dx, ypre, gamma, eps, M, T, dy32, dsub16, site, seedp, utt_offset, thresh, dscale,
+                                                              dgamma, dbeta);
+    ++launch_counter();
+    return cudaGetLastError();
+}
+// acc (16 floats) zeroed, loss and its gradients, loss_out[0] = the scalar loss
+inline cudaError_t launch_loss(const float* before, const float* after, const float* stop, const float* target, const int* lens, int B, int T,
+                               float pos_weight, float* acc, float* dbefore32, float* dafter32, float* dstop32, float* loss_out, cudaStream_t st) {
+    cudaError_t e = cudaMemsetAsync(acc, 0, 64, st);
+    if (e != cudaSuccess) return e;
+    const long M = (long)B * T;
+    loss_kernel<<<std::min<long>((M * 81 + 255) / 256, 2368), 256, 0, st>>>(before, after, stop, target, lens, B, T, pos_weight, acc, dbefore32,
+                                                                            dafter32, dstop32);
+    loss_finalize_kernel<<<1, 32, 0, st>>>(acc, lens, B, loss_out);
+    launch_counter() += 2;
+    return cudaGetLastError();
+}
+inline cudaError_t launch_head_grad(const float* dbefore32, const float* dafter32, const bf16* dpost0, int ldp, const float* dstop32, const int* lens,
+                                    int M, int T, bf16* dhead16, cudaStream_t st) {
+    head_grad_kernel<<<(unsigned)(((long)M * 128 + 255) / 256), 256, 0, st>>>(dbefore32, dafter32, dpost0, ldp, dstop32, lens, M, T, dhead16);
+    ++launch_counter();
+    return cudaGetLastError();
+}
+// the decoder's word-dropout backward runs on 1184 blocks, the encoder's (fewer rows) on 592
+inline cudaError_t launch_dropw_bwd(bool decoder, const float* d, bf16* out, int M, int T, int site, const uint64_t* seedp, int utt_offset,
+                                    uint32_t thresh, float dscale, const float* pe, float* dalpha, cudaStream_t st) {
+    dropw_bwd_kernel<<<decoder ? 1184 : 592, 256, 0, st>>>(d, out, M, T, site, seedp, utt_offset, thresh, dscale, pe, dalpha);
+    ++launch_counter();
+    return cudaGetLastError();
+}
+inline cudaError_t launch_embed_bwd(const bf16* d, const int64_t* ph, const int* lens, int M, int S, int V, float* dE, cudaStream_t st) {
+    embed_bwd_kernel<<<(unsigned)(((long)M * 512 + 255) / 256), 256, 0, st>>>(d, ph, lens, M, S, V, dE);
+    ++launch_counter();
+    return cudaGetLastError();
+}
+
 // ---------------------------------------------------------------------------------------------- Adam (Vaswani: beta (0.9, 0.98), eps 1e-9)
 __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, long n, float lr,
                             float beta1, float beta2, float eps, float bc1, float bc2, float grad_scale) {

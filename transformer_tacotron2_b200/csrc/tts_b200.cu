@@ -929,6 +929,87 @@ extern "C" int tts_k_philox_bits(uint64_t seed, int site, int T, int B, int C, i
 // training (train.cuh)
 #include "train.cuh"
 
+// per-kernel test entry points of the training step: each launches what the step launches, through the same helpers
+extern "C" int tts_k_wgrad(const void* dY, int ldy, int Cout, const void* X, int ldx, int Cin, int taps, int T, int nb, float* dW, float* dbias,
+                           void* stream) {
+    if (!dY || !X || !dW || Cout <= 0 || Cin <= 0 || T <= 0 || nb <= 0 || (taps != 1 && taps != 5) || ldy < Cout || ldx < Cin) return TTS_E_ARG;
+    WgradParams g;
+    g.dY = (const bf16*)dY; g.ldy = ldy; g.Cout = Cout; g.X = (const bf16*)X; g.ldx = ldx; g.Cin = Cin; g.taps = taps;
+    g.T = T; g.nb = nb; g.dW = dW; g.dbias = dbias;
+    return (int)launch_wgrad_tc(g, (cudaStream_t)stream);
+}
+extern "C" int tts_k_dgrad(const float* W, int N, int K, int taps, const void* dY, int ldy, int Kdy, int M, int T, float* out_f32, void* out_bf16,
+                           int ldo, void* scratch, void* stream) {
+    if (!W || !dY || !scratch || (!out_f32 == !out_bf16) || N <= 0 || K <= 0 || M <= 0 || T <= 0 || (M % T) || (taps != 1 && taps != 5) ||
+        Kdy < N || ldy < Kdy || ldo < K)
+        return TTS_E_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    const TrMat m = tr_mat_dims(N, K, taps);
+    int blocks = 0;
+    const PackDesc d = tr_pack_desc(m, 1, 0, 0, 0, &blocks);
+    PackDesc* dd = nullptr;
+    cudaError_t e = cudaMallocAsync(&dd, sizeof(PackDesc), st);
+    if (e != cudaSuccess) return (int)e;
+    e = cudaMemcpyAsync(dd, &d, sizeof(PackDesc), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) {
+        cast_pack_all_kernel<<<blocks, 256, 0, st>>>(dd, 1, W, (bf16*)scratch);
+        ++launch_counter();
+        e = cudaGetLastError();
+    }
+    const cudaError_t ef = cudaFreeAsync(dd, st);
+    if (e != cudaSuccess) return (int)e;
+    if (ef != cudaSuccess) return (int)ef;
+    GemmParams p = tr_dgrad_params(m, (const bf16*)scratch, (const bf16*)dY, ldy, Kdy, M, T);
+    p.out_f32 = out_f32; p.out_bf16 = (bf16*)out_bf16; p.ldo = ldo;
+    return (int)launch_gemm_tc(p, st);
+}
+extern "C" int tts_k_bn_train_fwd(const float* x, int B, int T, int C, const int32_t* lens, float* stat, const float* gamma, const float* beta,
+                                  float eps, int act, int site, const uint64_t* seed, int utt_offset, void* out16, int ldo, float* out32,
+                                  float* run_mean, float* run_var, void* stream) {
+    if (!x || !lens || !stat || !gamma || !beta || !seed || B <= 0 || T <= 0 || C <= 0 || (C % 4) || 2 * C > BN_STAT_FLOATS ||
+        (out16 && (ldo < C || (ldo % 4))) || (!run_mean != !run_var))
+        return TTS_E_ARG;
+    return (int)launch_bn_train_fwd(x, B * T, C, T, B, lens, stat, gamma, beta, eps, act, site, seed, utt_offset, (bf16*)out16, ldo, out32, run_mean,
+                                    run_var, (cudaStream_t)stream);
+}
+extern "C" int tts_k_bn_train_bwd(const void* dout, int dout_bf16, int ldd, const float* x, int B, int T, int C, const int32_t* lens, const float* stat,
+                                  const float* gamma, const float* beta, float eps, int act, int site, const uint64_t* seed, int utt_offset,
+                                  float* dgamma, float* dbeta, void* dx, int ldx, void* stream) {
+    if (!dout || !x || !lens || !stat || !gamma || !beta || !seed || !dgamma || !dbeta || !dx || B <= 0 || T <= 0 || C <= 0 || (C % 4) ||
+        2 * C > BN_STAT_FLOATS || ldd < C || ldx < C || (ldx % 4))
+        return TTS_E_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dout_bf16)
+        return (int)launch_bn_train_bwd<bf16>((const bf16*)dout, ldd, x, B * T, C, T, B, lens, stat, gamma, beta, eps, act, site, seed, utt_offset, dbeta,
+                                              dgamma, (bf16*)dx, ldx, st);
+    return (int)launch_bn_train_bwd<float>((const float*)dout, ldd, x, B * T, C, T, B, lens, stat, gamma, beta, eps, act, site, seed, utt_offset, dbeta,
+                                           dgamma, (bf16*)dx, ldx, st);
+}
+extern "C" int tts_k_ln_bwd(const float* dx, const float* ypre, const float* gamma, float eps, int M, int T, float* dy32, void* dsub16, int site,
+                            const uint64_t* seed, int utt_offset, uint32_t thresh, float dscale, float* dgamma, float* dbeta, void* stream) {
+    if (!dx || !ypre || !gamma || !seed || !dgamma || !dbeta || M <= 0 || T <= 0) return TTS_E_ARG;
+    return (int)launch_ln_bwd(dx, ypre, gamma, eps, M, T, dy32, (bf16*)dsub16, site, seed, utt_offset, thresh, dscale, dgamma, dbeta, (cudaStream_t)stream);
+}
+extern "C" int tts_k_loss(const float* before, const float* after, const float* stop, const float* target, const int32_t* lens, int B, int T,
+                          float pos_weight, float* acc, float* dbefore, float* dafter, float* dstop, float* loss, void* stream) {
+    if (!before || !after || !stop || !target || !lens || !acc || !dbefore || !dafter || !dstop || !loss || B <= 0 || T <= 0) return TTS_E_ARG;
+    return (int)launch_loss(before, after, stop, target, lens, B, T, pos_weight, acc, dbefore, dafter, dstop, loss, (cudaStream_t)stream);
+}
+extern "C" int tts_k_head_grad(const float* dbefore, const float* dafter, const void* dpost0, int ldp, const float* dstop, const int32_t* lens, int B,
+                               int T, void* dhead, void* stream) {
+    if (!dbefore || !dafter || !dpost0 || !dstop || !lens || !dhead || B <= 0 || T <= 0 || ldp < 80) return TTS_E_ARG;
+    return (int)launch_head_grad(dbefore, dafter, (const bf16*)dpost0, ldp, dstop, lens, B * T, T, (bf16*)dhead, (cudaStream_t)stream);
+}
+extern "C" int tts_k_dropw_bwd(const float* d, void* out, int B, int T, int site, const uint64_t* seed, int utt_offset, uint32_t thresh, float dscale,
+                               const float* pe, float* dalpha, int decoder, void* stream) {
+    if (!d || !out || !seed || !pe || !dalpha || B <= 0 || T <= 0) return TTS_E_ARG;
+    return (int)launch_dropw_bwd(decoder != 0, d, (bf16*)out, B * T, T, site, seed, utt_offset, thresh, dscale, pe, dalpha, (cudaStream_t)stream);
+}
+extern "C" int tts_k_embed_bwd(const void* d, const int64_t* ph, const int32_t* lens, int B, int S, int V, float* dE, void* stream) {
+    if (!d || !ph || !lens || !dE || B <= 0 || S <= 0 || V <= 0) return TTS_E_ARG;
+    return (int)launch_embed_bwd((const bf16*)d, ph, lens, B * S, S, V, dE, (cudaStream_t)stream);
+}
+
 extern "C" int tts_train_begin(TtsHandle* h) {
     if (!h) return TTS_E_ARG;
     if (!h->finalized) FAIL(TTS_E_STATE, "weights not finalised");

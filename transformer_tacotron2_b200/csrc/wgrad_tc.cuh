@@ -157,11 +157,7 @@ __global__ void __launch_bounds__(WG_THREADS, 1) wgrad_tc_kernel(const __grid_co
                         float* o = g.dW + (size_t)n * ldo;
                         if (p.tma_red) {
                             // handled below by the whole warp (rows past Cout / columns past Cin are clipped by the tensor map)
-                        } else if (g.taps == 1 && kcol + 32 <= g.Cin && (ldo & 3) == 0) {
-#pragma unroll
-                            for (int i = 0; i < 32; i += 4)
-                                fb_red4(o + kcol + i, __uint_as_float(v[i]), __uint_as_float(v[i + 1]), __uint_as_float(v[i + 2]), __uint_as_float(v[i + 3]));
-                        } else {
+                        } else {                     // any layout or alignment of dW (Cin % 4 != 0, taps > 1, dW not 16-byte aligned)
 #pragma unroll
                             for (int i = 0; i < 32; ++i)
                                 if (kcol + i < g.Cin) atomicAdd(o + (size_t)(kcol + i) * g.taps + tap, __uint_as_float(v[i]));
