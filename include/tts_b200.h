@@ -107,6 +107,25 @@ int tts_forward(TtsHandle* h, void* ws, const int64_t* phonemes, const int32_t* 
                 const float* mels, const int32_t* mel_lens, int B, int S, int T, uint64_t seed, int utt_offset,
                 float* mel_before, float* mel_after, float* stop_logits, void* stream);
 
+/* ---- encoder-decoder attention alignments and phoneme durations (teacher-forced, eval mode) ----------------------------- */
+/* Bytes of device scratch tts_forward_align needs for focus / durations / head: per-row statistics of the cross-attention,
+ * rowmax fp32 + argmax int16 [6][B][H][T], and the focus rates fp32 [6][B][H]. */
+size_t tts_align_scratch_bytes(TtsHandle* h, int B, int S, int T);
+/* Teacher-forced eval forward, launch for launch tts_forward, plus the cross-attention P[b][h][t][s] = softmax_s(q_t . k_s / 8)
+ * of the decoder layers in layer_mask (bit l = layer l, 1 .. 0x3f), computed from the same bf16 operands as the forward's
+ * attention.  Keys s >= phoneme_lens[b] and rows t >= mel_lens[b] are zero.  Device pointers; every output may be NULL:
+ *   mel_before / mel_after / stop_logits  as tts_forward; all three NULL skips the heads and the postnet (all or none);
+ *   align      fp32 [popcount(layer_mask)][B][H][T][S], the selected layers in ascending order;
+ *   focus      fp32 [6][B][H]: focus rate = mean over t < mel_lens[b] of max_s P (unselected layers -1);
+ *   durations  int32 [B][S]: number of frames t < mel_lens[b] whose first-maximal key is s (sums to mel_lens[b] when
+ *              phoneme_lens[b] >= 1), for the head head[b] (int32 [B], = layer * 8 + h): the one with the largest focus rate
+ *              among the selected layers (ties: lowest index), or fixed_head if >= 0 (its layer must be selected).
+ * scratch (tts_align_scratch_bytes) is needed when focus, durations or head is requested.  No host synchronisation. */
+int tts_forward_align(TtsHandle* h, void* ws, void* scratch, const int64_t* phonemes, const int32_t* phoneme_lens,
+                      const float* mels, const int32_t* mel_lens, int B, int S, int T, uint64_t seed, int utt_offset,
+                      uint32_t layer_mask, int fixed_head, float* mel_before, float* mel_after, float* stop_logits,
+                      float* align, float* focus, int32_t* durations, int32_t* head, void* stream);
+
 /* Optional per-utterance controls of a decode session (between tts_decode_begin and the first tts_decode_steps; device int32 [B],
  * either may be NULL):
  *   utt_ids   global utterance id of every row = its dropout key (default utt_offset + row).  With ids the batch may be decoded in
@@ -213,6 +232,11 @@ int tts_k_attention_lse(const void* Q, const void* K, const void* V, void* O, fl
 int tts_k_attention_bwd(const void* Q, const void* K, const void* V, const void* O, const void* dO, const float* lse,
                         const int32_t* klens, void* dQ, void* dK, void* dV, float* scratch,
                         int B, int H, int Lq, int Lk, int causal, void* stream);
+/* Cross-attention probabilities (align.cuh): Q [B][Lq][ldq] bf16 (head h at column 64 h), K [B][H][Lk][64] bf16 ->
+ * P [B][H][Lq][Lk] fp32, rowmax [B][H][Lq] fp32 (max_s P), argmax [B][H][Lq] int16 (first key with the largest score; -1 for
+ * rows t >= qlens[b] or with no valid key).  qlens / klens int32 [B] may be NULL (all valid); every output may be NULL. */
+int tts_k_cross_align(const void* Q, int ldq, const void* K, const int32_t* qlens, const int32_t* klens,
+                      int B, int H, int Lq, int Lk, float* P, float* rowmax, int16_t* argmax, void* stream);
 /* LayerNorm over rows of 512: fp32 in -> bf16 out. */
 int tts_k_layernorm(const float* X, const float* gamma, const float* beta, void* Y_bf16, int M, float eps, void* stream);
 /* Keep-bits of a p = 0.5 dropout site: out[t][b][c] (uint8) for t < T, b < B, c < C. */

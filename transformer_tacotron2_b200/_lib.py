@@ -41,6 +41,8 @@ SIGNATURES = {
     "tts_decode_get_frame": (_I, [_P, _P, _I, _P, _P, _P]),
     "tts_infer_host": (_I, [_P, _P, _P, _P, _I, _I, _I, _U64, _I, _P, _P, _P, C.POINTER(_I), _P]),
     "tts_forward": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _U64, _I, _P, _P, _P, _P]),
+    "tts_align_scratch_bytes": (_SZ, [_P, _I, _I, _I]),
+    "tts_forward_align": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _U64, _I, C.c_uint32, _I] + [_P] * 8),
     "tts_debug_phase_timestamps": (_I, [_P, _P, _P, _I, _P]),
     "tts_debug_read_dump": (_I, [_P, _P, _I64, _I64, _P, _P]),
     "tts_debug_kv_index": (_I, [_I, _I, _I]),
@@ -67,6 +69,7 @@ SIGNATURES = {
     "tts_k_attention": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "tts_k_attention_lse": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "tts_k_attention_bwd": (_I, [_P] * 11 + [_I, _I, _I, _I, _I, _P]),
+    "tts_k_cross_align": (_I, [_P, _I, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P]),
     "tts_k_layernorm": (_I, [_P, _P, _P, _P, _I, C.c_float, _P]),
     "tts_k_philox_bits": (_I, [_U64, _I, _I, _I, _I, _I, _P, _P]),
     "tts_k_wgrad": (_I, [_P, _I, _I, _P, _I, _I, _I, _I, _I, _P, _P, _P]),

@@ -21,6 +21,7 @@
 #include "decode_cluster.cuh"
 #include "train_kernels.cuh"
 #include "wgrad_tc.cuh"
+#include "align.cuh"
 
 using namespace tts;
 
@@ -724,16 +725,21 @@ extern "C" int tts_infer_host(TtsHandle* h, void* ws, const int64_t* phonemes, c
 }
 
 // ------------------------------------------------------------------------------------------------
-extern "C" int tts_forward(TtsHandle* h, void* ws, const int64_t* phonemes, const int32_t* phoneme_lens, const float* mels,
-                           const int32_t* mel_lens, int B, int S, int T, uint64_t seed, int utt_offset, float* mel_before,
-                           float* mel_after, float* stop_logits, void* stream) {
-    if (!h || !ws || !phonemes || !phoneme_lens || !mels || !mel_lens || !mel_before || !mel_after || !stop_logits) return TTS_E_ARG;
-    if (B <= 0 || S <= 0 || T <= 0) return TTS_E_ARG;
-    if (!h->finalized) FAIL(TTS_E_STATE, "weights not finalised");
-    if (S > h->cfg.max_pos || T > h->cfg.max_pos) FAIL(TTS_E_ARG, "sequence exceeds max_pos");
-    DEV_GUARD(h);
-    cudaStream_t st = (cudaStream_t)stream;
-    const Ws L = Ws::make(B, S, T);
+// Where the teacher-forced forward sends the cross-attention of the decoder layers in layer_mask: P of the selected layers in
+// ascending layer order (align, may be null) and the per-row statistics [6][B][H][T] (rowmax / argmax, may be null).
+struct AlignSink {
+    uint32_t layer_mask;
+    float* align;
+    float* rowmax;
+    int16_t* argmax;
+};
+
+// Teacher-forced eval forward (encoder, prenet, decoder, heads, postnet).  With a sink, the cross-attention probabilities of the
+// selected layers are computed right after that layer's flash launch, while x2 still holds its queries; without one the
+// launches are exactly those of tts_forward.  mel_before == null skips the heads and the postnet.
+static int run_teacher_forced(TtsHandle* h, void* ws, const Ws& L, const int64_t* phonemes, const int32_t* phoneme_lens, const float* mels,
+                              const int32_t* mel_lens, int B, int S, int T, uint64_t seed, int utt_offset, float* mel_before,
+                              float* mel_after, float* stop_logits, const AlignSink* sink, cudaStream_t st) {
     int r = run_encoder(h, ws, L, phonemes, phoneme_lens, B, S, false, st);
     if (r) return r;
     const int M = B * T;
@@ -776,6 +782,18 @@ extern "C" int tts_forward(TtsHandle* h, void* ws, const int64_t* phonemes, cons
         at.K = ckv + (size_t)(l * 2) * ckv_layer; at.V = ckv + (size_t)(l * 2 + 1) * ckv_layer;     // [B][H][S][64]
         at.k_bs = at.v_bs = (long)kHeads * L.Spad * kDHead; at.k_hs = at.v_hs = (long)L.Spad * kDHead; at.k_rs = at.v_rs = kDHead;
         CK(launch_flash_attn_tc(at, st));
+        if (sink && ((sink->layer_mask >> l) & 1u)) {
+            AlignParams al; memset(&al, 0, sizeof(al));
+            al.Q = x2; al.q_bs = (long)T * 512; al.q_rs = 512;
+            al.K = at.K; al.k_bs = at.k_bs; al.k_hs = at.k_hs;
+            al.qlens = mel_lens; al.klens = phoneme_lens;
+            al.B = B; al.H = kHeads; al.Lq = T; al.Lk = S; al.scale_log2 = at.scale_log2;
+            const size_t per_layer = (size_t)B * kHeads * T;
+            if (sink->align) al.P = sink->align + (size_t)__builtin_popcount(sink->layer_mask & ((1u << l) - 1u)) * per_layer * S;
+            if (sink->rowmax) al.rowmax = sink->rowmax + (size_t)l * per_layer;
+            if (sink->argmax) al.argmax = sink->argmax + (size_t)l * per_layer;
+            CK(launch_cross_align(al, st));
+        }
         p = gp(a, 512, W.wo2, 512, M, 512, 512); p.bias = W.bo2; p.resid_bf16 = x; p.ldr = 512; p.out_f32 = y; p.ldo = 512;
         CK(launch_gemm_tc(p, st));
         CK(layernorm(y, W.ln2g, W.ln2b, x, nullptr, M, h->cfg.ln_eps, st));
@@ -785,6 +803,7 @@ extern "C" int tts_forward(TtsHandle* h, void* ws, const int64_t* phonemes, cons
         CK(launch_gemm_tc(p, st));
         CK(layernorm(y, W.ln3g, W.ln3b, x, nullptr, M, h->cfg.ln_eps, st));
     }
+    if (!mel_before) return 0;
     {   // [mel | stop] heads, zeroed past mel_lens
         GemmParams p = gp(x, 512, h->head_w, 512, M, 81, 512);
         p.T = T; p.bias = h->head_b; p.lens = mel_lens; p.scatter = SC_HEAD; p.out_f32 = mel_before; p.out2_f32 = stop_logits;
@@ -797,6 +816,76 @@ extern "C" int tts_forward(TtsHandle* h, void* ws, const int64_t* phonemes, cons
         CK(cudaGetLastError());
     }
     return run_postnet(h, ws, L, mel_lens, B, T, mel_after, st);
+}
+
+extern "C" int tts_forward(TtsHandle* h, void* ws, const int64_t* phonemes, const int32_t* phoneme_lens, const float* mels,
+                           const int32_t* mel_lens, int B, int S, int T, uint64_t seed, int utt_offset, float* mel_before,
+                           float* mel_after, float* stop_logits, void* stream) {
+    if (!h || !ws || !phonemes || !phoneme_lens || !mels || !mel_lens || !mel_before || !mel_after || !stop_logits) return TTS_E_ARG;
+    if (B <= 0 || S <= 0 || T <= 0) return TTS_E_ARG;
+    if (!h->finalized) FAIL(TTS_E_STATE, "weights not finalised");
+    if (S > h->cfg.max_pos || T > h->cfg.max_pos) FAIL(TTS_E_ARG, "sequence exceeds max_pos");
+    DEV_GUARD(h);
+    return run_teacher_forced(h, ws, Ws::make(B, S, T), phonemes, phoneme_lens, mels, mel_lens, B, S, T, seed, utt_offset, mel_before,
+                              mel_after, stop_logits, nullptr, (cudaStream_t)stream);
+}
+
+// ------------------------------------------------------------------------------------------------
+// alignments and durations (align.cuh).  Scratch: rowmax fp32 [6][B][H][T] | argmax int16 [6][B][H][T] | focus fp32 [6][B][H].
+namespace {
+struct AlignScratch {
+    size_t rowmax, argmax, focus, total;
+    static AlignScratch make(int B, int T) {
+        AlignScratch a; size_t o = 0;
+        auto take = [&](size_t bytes) { size_t r = o; o = align_up(o + bytes); return r; };
+        const size_t rows = (size_t)6 * B * kHeads * T;
+        a.rowmax = take(rows * 4); a.argmax = take(rows * 2); a.focus = take((size_t)6 * B * kHeads * 4);
+        a.total = o;
+        return a;
+    }
+};
+}  // namespace
+
+extern "C" size_t tts_align_scratch_bytes(TtsHandle* h, int B, int S, int T) {
+    if (!h || B <= 0 || S <= 0 || T <= 0) return 0;
+    return AlignScratch::make(B, T).total;
+}
+
+extern "C" int tts_forward_align(TtsHandle* h, void* ws, void* scratch, const int64_t* phonemes, const int32_t* phoneme_lens,
+                                 const float* mels, const int32_t* mel_lens, int B, int S, int T, uint64_t seed, int utt_offset,
+                                 uint32_t layer_mask, int fixed_head, float* mel_before, float* mel_after, float* stop_logits,
+                                 float* align, float* focus, int32_t* durations, int32_t* head, void* stream) {
+    if (!h || !ws || !phonemes || !phoneme_lens || !mels || !mel_lens || B <= 0 || S <= 0 || T <= 0) return TTS_E_ARG;
+    if (!h->finalized) FAIL(TTS_E_STATE, "weights not finalised");
+    if (S > h->cfg.max_pos || T > h->cfg.max_pos) FAIL(TTS_E_ARG, "sequence exceeds max_pos");
+    if (S > 32767) FAIL(TTS_E_ARG, "S exceeds the int16 range of the per-row argmax");
+    if (!mel_before != !mel_after || !mel_before != !stop_logits) FAIL(TTS_E_ARG, "mel_before, mel_after and stop_logits: all or none");
+    if (layer_mask == 0 || layer_mask > 0x3fu) FAIL(TTS_E_ARG, "layer_mask must select decoder layers 0..5 (1 .. 0x3f)");
+    if (fixed_head < -1 || fixed_head >= 6 * kHeads || (fixed_head >= 0 && !((layer_mask >> (fixed_head / kHeads)) & 1u)))
+        FAIL(TTS_E_ARG, "fixed_head must be -1 or layer * 8 + h of a selected layer");
+    const bool stats = focus || durations || head;
+    if (stats && !scratch) FAIL(TTS_E_ARG, "focus / durations / head need the scratch of tts_align_scratch_bytes");
+    DEV_GUARD(h);
+    cudaStream_t st = (cudaStream_t)stream;
+    const AlignScratch A = AlignScratch::make(B, T);
+    AlignSink sink{layer_mask, align, stats ? wsp<float>(scratch, A.rowmax) : nullptr, stats ? wsp<int16_t>(scratch, A.argmax) : nullptr};
+    int r = run_teacher_forced(h, ws, Ws::make(B, S, T), phonemes, phoneme_lens, mels, mel_lens, B, S, T, seed, utt_offset, mel_before,
+                               mel_after, stop_logits, (align || stats) ? &sink : nullptr, st);
+    if (r) return r;
+    float* f = focus ? focus : wsp<float>(scratch, A.focus);
+    if (focus || ((durations || head) && fixed_head < 0)) {
+        const int warps = 6 * B * kHeads;
+        focus_kernel<<<(warps + 7) / 8, 256, 0, st>>>(sink.rowmax, mel_lens, B, kHeads, T, layer_mask, f);
+        ++launch_counter();
+        CK(cudaGetLastError());
+    }
+    if (durations || head) {
+        durations_kernel<<<B, 256, (size_t)S * 4, st>>>(f, sink.argmax, mel_lens, phoneme_lens, B, kHeads, S, T, layer_mask, fixed_head,
+                                                        durations, head);
+        ++launch_counter();
+        CK(cudaGetLastError());
+    }
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -867,6 +956,16 @@ extern "C" int tts_k_attention_lse(const void* Q, const void* K, const void* V, 
     AttnParams a = ap_packed((const bf16*)Q, ld, (const bf16*)K, ld, (const bf16*)V, ld, (bf16*)O, ld, B, Lq, Lk, klens, causal);
     a.H = H; a.lse = lse;
     return (int)launch_flash_attn_tc(a, (cudaStream_t)stream);
+}
+extern "C" int tts_k_cross_align(const void* Q, int ldq, const void* K, const int32_t* qlens, const int32_t* klens, int B, int H, int Lq,
+                                 int Lk, float* P, float* rowmax, int16_t* argmax, void* stream) {
+    if (!Q || !K || B <= 0 || H <= 0 || Lq <= 0 || Lk <= 0 || Lk > 32767 || ldq < H * 64 || (ldq % 8)) return TTS_E_ARG;
+    AlignParams a; memset(&a, 0, sizeof(a));
+    a.Q = (const bf16*)Q; a.q_bs = (long)Lq * ldq; a.q_rs = ldq;
+    a.K = (const bf16*)K; a.k_hs = (long)Lk * 64; a.k_bs = (long)H * Lk * 64;
+    a.qlens = qlens; a.klens = klens; a.B = B; a.H = H; a.Lq = Lq; a.Lk = Lk; a.scale_log2 = 0.125f * kLog2e;
+    a.P = P; a.rowmax = rowmax; a.argmax = argmax;
+    return (int)launch_cross_align(a, (cudaStream_t)stream);
 }
 namespace {
 // fp32 -> bf16 rows (dQ accumulator -> operand)

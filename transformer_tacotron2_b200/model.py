@@ -293,6 +293,75 @@ class TransformerTTS(nn.Module):
         self._check(rc, "tts_forward")
         return mb, ma, st
 
+    # ------------------------------------------------------------------ cross-attention alignments / durations
+    @torch.no_grad()
+    def alignments(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_ids=None, utt_offset: int = 0, layers=None
+                   ) -> torch.Tensor:
+        """Encoder-decoder attention of the teacher-forced forward (eval mode): [n_layers, B, 8, T, S] fp32, P[l, b, h, t, s] =
+        softmax_s(q_t . k_s / 8) of decoder layer layers[l] (default: all six, ascending), zero at frames t >= mel_lens[b] and
+        phonemes s >= phoneme_lens[b].  Same inputs as forward(); CUDA tensors in -> CUDA tensor out, CPU in -> CPU out.
+
+        Alignments of a free-running (AR) output: `_, lens, _, mb = model.inference(ph, pl, ..., return_before=True)` then
+        `model.alignments(ph, pl, mb, lens)` with the same seed -- the teacher-forced decoder then sees exactly the frames the
+        AR decoder fed back (shifted right behind the zero go-frame, same prenet dropout masks)."""
+        ls, mask = self._align_layers(layers)
+        out = self._forward_align(phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset, mask, -1, True, False)
+        return out["align"] if phonemes.is_cuda else out["align"].cpu()
+
+    @torch.no_grad()
+    def durations(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_ids=None, utt_offset: int = 0, layers=None,
+                  head: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """FastSpeech duration targets from the teacher-forced cross-attention (Ren et al., 2019, section 3.3; ESPnet's
+        DurationCalculator), computed on the GPU without forming P in memory.
+        -> durations [B, S] int32 (frames t < mel_lens[b] whose most-attended phoneme is s; sums to mel_lens[b]),
+           head [B] int32 (layer * 8 + h used for utterance b: the one with the largest focus rate among `layers`, lowest index
+           on ties, unless `head` = layer * 8 + h fixes it), focus [6, B, 8] fp32 (focus rate = mean over valid frames of
+           max_s P; -1 for layers not selected)."""
+        ls, mask = self._align_layers(layers)
+        fixed = -1 if head is None else int(head)
+        if fixed != -1 and not (0 <= fixed < 48 and fixed // 8 in ls):
+            raise ValueError("head must be layer * 8 + h of a selected layer")
+        out = self._forward_align(phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset, mask, fixed, False, True)
+        res = (out["durations"], out["head"], out["focus"])
+        return res if phonemes.is_cuda else tuple(t.cpu() for t in res)
+
+    @staticmethod
+    def _align_layers(layers):
+        ls = list(range(6)) if layers is None else sorted({int(v) for v in layers})
+        if not ls or ls[0] < 0 or ls[-1] > 5:
+            raise ValueError("layers must be decoder layer indices in 0..5")
+        return ls, sum(1 << v for v in ls)
+
+    def _forward_align(self, phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset, layer_mask, fixed_head,
+                       want_align, want_durations):
+        if self.training:
+            raise RuntimeError("alignments() / durations() are eval-mode paths: call model.eval() first")
+        lib = self._ensure_handle()
+        self.sync_weights()
+        dev = self.device
+        B, S = phonemes.shape
+        T = mels.shape[1]
+        ph = phonemes.to(dev, torch.int64).contiguous()
+        pl = phoneme_lens.to(dev, torch.int32).contiguous()
+        ml = mel_lens.to(dev, torch.int32).contiguous()
+        m = mels.to(dev, torch.float32).contiguous()
+        ws = self._workspace(B, S, T)
+        out, scratch = {}, None
+        if want_align:
+            out["align"] = torch.empty(bin(layer_mask).count("1"), B, 8, T, S, device=dev)
+        if want_durations:
+            scratch = torch.empty(lib.tts_align_scratch_bytes(self._handle, B, S, T), dtype=torch.uint8, device=dev)
+            out["durations"] = torch.empty(B, S, dtype=torch.int32, device=dev)
+            out["head"] = torch.empty(B, dtype=torch.int32, device=dev)
+            out["focus"] = torch.empty(6, B, 8, device=dev)
+        ptr = lambda k: out[k].data_ptr() if k in out else None                                          # noqa: E731
+        rc = lib.tts_forward_align(self._handle, ws.data_ptr(), scratch.data_ptr() if scratch is not None else None, ph.data_ptr(),
+                                   pl.data_ptr(), m.data_ptr(), ml.data_ptr(), B, S, T, int(seed), self._utt_offset(utt_ids, B, utt_offset),
+                                   layer_mask, fixed_head, None, None, None, ptr("align"), ptr("focus"), ptr("durations"), ptr("head"),
+                                   self._stream())
+        self._check(rc, "tts_forward_align")
+        return out
+
     def _train_forward(self, phonemes, phoneme_lens, mels, mel_lens, seed, utt_offset):
         """Train-mode forward with autograd: `model.train(); out = model(...); loss_fn(*out).backward(); optimiser.step()` works on
         the module exactly as on the oracle (oracle/transformer_tts.py: forward in .train() mode).  Arithmetic: the library's
