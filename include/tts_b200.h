@@ -93,6 +93,23 @@ int tts_decode_status(TtsHandle* h, void* ws, int* t_done, int* n_finished, void
  * mel_after [B][T_out][80] f32, mel_lens [B] i32, stop_logits [B][T_out] f32, mel_before (optional). */
 int tts_decode_end(TtsHandle* h, void* ws, int T_out, float* mel_after, int32_t* mel_lens,
                    float* stop_logits, float* mel_before, void* stream);
+/* Streaming: postnet-refined frames of a running decode session, emitted while the decoder keeps going.
+ * The postnet is eval-mode arithmetic with a receptive field of halo = postnet_layers * (conv_kernel / 2) = 10 frames per side, so
+ * frame t is final once frame t + halo is decoded.  Every tts_decode_status fixes the frontier: the decoded frame count if every
+ * utterance has stopped or max_len is reached, else that count - halo; tts_decode_steps does not move it.
+ * Bytes of device scratch for tts_decode_emit calls of at most max_frames frames (window = max_frames + 2 * halo rows). */
+size_t tts_stream_scratch_bytes(TtsHandle* h, int B, int max_frames);
+/* mel_after / stop_logits of frames [t_begin, t_end) of every utterance of the running decode session, as tts_decode_end would
+ * return them: compact [B][t_end - t_begin][80] / [B][t_end - t_begin] fp32, zero at t >= the utterance's length.  Optional:
+ * mel_before (same layout) and mel_lens int32 [B] (the length of every utterance that had stopped by the last status, as
+ * tts_decode_end's mel_lens; -1 for one still running).  t_end must not exceed the frontier; scratch holds scratch_bytes bytes,
+ * at least what tts_stream_scratch_bytes gives for t_end - t_begin frames.  TTS_E_STATE without a session or before its first
+ * status call, TTS_E_ARG for t_begin < 0, t_end <= t_begin, t_end past the frontier or a scratch too small, all before any launch.
+ * May run on another stream concurrently with tts_decode_steps: it reads only frames below the frontier, writes only the scratch
+ * and the outputs, and its GEMMs use only the SMs the decode kernel's clusters leave free.  One window kernel and five
+ * postnet GEMM launches per call. */
+int tts_decode_emit(TtsHandle* h, void* ws, void* scratch, size_t scratch_bytes, int t_begin, int t_end, float* mel_after,
+                    float* stop_logits, int32_t* mel_lens, float* mel_before, void* stream);
 /* The whole of .inference() with HOST buffers (pageable or pinned): H2D, encode, decode loop,
  * postnet, D2H.  Outputs are written compactly as [B][T_out]...; *T_out returns the frames run.
  * `ws` is device scratch of tts_workspace_bytes(B, S, max_len). [sync] */

@@ -39,6 +39,8 @@ SIGNATURES = {
     "tts_decode_set_batch": (_I, [_P, _P, _P, _P, _I, _P]),
     "tts_decode_set_frame": (_I, [_P, _P, _I, _P, _P]),
     "tts_decode_get_frame": (_I, [_P, _P, _I, _P, _P, _P]),
+    "tts_stream_scratch_bytes": (_SZ, [_P, _I, _I]),
+    "tts_decode_emit": (_I, [_P, _P, _P, _SZ, _I, _I, _P, _P, _P, _P, _P]),
     "tts_infer_host": (_I, [_P, _P, _P, _P, _I, _I, _I, _U64, _I, _P, _P, _P, C.POINTER(_I), _P]),
     "tts_forward": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _U64, _I, _P, _P, _P, _P]),
     "tts_align_scratch_bytes": (_SZ, [_P, _I, _I, _I]),

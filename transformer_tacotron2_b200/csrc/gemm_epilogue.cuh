@@ -35,6 +35,7 @@ struct GemmParams {
     // SC_HEAD    : out_f32 = mel_before [M][80], out2_f32 = stop_logits [M]
     float* out2_f32; int B;
     int Lpad;                        // SC_CROSS_KV*: row capacity of the cache per (layer, b, h): multiple of 16 (row-major) / 64 (blocks)
+    int max_ctas;                    // launch_gemm_tc: at most this many persistent CTAs (0 = one per SM); leaves SMs to a concurrent kernel
 };
 
 TTS_D void gemm_store(const GemmParams& p, int m, int n, float v0, float v1) {

@@ -381,7 +381,9 @@ inline cudaError_t launch_gemm_tc(const GemmParams& g, cudaStream_t stream) {
     }
     p.n_tiles_n = (g.N + TC_BN - 1) / TC_BN;
     p.n_tiles = p.n_tiles_n * nb * p.tiles_per_utt;
-    const int grid = p.n_tiles < num_sms ? p.n_tiles : num_sms;          // persistent: one CTA per SM, static round-robin tiles
+    int grid = p.n_tiles < num_sms ? p.n_tiles : num_sms;                // persistent: one CTA per SM, static round-robin tiles
+    // capped beside a running kernel: a CTA that finds no free SM would hold its round-robin tiles until that kernel ends
+    if (g.max_ctas > 0 && grid > g.max_ctas) grid = g.max_ctas;
     if (TC_BN == 256) gemm_tc_kernel<256><<<grid, TC_THREADS, tc_smem_bytes(256), stream>>>(p);
     else gemm_tc_kernel<128><<<grid, TC_THREADS, tc_smem_bytes(128), stream>>>(p);
     ++launch_counter();

@@ -77,6 +77,37 @@ __global__ void finalize_stop_kernel(const float* __restrict__ stop, int T_src, 
     if (idx < B && lens_out) lens_out[idx] = lens[idx];
 }
 
+// Postnet input of frames [a, a + W) of a running decode session (tts_decode_emit), the window counterpart of mel_to_bf16_kernel +
+// finalize_stop_kernel: bf16 [B][W][96] (zero channel padding) and the fp32 residual [B][W][80], both zero at t >= len;
+// wlens[b] = len - a clamped to [0, W] (the postnet's per-layer mask); stop [B][n] of frames [t_begin, t_begin + n), zero at
+// t >= len; lens_out[b] (optional) = lens[b] if the utterance had stopped by t_status, else -1.  Here len = min(lens[b], t_status).
+// lens[] may be written meanwhile by a decode launch from t_status on (an utterance stopping in it gets lens = t + 1 > t_status),
+// so either value gives the same len and the same lens_out; the frames read (< t_status) are written by no such launch.
+__global__ void stream_window_kernel(const float* __restrict__ mel, const float* __restrict__ stop, int T_src, const int* lens,
+                                     int t_status, int a, int W, int t_begin, int n, bf16* __restrict__ out16,
+                                     float* __restrict__ out32, int* __restrict__ wlens, float* __restrict__ stop_out,
+                                     int* __restrict__ lens_out, int B) {
+    const int idx = blockIdx.x * blockDim.x + threadIdx.x;            // one thread per (row, 4 channels); 24 groups/row
+    if (idx < B * W * 24) {
+        const int row = idx / 24, cg = idx - row * 24, b = row / W, t = a + (row - b * W);
+        const int len = min(*(volatile const int*)(lens + b), t_status);
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (cg < 20 && t < len) v = *reinterpret_cast<const float4*>(mel + ((size_t)b * T_src + t) * 80 + cg * 4);
+        *reinterpret_cast<uint2*>(out16 + (size_t)row * 96 + cg * 4) = make_uint2(pack_bf16x2(v.x, v.y), pack_bf16x2(v.z, v.w));
+        if (cg < 20) *reinterpret_cast<float4*>(out32 + (size_t)row * 80 + cg * 4) = v;
+    }
+    if (idx < B * n) {
+        const int b = idx / n, t = t_begin + (idx - b * n);
+        const int len = min(*(volatile const int*)(lens + b), t_status);
+        stop_out[idx] = t < len ? stop[(size_t)b * T_src + t] : 0.f;
+    }
+    if (idx < B) {
+        const int l = *(volatile const int*)(lens + idx);
+        wlens[idx] = max(0, min(min(l, t_status) - a, W));
+        if (lens_out) lens_out[idx] = l <= t_status ? l : -1;
+    }
+}
+
 __global__ void bf16_to_f32_kernel(const bf16* __restrict__ in, float* __restrict__ out, size_t n) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = __bfloat162float(in[i]);

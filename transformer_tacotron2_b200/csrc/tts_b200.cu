@@ -58,6 +58,7 @@ struct TtsHandle {
     bool dec_ids = false, dec_tlens = false, dec_steal = false;       // tts_decode_set_batch
     bool dec_active = false; int dec_B = 0, dec_S = 0, dec_T = 0, dec_t = 0; uint64_t dec_seed = 0; int dec_utt0 = 0;
     int* h_status = nullptr;                                          // pinned: t_done, n_finished
+    int dec_t_status = -1, dec_frontier = 0;                          // last tts_decode_status: frames decoded, frames final (-1: none yet)
     TtsTrain* train = nullptr;                                        // training state (train.cuh), built by tts_train_begin
     int train_graph = 1;                                              // replay the train step from a CUDA graph (option "train_graph")
 };
@@ -490,21 +491,26 @@ static int run_encoder(TtsHandle* h, void* ws, const Ws& L, const int64_t* ph, c
     return 0;
 }
 
-// Postnet (C8) over compact rows: in16 bf16 [B*T][96] masked, resid32 fp32 [B*T][80] masked -> mel_after [B*T][80].
-static int run_postnet(TtsHandle* h, void* ws, const Ws& L, const int* mlens, int B, int T, float* mel_after, cudaStream_t st) {
+// Postnet (C8) over compact rows: in16 bf16 [B*T][96] masked, resid32 fp32 [B*T][80] masked -> mel_after [B*T][80]; x / x2 are
+// bf16 [B*T][512] activations.  max_ctas caps the persistent GEMM grid (0: one CTA per SM).
+static int run_postnet_rows(TtsHandle* h, const bf16* in16, const float* resid32, bf16* x, bf16* x2, const int* mlens, int B, int T,
+                            float* mel_after, int max_ctas, cudaStream_t st) {
     const int M = B * T;
-    bf16 *x = wsp<bf16>(ws, L.x2), *x2 = wsp<bf16>(ws, L.a);
-    const bf16* in = wsp<bf16>(ws, L.mel16);
+    const bf16* in = in16;
     for (int i = 0; i < 5; ++i) {
         const int K = i == 0 ? 96 : 512, N = i == 4 ? 80 : 512;
         GemmParams p = gp(in, K, h->post_w[i], K, M, N, K);
-        p.taps = 5; p.T = T; p.bias = h->post_b[i]; p.lens = mlens;
+        p.taps = 5; p.T = T; p.bias = h->post_b[i]; p.lens = mlens; p.max_ctas = max_ctas;
         if (i < 4) { p.act = ACT_TANH; p.out_bf16 = x; p.ldo = 512; }
-        else { p.resid_f32 = wsp<float>(ws, L.mel32); p.ldr = 80; p.out_f32 = mel_after; p.ldo = 80; }
+        else { p.resid_f32 = resid32; p.ldr = 80; p.out_f32 = mel_after; p.ldo = 80; }
         CKL(launch_gemm_tc(p, st));
         in = x; std::swap(x, x2);
     }
     return 0;
+}
+static int run_postnet(TtsHandle* h, void* ws, const Ws& L, const int* mlens, int B, int T, float* mel_after, cudaStream_t st) {
+    return run_postnet_rows(h, wsp<bf16>(ws, L.mel16), wsp<float>(ws, L.mel32), wsp<bf16>(ws, L.x2), wsp<bf16>(ws, L.a), mlens, B, T,
+                            mel_after, 0, st);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -538,6 +544,7 @@ extern "C" int tts_decode_begin(TtsHandle* h, void* ws, int B, int S, int max_le
     const Ws L = Ws::make(B, S, max_len);
     h->dec_ids = h->dec_tlens = h->dec_steal = false;
     h->dec_active = true; h->dec_B = B; h->dec_S = S; h->dec_T = max_len; h->dec_t = 0; h->dec_seed = seed; h->dec_utt0 = utt_offset;
+    h->dec_t_status = -1; h->dec_frontier = 0;
     init_decode_state_kernel<<<(std::max(B, 4) + 255) / 256, 256, 0, st>>>(wsp<int>(ws, L.lens), wsp<int>(ws, L.finished),
                                                                           wsp<int>(ws, L.scalars), B, max_len);
     ++launch_counter();
@@ -610,6 +617,9 @@ extern "C" int tts_decode_steps(TtsHandle* h, void* ws, int n_steps, void* strea
     return 0;
 }
 
+// Frames on each side of a frame that the postnet's output at that frame depends on: layers x (kernel / 2).
+static int postnet_halo(const TtsHandle* h) { return h->cfg.postnet_layers * (h->cfg.conv_kernel / 2); }
+
 extern "C" int tts_decode_status(TtsHandle* h, void* ws, int* t_done, int* n_finished, void* stream) {
     if (!h || !ws) return TTS_E_ARG;
     if (!h->dec_active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
@@ -625,6 +635,11 @@ extern "C" int tts_decode_status(TtsHandle* h, void* ws, int* t_done, int* n_fin
         int mx = 0; for (int v : lens) mx = std::max(mx, v);
         h->dec_t = mx;
     }
+    // tts_decode_emit's frontier: a frame's postnet output is final once the postnet's halo past it is decoded, or once the session
+    // has ended (every utterance stopped, or max_len reached).  Only this call moves it; tts_decode_steps does not.
+    const bool ended = nf >= h->dec_B || h->dec_t >= h->dec_T;
+    h->dec_t_status = h->dec_t;
+    h->dec_frontier = ended ? h->dec_t : std::max(0, h->dec_t - postnet_halo(h));
     if (n_finished) *n_finished = nf;
     if (t_done) *t_done = h->dec_t;
     return 0;
@@ -690,6 +705,65 @@ extern "C" int tts_decode_end(TtsHandle* h, void* ws, int T_out, float* mel_afte
     }
     if (mel_before) CK(cudaMemcpyAsync(mel_before, wsp<float>(ws, L.mel32), (size_t)B * T_out * 80 * 4, cudaMemcpyDeviceToDevice, st));
     return run_postnet(h, ws, L, lens, B, T_out, mel_after, st);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Streaming: the postnet over a window of frames of a running decode session.  Scratch: postnet input bf16 [B][W][96] | residual
+// fp32 [B][W][80] | two bf16 activations [B][W][512] | output fp32 [B][W][80] | window lengths int32 [B].
+namespace {
+struct StreamScratch {
+    size_t in16, res32, xa, xb, out32, wlens, total;
+    static StreamScratch make(int B, int W) {
+        StreamScratch s; size_t o = 0;
+        auto take = [&](size_t bytes) { size_t r = o; o = align_up(o + bytes); return r; };
+        const size_t rows = (size_t)B * W;
+        s.in16 = take(rows * 96 * 2); s.res32 = take(rows * 80 * 4); s.xa = take(rows * 512 * 2); s.xb = take(rows * 512 * 2);
+        s.out32 = take(rows * 80 * 4); s.wlens = take((size_t)B * 4);
+        s.total = o;
+        return s;
+    }
+};
+}  // namespace
+
+extern "C" size_t tts_stream_scratch_bytes(TtsHandle* h, int B, int max_frames) {
+    if (!h || B <= 0 || max_frames <= 0) return 0;
+    return StreamScratch::make(B, max_frames + 2 * postnet_halo(h)).total;
+}
+
+extern "C" int tts_decode_emit(TtsHandle* h, void* ws, void* scratch, size_t scratch_bytes, int t_begin, int t_end, float* mel_after,
+                               float* stop_logits, int32_t* mel_lens, float* mel_before, void* stream) {
+    if (!h || !ws || !scratch || !mel_after || !stop_logits) return TTS_E_ARG;
+    if (!h->dec_active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
+    if (h->dec_t_status < 0) FAIL(TTS_E_STATE, "tts_decode_emit needs a tts_decode_status call first");
+    if (t_begin < 0 || t_end <= t_begin) FAIL(TTS_E_ARG, "frame range must be non-empty and start at >= 0");
+    if (t_end > h->dec_frontier) FAIL(TTS_E_ARG, "t_end lies past the frontier of the last tts_decode_status");
+    const int halo = postnet_halo(h), B = h->dec_B, n = t_end - t_begin;
+    const int a = std::max(0, t_begin - halo), e = std::min(t_end + halo, h->dec_t_status), W = e - a;
+    const StreamScratch S = StreamScratch::make(B, W);
+    if (S.total > scratch_bytes) FAIL(TTS_E_ARG, "scratch too small for this window (tts_stream_scratch_bytes)");
+    // the decode kernel holds CL_SIZE SMs per co-resident cluster while it runs; the postnet GEMMs take only the others
+    const int max_ctas = h->num_sms - CL_SIZE * std::min(h->cparams.ngroups, h->max_clusters);
+    if (max_ctas < 1) FAIL(TTS_E_DEVICE, "no SM left beside the decode kernel");
+    DEV_GUARD(h);
+    cudaStream_t st = (cudaStream_t)stream;
+    const Ws L = Ws::make(B, h->dec_S, h->dec_T);
+    const int nthreads = std::max(B * W * 24, B * n);
+    stream_window_kernel<<<(nthreads + 255) / 256, 256, 0, st>>>(wsp<float>(ws, L.mel_before), wsp<float>(ws, L.stop_logits), h->dec_T,
+                                                                 wsp<int>(ws, L.lens), h->dec_t_status, a, W, t_begin, n,
+                                                                 wsp<bf16>(scratch, S.in16), wsp<float>(scratch, S.res32),
+                                                                 wsp<int>(scratch, S.wlens), stop_logits, mel_lens, B);
+    ++launch_counter();
+    CK(cudaGetLastError());
+    // Rows within `halo` of a window edge that is not a true edge (t = 0 or the session's end) see zeros where the whole-utterance
+    // postnet sees frames: they are computed and dropped.  Rows [t_begin, t_end) see exactly what that postnet sees.
+    int r = run_postnet_rows(h, wsp<bf16>(scratch, S.in16), wsp<float>(scratch, S.res32), wsp<bf16>(scratch, S.xa), wsp<bf16>(scratch, S.xb),
+                             wsp<int>(scratch, S.wlens), B, W, wsp<float>(scratch, S.out32), max_ctas, st);
+    if (r) return r;
+    const size_t row_bytes = (size_t)n * 80 * 4, pitch = (size_t)W * 80 * 4, off = (size_t)(t_begin - a) * 80;
+    CK(cudaMemcpy2DAsync(mel_after, row_bytes, wsp<float>(scratch, S.out32) + off, pitch, row_bytes, (size_t)B, cudaMemcpyDeviceToDevice, st));
+    if (mel_before)
+        CK(cudaMemcpy2DAsync(mel_before, row_bytes, wsp<float>(scratch, S.res32) + off, pitch, row_bytes, (size_t)B, cudaMemcpyDeviceToDevice, st));
+    return 0;
 }
 
 extern "C" int tts_infer_host(TtsHandle* h, void* ws, const int64_t* phonemes, const int32_t* phoneme_lens, int B, int S,

@@ -10,7 +10,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass, asdict
-from typing import Optional, Tuple
+from typing import NamedTuple, Optional, Tuple
 
 import torch
 import torch.nn as nn
@@ -38,6 +38,46 @@ class TTSConfig:
 
     def to_dict(self):
         return asdict(self)
+
+
+def postnet_halo(cfg: TTSConfig) -> int:
+    """Frames on each side of a frame that the postnet's output there depends on (each conv layer reaches kernel // 2)."""
+    return cfg.postnet_layers * (cfg.conv_kernel // 2)
+
+
+class StreamSchedule:
+    """Decode / emit schedule of TransformerTTS.inference_stream(), kept apart from the device calls so that it can be checked
+    without a GPU.  The first decode launch runs chunk_frames + halo steps, every later one chunk_frames.  After each status
+    (frames decoded t_done; `ended` = every utterance stopped or max_len reached), after_status() returns the steps of the next
+    launch (0: none) and the frame range to emit (None: nothing new).  The range ends at the frontier: t_done once the session
+    has ended, else t_done - halo, since the postnet output of a later frame still depends on frames not decoded yet."""
+
+    def __init__(self, chunk_frames: int, halo: int, max_len: int):
+        if chunk_frames < 1:
+            raise ValueError("chunk_frames must be >= 1")
+        self.chunk, self.halo, self.max_len, self.emitted = int(chunk_frames), int(halo), int(max_len), 0
+
+    def first_steps(self) -> int:
+        return min(self.chunk + self.halo, self.max_len)
+
+    def max_emit_frames(self) -> int:
+        """Largest range after_status() returns: chunk + halo (the first, or the last after the session ends)."""
+        return min(self.chunk + self.halo, self.max_len)
+
+    def after_status(self, t_done: int, ended: bool):
+        frontier = t_done if ended else max(0, t_done - self.halo)
+        rng = (self.emitted, frontier) if frontier > self.emitted else None
+        self.emitted = max(self.emitted, frontier)
+        return (0 if ended else self.chunk), rng
+
+
+class StreamChunk(NamedTuple):
+    """Frames [start, start + n) of every utterance of a streamed batch."""
+    start: int
+    mel_after: torch.Tensor      # [B, n, 80] fp32, zero past each utterance's end
+    stop_logits: torch.Tensor    # [B, n] fp32, zero past each utterance's end
+    n_valid: torch.Tensor        # [B] int32: frames of utterance b inside the chunk
+    finished: torch.Tensor       # [B] bool: utterance b has stopped (or reached its frame budget / max_len)
 
 
 # ---- parameter containers: the state_dict layout of the module API -----------------------------
@@ -162,8 +202,10 @@ class TransformerTTS(nn.Module):
         self._synced_version = None
         self.profile_events = False      # bench.py: CUDA-event time of the decode loop per inference()
         self.decode_ms = []
+        self.emit_ms = []                # inference_stream(): CUDA-event time of every tts_decode_emit (with profile_events)
         self._ws = None
         self._ws_key = None
+        self._ws_uses = 0                # calls of _workspace(): an open inference_stream() detects a call that took the workspace
         self.eval()
 
     # ------------------------------------------------------------------ plumbing
@@ -233,6 +275,7 @@ class TransformerTTS(nn.Module):
 
     def _workspace(self, B, S, T):
         lib = self._ensure_handle()
+        self._ws_uses += 1
         key = (B, S, T)
         if self._ws_key != key:
             n = lib.tts_workspace_bytes(self._handle, B, S, T)
@@ -484,6 +527,93 @@ class TransformerTTS(nn.Module):
         if to_host:
             out = tuple(t.cpu() for t in out)
         return out
+
+    @torch.no_grad()
+    def inference_stream(self, phonemes, phoneme_lens, max_len: int = 800, seed: int = 0, chunk_frames: int = 50, utt_ids=None,
+                         utt_offset: int = 0, max_lens=None):
+        """Greedy AR like inference(), yielding StreamChunk(start, mel_after, stop_logits, n_valid, finished) while the decoder keeps
+        running.  The chunks cover consecutive frame ranges; concatenated along time they are exactly inference()'s mel_after and
+        stop_logits, and their n_valid sum to its mel_lens.  CUDA inputs give CUDA chunks (ready when yielded), CPU inputs CPU chunks.
+
+        A frame's postnet output is final once the `halo` (10) frames after it are decoded or its utterance has stopped, so the
+        first chunk comes after chunk_frames + 10 decoder steps and each later one after chunk_frames more.  The decoder runs one
+        chunk ahead: the next decode launch is queued on the current stream before the postnet window of the current chunk runs on
+        a side stream, on the SMs the decode kernel leaves idle.  `utt_ids` / `max_lens` as in inference() (no sorting, no work
+        stealing).  Closing the generator early leaves the module ready for the next call.
+
+        The stream's decode session lives in the module's workspace until the generator is exhausted or closed.  Any other call
+        on the module that runs in between (inference(), forward(), alignments(), encode(), another stream) takes that workspace
+        over; the open generator then raises RuntimeError on its next step instead of yielding frames of the other call.  Serve
+        concurrent requests from one module by batching them, or give each open stream its own module."""
+        lib = self._ensure_handle()
+        self.sync_weights()
+        B, S = phonemes.shape
+        max_len = int(max_len)
+        ids = None
+        if utt_ids is not None:
+            ids = torch.as_tensor([int(v) for v in utt_ids], dtype=torch.int32)
+            if ids.tolist() == list(range(int(ids[0]), int(ids[0]) + B)):
+                utt_offset, ids = int(ids[0]), None
+        sched = StreamSchedule(chunk_frames, postnet_halo(self.cfg), max_len)
+        dev = self.device
+        to_host = not phonemes.is_cuda
+        ph = phonemes.to(dev, torch.int64).contiguous()
+        pl = phoneme_lens.to(dev, torch.int32).contiguous()
+        mlens_d = None if max_lens is None else torch.as_tensor(max_lens).to(dev, torch.int32).clamp(1, max_len).contiguous()
+        ids_d = None if ids is None else ids.to(dev)
+        ws = self._workspace(B, S, max_len)
+        ws_use = self._ws_uses
+        if getattr(self, "_side_stream", None) is None:
+            self._side_stream = torch.cuda.Stream(dev)
+        side, cur = self._side_stream, torch.cuda.current_stream(dev)
+        stream, side_ptr = self._stream(), C.c_void_p(side.cuda_stream)
+        h, wsp = self._handle, ws.data_ptr()
+        self._check(lib.tts_decode_begin(h, wsp, B, S, max_len, int(seed), int(utt_offset), stream), "tts_decode_begin")
+        if ids_d is not None or mlens_d is not None:
+            self._check(lib.tts_decode_set_batch(h, wsp, ids_d.data_ptr() if ids_d is not None else None,
+                                                 mlens_d.data_ptr() if mlens_d is not None else None, 0, stream), "tts_decode_set_batch")
+        self._check(lib.tts_encode(h, wsp, ph.data_ptr(), pl.data_ptr(), B, S, max_len, None, stream), "tts_encode")
+        nbytes = lib.tts_stream_scratch_bytes(h, B, sched.max_emit_frames())
+        with torch.cuda.stream(side):
+            scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        self._check(lib.tts_decode_steps(h, wsp, sched.first_steps(), stream), "tts_decode_steps")
+        td, nf = C.c_int(0), C.c_int(0)
+        while True:
+            if self._ws_uses != ws_use:
+                raise RuntimeError("inference_stream(): another call on this module took its workspace and decode session "
+                                   "between two chunks; the stream cannot continue")
+            self._check(lib.tts_decode_status(h, wsp, C.byref(td), C.byref(nf), stream), "tts_decode_status")
+            ended = nf.value >= B or td.value >= max_len
+            steps, rng = sched.after_status(td.value, ended)
+            if steps:                                      # decode chunk k + 1 is queued before the postnet of chunk k
+                self._check(lib.tts_decode_steps(h, wsp, steps, stream), "tts_decode_steps")
+            if rng is not None:
+                t0, t1 = rng
+                n = t1 - t0
+                with torch.cuda.stream(side):
+                    ma = torch.empty(B, n, 80, device=dev); st = torch.empty(B, n, device=dev)
+                    ln = torch.empty(B, dtype=torch.int32, device=dev)
+                    if self.profile_events:
+                        ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+                        ev[0].record(side)
+                    self._check(lib.tts_decode_emit(h, wsp, scratch.data_ptr(), nbytes, t0, t1, ma.data_ptr(), st.data_ptr(),
+                                                    ln.data_ptr(), None, side_ptr), "tts_decode_emit")
+                    if self.profile_events:
+                        ev[1].record(side)
+                    fin = ln >= 0
+                    nv = torch.where(fin, (ln - t0).clamp(0, n), torch.full_like(ln, n))
+                    out = (ma, st, nv, fin)
+                    if to_host:                            # copied on the side stream: the next decode launch keeps running
+                        out = tuple(t.cpu() for t in out)
+                side.synchronize()
+                if self.profile_events:
+                    self.emit_ms.append(ev[0].elapsed_time(ev[1]))
+                if not to_host:
+                    for t in out:                          # allocated on the side stream, consumed on the caller's
+                        t.record_stream(cur)
+                yield StreamChunk(t0, *out)
+            if ended:
+                return
 
     def phase_timestamps(self, n_steps: int) -> torch.Tensor:
         """[n_steps, n_phases] int64 ns stamps of the last persistent decode (option decode_timestamps = 1)."""
