@@ -368,8 +368,8 @@ int tr_conv_bwd(TrCtx& c, const TrConv& cv, const TD* dout, int ldd, const float
     return 0;
 }
 
-// The training step in three parts (tts_train_step runs all three; the module's autograd bridge -- tts_train_forward /
-// tts_train_backward -- runs the first and, with the caller's output gradients, the third).
+// The training step in three parts: forward, loss, backward (tts_train_step runs all three through train_forward_backward; the
+// module's autograd bridge -- tts_train_forward / tts_train_backward -- runs the first and, with the caller's output gradients, the third).
 // ---- train-mode forward: every activation the backward pass needs stays in the workspace
 int train_forward(TrCtx& c) {
     TtsHandle* h = c.h; TtsTrain* t = c.t; TrWs& w = c.w; cudaStream_t st = c.st;
@@ -377,7 +377,6 @@ int train_forward(TrCtx& c) {
     const float eps = h->cfg.ln_eps;
     const int* plens = w.plens; const int* mlens = w.mlens;
     const int64_t* ph = w.ph_in; const float* mels = w.mels_in;
-    (void)eps; (void)mels;
     // ================================================================ forward (train mode)
     embed_kernel<<<(Me + 3) / 4, 256, 0, st>>>(ph, plens, t->mats[t->embed].fwd, w.e[0], B, S, h->cfg.n_vocab);
     ++launch_counter();
@@ -461,28 +460,12 @@ int train_forward(TrCtx& c) {
     TRL(cudaGetLastError());
     return 0;
 }
-// ---- loss P13 and its gradient with respect to (mel_before, mel_after, stop_logits) -> w.dbefore / w.dafter / w.dstop
-int train_loss(TrCtx& c, float* loss_out, float pos_weight) {
-    TtsHandle* h = c.h; TtsTrain* t = c.t; TrWs& w = c.w; cudaStream_t st = c.st;
-    const int B = c.B, S = c.S, T = c.T, Me = B * S, Md = B * T;
-    const float eps = h->cfg.ln_eps;
-    const int* plens = w.plens; const int* mlens = w.mlens;
-    const int64_t* ph = w.ph_in; const float* mels = w.mels_in;
-    (void)h; (void)t; (void)S; (void)Me; (void)eps; (void)plens; (void)ph;
-    // ================================================================ loss (P13) and its gradient
-    (void)Md;
-    TRL(launch_loss(w.mel_before, w.mel_after, w.stop, mels, mlens, B, T, pos_weight, w.acc, w.dbefore, w.dafter, w.dstop, loss_out, st));
-
-    return 0;
-}
 // ---- backward from the output gradients in w.dbefore [Md][80], w.dafter [Md][80], w.dstop [Md] (fp32) into the flat gradient buffer
 int train_backward(TrCtx& c) {
     TtsHandle* h = c.h; TtsTrain* t = c.t; TrWs& w = c.w; cudaStream_t st = c.st;
     const int B = c.B, S = c.S, T = c.T, Me = B * S, Md = B * T;
-    const float eps = h->cfg.ln_eps;
     const int* plens = w.plens; const int* mlens = w.mlens;
-    const int64_t* ph = w.ph_in; const float* mels = w.mels_in;
-    (void)mels;
+    const int64_t* ph = w.ph_in;
     TRL(cudaMemsetAsync(c.G, 0, t->n * 4, st));
     // ================================================================ backward
     // postnet: d mel_after flows into conv 4 .. 0
@@ -604,9 +587,11 @@ int train_backward(TrCtx& c) {
 
 int train_forward_backward(TrCtx& c, float* loss_out, float pos_weight) {
     int r = train_forward(c);
-    if (!r) r = train_loss(c, loss_out, pos_weight);
-    if (!r) r = train_backward(c);
-    return r;
+    if (r) return r;
+    // loss P13 and its gradient with respect to (mel_before, mel_after, stop_logits) -> w.dbefore / w.dafter / w.dstop
+    const TrWs& w = c.w;
+    TRL(launch_loss(w.mel_before, w.mel_after, w.stop, w.mels_in, w.mlens, c.B, c.T, pos_weight, w.acc, w.dbefore, w.dafter, w.dstop, loss_out, c.st));
+    return train_backward(c);
 }
 
 __global__ void set_u64_kernel(uint64_t* p, uint64_t v) { *p = v; }

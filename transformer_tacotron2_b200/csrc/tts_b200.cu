@@ -25,63 +25,7 @@
 
 using namespace tts;
 
-struct TtsTrain;
-// ------------------------------------------------------------------------------------------------
-struct TtsHandle {
-    TtsConfig cfg;
-    int device = 0, num_sms = 0;
-    std::string err;
-    std::map<std::string, std::vector<float>> staged;
-    bool finalized = false;
-    int decode_timestamps = 0, decode_debug = 0;
-    int cluster_group = 0;                                            // utterances per cluster (1..8); 0 = auto
-    int cluster_ok = -1, max_clusters = 0;                            // probed lazily
-    unsigned char* cl_wpack = nullptr;                                // [16][CLW_RANK_BYTES] (own allocation)
-    ClusterParams cparams;
-    unsigned char* arena = nullptr; size_t arena_bytes = 0;
-    // ---- device weights (pointers into arena)
-    bf16* embed = nullptr;
-    bf16* enc_conv_w[3] = {}; float* enc_conv_b[3] = {};
-    bf16* enc_proj_w = nullptr; float* enc_proj_b = nullptr;
-    float enc_alpha = 1.f, dec_alpha = 1.f;
-    struct EncLayer { bf16 *wqkv, *wo, *w1, *w2; float *bqkv, *bo, *b1, *b2, *ln1g, *ln1b, *ln2g, *ln2b; } enc[6];
-    bf16* ckv_w = nullptr; float* ckv_b = nullptr;                   // [6*1024][512]
-    struct DecLayer {
-        bf16 *wqkv, *wo, *wq2, *wo2, *w1, *w2;                       // row-major (teacher-forced GEMMs)
-        float *bqkv, *bo, *bq2, *bo2, *b1, *b2, *ln1g, *ln1b, *ln2g, *ln2b, *ln3g, *ln3b;
-    } dec[6];
-    bf16 *pre_fc1, *pre_fc2, *pre_proj, *head_w;
-    float *pre_b1, *pre_b2, *pre_bp, *head_b;
-    bf16* post_w[5] = {}; float* post_b[5] = {};
-    float* pe = nullptr;
-    // ---- decode session
-    bool dec_ids = false, dec_tlens = false, dec_steal = false;       // tts_decode_set_batch
-    bool dec_active = false; int dec_B = 0, dec_S = 0, dec_T = 0, dec_t = 0; uint64_t dec_seed = 0; int dec_utt0 = 0;
-    int* h_status = nullptr;                                          // pinned: t_done, n_finished
-    int dec_t_status = -1, dec_frontier = 0;                          // last tts_decode_status: frames decoded, frames final (-1: none yet)
-    TtsTrain* train = nullptr;                                        // training state (train.cuh), built by tts_train_begin
-    int train_graph = 1;                                              // replay the train step from a CUDA graph (option "train_graph")
-};
-
-#define CK(call)                                                                                     \
-    do {                                                                                             \
-        cudaError_t e_ = (call);                                                                     \
-        if (e_ != cudaSuccess) {                                                                     \
-            h->err = std::string(#call) + ": " + cudaGetErrorString(e_);                             \
-            return (int)e_;                                                                          \
-        }                                                                                            \
-    } while (0)
-#define FAIL(code, msg) do { h->err = (msg); return (code); } while (0)
-// makes the handle's device current for the rest of the entry point and restores the caller's device on return
-#define DEV_GUARD(h) DeviceGuard dev_guard_((h)->device); CK(dev_guard_.err)
-
 static inline size_t align_up(size_t x, size_t a = 256) { return (x + a - 1) / a * a; }
-static inline uint16_t f2bf(float f) {                                // round-to-nearest-even, as __float2bfloat16_rn
-    uint32_t u; memcpy(&u, &f, 4);
-    if ((u & 0x7fffffffu) > 0x7f800000u) return (uint16_t)((u >> 16) | 0x40);
-    u += 0x7fffu + ((u >> 16) & 1u);
-    return (uint16_t)(u >> 16);
-}
 
 // ------------------------------------------------------------------------------------------------
 // Workspace layout
@@ -117,6 +61,64 @@ struct Ws {
     }
 };
 template <typename T> static inline T* wsp(void* ws, size_t off) { return reinterpret_cast<T*>(reinterpret_cast<unsigned char*>(ws) + off); }
+
+struct TtsTrain;
+// ------------------------------------------------------------------------------------------------
+struct TtsHandle {
+    TtsConfig cfg;
+    int device = 0, num_sms = 0;
+    std::string err;
+    std::map<std::string, std::vector<float>> staged;
+    bool finalized = false;
+    int decode_timestamps = 0, decode_debug = 0;
+    int cluster_group = 0;                                            // utterances per cluster (1..8); 0 = auto
+    int cluster_ok = -1, max_clusters = 0;                            // probed lazily
+    unsigned char* cl_wpack = nullptr;                                // [16][CLW_RANK_BYTES] (own allocation)
+    unsigned char* arena = nullptr; size_t arena_bytes = 0;
+    // ---- device weights (pointers into arena)
+    bf16* embed = nullptr;
+    bf16* enc_conv_w[3] = {}; float* enc_conv_b[3] = {};
+    bf16* enc_proj_w = nullptr; float* enc_proj_b = nullptr;
+    float enc_alpha = 1.f, dec_alpha = 1.f;
+    struct EncLayer { bf16 *wqkv, *wo, *w1, *w2; float *bqkv, *bo, *b1, *b2, *ln1g, *ln1b, *ln2g, *ln2b; } enc[6];
+    bf16* ckv_w = nullptr; float* ckv_b = nullptr;                   // [6*1024][512]
+    struct DecLayer {
+        bf16 *wqkv, *wo, *wq2, *wo2, *w1, *w2;                       // row-major (teacher-forced GEMMs)
+        float *bqkv, *bo, *bq2, *bo2, *b1, *b2, *ln1g, *ln1b, *ln2g, *ln2b, *ln3g, *ln3b;
+    } dec[6];
+    bf16 *pre_fc1, *pre_fc2, *pre_proj, *head_w;
+    float *pre_b1, *pre_b2, *pre_bp, *head_b;
+    bf16* post_w[5] = {}; float* post_b[5] = {};
+    float* pe = nullptr;
+    // ---- decode session: set up by tts_decode_begin, ended by the next tts_decode_begin or tts_finalize_weights
+    struct DecodeSession {
+        bool active = false; int B = 0, S = 0, T = 0, t = 0;          // T = max_len; t: frames decoded (upper bound until tts_decode_status)
+        int t_status = -1, frontier = 0;                              // last tts_decode_status: frames decoded, frames final (-1: none yet)
+        Ws L; ClusterParams cp;                                       // workspace layout of (B, S, T); decode kernel arguments
+    } session;
+    int* h_status = nullptr;                                          // pinned: t_done, n_finished
+    TtsTrain* train = nullptr;                                        // training state (train.cuh), built by tts_train_begin
+    int train_graph = 1;                                              // replay the train step from a CUDA graph (option "train_graph")
+};
+
+#define CK(call)                                                                                     \
+    do {                                                                                             \
+        cudaError_t e_ = (call);                                                                     \
+        if (e_ != cudaSuccess) {                                                                     \
+            h->err = std::string(#call) + ": " + cudaGetErrorString(e_);                             \
+            return (int)e_;                                                                          \
+        }                                                                                            \
+    } while (0)
+#define FAIL(code, msg) do { h->err = (msg); return (code); } while (0)
+// makes the handle's device current for the rest of the entry point and restores the caller's device on return
+#define DEV_GUARD(h) DeviceGuard dev_guard_((h)->device); CK(dev_guard_.err)
+
+static inline uint16_t f2bf(float f) {                                // round-to-nearest-even, as __float2bfloat16_rn
+    uint32_t u; memcpy(&u, &f, 4);
+    if ((u & 0x7fffffffu) > 0x7f800000u) return (uint16_t)((u >> 16) | 0x40);
+    u += 0x7fffu + ((u >> 16) & 1u);
+    return (uint16_t)(u >> 16);
+}
 
 // ------------------------------------------------------------------------------------------------
 extern "C" const char* tts_version(void) { return "tts_b200 0.1 sm_100a"; }
@@ -164,7 +166,7 @@ extern "C" int tts_set_option(TtsHandle* h, const char* key, int64_t value) {
     if (!strcmp(key, "decode_debug")) { if (value < 0 || value > 8) FAIL(TTS_E_ARG, "decode_debug: 0 off, 1 + rank of the dumping CTA"); h->decode_debug = (int)value; return 0; }
     if (!strcmp(key, "cluster_group")) { if (value < 0 || value > CL_G) FAIL(TTS_E_ARG, "cluster_group must be 0 (auto) or 1..5"); h->cluster_group = (int)value; return 0; }
     if (!strcmp(key, "train_graph")) { h->train_graph = value ? 1 : 0; return 0; }
-    if (!strcmp(key, "print_info")) { fprintf(stderr, "[tts_b200] sms=%d cluster_ok=%d max_clusters=%d group=%d ngroups=%d\n", h->num_sms, h->cluster_ok, h->max_clusters, h->cparams.G, h->cparams.ngroups); return 0; }
+    if (!strcmp(key, "print_info")) { fprintf(stderr, "[tts_b200] sms=%d cluster_ok=%d max_clusters=%d group=%d ngroups=%d\n", h->num_sms, h->cluster_ok, h->max_clusters, h->session.cp.G, h->session.cp.ngroups); return 0; }
     FAIL(TTS_E_ARG, std::string("unknown option ") + key);
 }
 
@@ -403,7 +405,7 @@ extern "C" int tts_finalize_weights(TtsHandle* h) {
     CK(cudaMemcpy(h->arena, ar.host.data(), ar.host.size(), cudaMemcpyHostToDevice));
     for (auto& f : fixes) *f.dst = h->arena + f.off;
     CK(cudaDeviceSynchronize());
-    h->dec_active = false;                                            // a decode session holds pointers into the old arena
+    h->session.active = false;                                        // a decode session holds pointers into the old arena
     h->finalized = true;                                              // (the staged fp32 copies stay: tts_train_begin builds the master from them)
     return 0;
 }
@@ -441,8 +443,6 @@ cudaError_t layernorm(const float* x, const float* g, const float* b, bf16* o16,
 }
 }  // namespace
 
-#define CKL(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { h->err = std::string(#call) + ": " + cudaGetErrorString(e_); return (int)e_; } } while (0)
-
 // Encoder (C1-C4) + hoisted cross-K/V projection.  Result: memory in ws.x (bf16 [B*S][512]).
 static int run_encoder(TtsHandle* h, void* ws, const Ws& L, const int64_t* ph, const int* plens, int B, int S, bool v_blocked, cudaStream_t st) {
     const int M = B * S;
@@ -450,43 +450,43 @@ static int run_encoder(TtsHandle* h, void* ws, const Ws& L, const int64_t* ph, c
     float* y = wsp<float>(ws, L.y);
     embed_kernel<<<(M + 3) / 4, 256, 0, st>>>(ph, plens, h->embed, x, B, S, h->cfg.n_vocab);
     ++launch_counter();
-    CKL(cudaGetLastError());
+    CK(cudaGetLastError());
     for (int i = 0; i < 3; ++i) {                                      // conv k5 + folded BN + ReLU + length mask
         GemmParams p = gp(x, 512, h->enc_conv_w[i], 512, M, 512, 512);
         p.taps = 5; p.T = S; p.bias = h->enc_conv_b[i]; p.act = ACT_RELU; p.lens = plens; p.out_bf16 = x2; p.ldo = 512;
-        CKL(launch_gemm_tc(p, st));
+        CK(launch_gemm_tc(p, st));
         std::swap(x, x2);
     }
     {   // linear + alpha * PE
         GemmParams p = gp(x, 512, h->enc_proj_w, 512, M, 512, 512);
         p.T = S; p.bias = h->enc_proj_b; p.pe = h->pe; p.alpha = h->enc_alpha; p.out_bf16 = x2; p.ldo = 512;
-        CKL(launch_gemm_tc(p, st));
+        CK(launch_gemm_tc(p, st));
         std::swap(x, x2);
     }
     for (int l = 0; l < 6; ++l) {
         auto& W = h->enc[l];
         GemmParams p = gp(x, 512, W.wqkv, 512, M, 1536, 512); p.bias = W.bqkv; p.out_bf16 = wide; p.ldo = 1536;
-        CKL(launch_gemm_tc(p, st));
+        CK(launch_gemm_tc(p, st));
         AttnParams at = ap_packed(wide, 1536, wide + 512, 1536, wide + 1024, 1536, a, 512, B, S, S, plens, 0);
-        CKL(launch_flash_attn_tc(at, st));
+        CK(launch_flash_attn_tc(at, st));
         p = gp(a, 512, W.wo, 512, M, 512, 512); p.bias = W.bo; p.resid_bf16 = x; p.ldr = 512; p.out_f32 = y; p.ldo = 512;
-        CKL(launch_gemm_tc(p, st));
-        CKL(layernorm(y, W.ln1g, W.ln1b, x, nullptr, M, h->cfg.ln_eps, st));
+        CK(launch_gemm_tc(p, st));
+        CK(layernorm(y, W.ln1g, W.ln1b, x, nullptr, M, h->cfg.ln_eps, st));
         p = gp(x, 512, W.w1, 512, M, 2048, 512); p.bias = W.b1; p.act = ACT_RELU; p.out_bf16 = wide; p.ldo = 2048;
-        CKL(launch_gemm_tc(p, st));
+        CK(launch_gemm_tc(p, st));
         p = gp(wide, 2048, W.w2, 2048, M, 512, 2048); p.bias = W.b2; p.resid_bf16 = x; p.ldr = 512; p.out_f32 = y; p.ldo = 512;
-        CKL(launch_gemm_tc(p, st));
-        CKL(layernorm(y, W.ln2g, W.ln2b, x, nullptr, M, h->cfg.ln_eps, st));
+        CK(launch_gemm_tc(p, st));
+        CK(layernorm(y, W.ln2g, W.ln2b, x, nullptr, M, h->cfg.ln_eps, st));
     }
     if (x != wsp<bf16>(ws, L.x)) {                                     // keep memory in ws.x
-        CKL(cudaMemcpyAsync(wsp<bf16>(ws, L.x), x, (size_t)M * 512 * 2, cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(wsp<bf16>(ws, L.x), x, (size_t)M * 512 * 2, cudaMemcpyDeviceToDevice, st));
     }
     {   // cross K/V of all decoder layers -> cache [6][2][B][H][S][64]
         GemmParams p = gp(wsp<bf16>(ws, L.x), 512, h->ckv_w, 512, M, 6 * 1024, 512);
         // rows past S of every (layer, b, h) stay zero: the decode kernel copies the cache at 16-row granularity
-        CKL(cudaMemsetAsync(wsp<bf16>(ws, L.cross_kv), 0, L.cross_kv_bytes, st));
+        CK(cudaMemsetAsync(wsp<bf16>(ws, L.cross_kv), 0, L.cross_kv_bytes, st));
         p.T = S; p.B = B; p.Lpad = v_blocked ? L.nblk_cross * KV_BLOCK_ROWS : L.Spad; p.bias = h->ckv_b; p.scatter = v_blocked ? SC_CROSS_KV_VT : SC_CROSS_KV; p.out_bf16 = wsp<bf16>(ws, L.cross_kv);
-        CKL(launch_gemm_tc(p, st));
+        CK(launch_gemm_tc(p, st));
     }
     return 0;
 }
@@ -503,7 +503,7 @@ static int run_postnet_rows(TtsHandle* h, const bf16* in16, const float* resid32
         p.taps = 5; p.T = T; p.bias = h->post_b[i]; p.lens = mlens; p.max_ctas = max_ctas;
         if (i < 4) { p.act = ACT_TANH; p.out_bf16 = x; p.ldo = 512; }
         else { p.resid_f32 = resid32; p.ldr = 80; p.out_f32 = mel_after; p.ldo = 80; }
-        CKL(launch_gemm_tc(p, st));
+        CK(launch_gemm_tc(p, st));
         in = x; std::swap(x, x2);
     }
     return 0;
@@ -541,10 +541,10 @@ extern "C" int tts_decode_begin(TtsHandle* h, void* ws, int B, int S, int max_le
     if (max_len > h->cfg.max_pos) FAIL(TTS_E_ARG, "max_len exceeds max_pos");
     DEV_GUARD(h);
     cudaStream_t st = (cudaStream_t)stream;
-    const Ws L = Ws::make(B, S, max_len);
-    h->dec_ids = h->dec_tlens = h->dec_steal = false;
-    h->dec_active = true; h->dec_B = B; h->dec_S = S; h->dec_T = max_len; h->dec_t = 0; h->dec_seed = seed; h->dec_utt0 = utt_offset;
-    h->dec_t_status = -1; h->dec_frontier = 0;
+    auto& ds = h->session;
+    ds.active = true; ds.B = B; ds.S = S; ds.T = max_len; ds.t = 0; ds.t_status = -1; ds.frontier = 0;
+    ds.L = Ws::make(B, S, max_len);
+    const Ws& L = ds.L;
     init_decode_state_kernel<<<(std::max(B, 4) + 255) / 256, 256, 0, st>>>(wsp<int>(ws, L.lens), wsp<int>(ws, L.finished),
                                                                           wsp<int>(ws, L.scalars), B, max_len);
     ++launch_counter();
@@ -568,7 +568,7 @@ extern "C" int tts_decode_begin(TtsHandle* h, void* ws, int B, int S, int max_le
     }
     if (h->cluster_ok != 1) FAIL(TTS_E_DEVICE, "device cannot co-schedule an 8-CTA cluster of the decode kernel");
 
-    ClusterParams& cp = h->cparams; memset(&cp, 0, sizeof(cp));
+    ClusterParams& cp = ds.cp; memset(&cp, 0, sizeof(cp));
     cp.B = B; cp.Tmax = max_len; cp.S = S; cp.nblk_self = L.nblk_self; cp.nblk_cross = L.nblk_cross;
     // utterances per cluster: as few as the co-resident cluster count allows (more SMs stream K/V), at most 8
     cp.G = h->cluster_group > 0 ? std::min(CL_G, h->cluster_group)
@@ -588,32 +588,28 @@ extern "C" int tts_decode_begin(TtsHandle* h, void* ws, int B, int S, int max_le
 
 extern "C" int tts_decode_steps(TtsHandle* h, void* ws, int n_steps, void* stream) {
     if (!h || !ws || n_steps < 0) return TTS_E_ARG;
-    if (!h->dec_active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
+    auto& ds = h->session;
+    if (!ds.active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
     DEV_GUARD(h);
     cudaStream_t st = (cudaStream_t)stream;
-    n_steps = std::min(n_steps, h->dec_T - h->dec_t);
+    n_steps = std::min(n_steps, ds.T - ds.t);
     if (n_steps <= 0) return 0;
+    ClusterParams& cp = ds.cp;
     cudaLaunchConfig_t cfg; memset(&cfg, 0, sizeof(cfg));
-    const int ncl = std::min(h->cparams.ngroups, h->max_clusters);
+    const int ncl = std::min(cp.ngroups, h->max_clusters);
     cfg.gridDim = dim3(CL_SIZE * ncl); cfg.blockDim = dim3(CL_THREADS); cfg.dynamicSmemBytes = CL_SMEM_BYTES; cfg.stream = st;
     cudaLaunchAttribute at[1]; at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = CL_SIZE; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
-    h->cparams.ts = h->decode_timestamps ? wsp<unsigned long long>(ws, Ws::make(h->dec_B, h->dec_S, h->dec_T).ts) : nullptr;
+    cp.ts = h->decode_timestamps ? wsp<unsigned long long>(ws, ds.L.ts) : nullptr;
+    if (cp.group_queue) CK(cudaMemsetAsync(cp.group_queue, 0, 4, st));  // work stealing: every launch starts from a fresh queue
     // (the debug dump lands in the `wide` activation buffer, idle during the decode loop: >= B * 2048 * 2 bytes per row of S/T)
-    {
-        const Ws L = Ws::make(h->dec_B, h->dec_S, h->dec_T);
-        h->cparams.utt_ids = h->dec_ids ? wsp<int>(ws, L.utt_ids) : nullptr;
-        h->cparams.tlens = h->dec_tlens ? wsp<int>(ws, L.tlens) : nullptr;
-        h->cparams.group_queue = h->dec_steal ? wsp<int>(ws, L.scalars) + 1 : nullptr;
-        if (h->dec_steal) CK(cudaMemsetAsync(wsp<int>(ws, L.scalars) + 1, 0, 4, st));
-    }
-    h->cparams.dbg_rank = h->decode_debug - 1;
-    h->cparams.dbg = h->decode_debug ? wsp<float>(ws, Ws::make(h->dec_B, h->dec_S, h->dec_T).wide) : nullptr;
-    if (h->cparams.ts || h->cparams.dbg) CK(cudaLaunchKernelEx(&cfg, decode_cluster_kernel<true>, h->cparams, h->dec_t, n_steps));
-    else CK(cudaLaunchKernelEx(&cfg, decode_cluster_kernel<false>, h->cparams, h->dec_t, n_steps));
+    cp.dbg_rank = h->decode_debug - 1;
+    cp.dbg = h->decode_debug ? wsp<float>(ws, ds.L.wide) : nullptr;
+    if (cp.ts || cp.dbg) CK(cudaLaunchKernelEx(&cfg, decode_cluster_kernel<true>, cp, ds.t, n_steps));
+    else CK(cudaLaunchKernelEx(&cfg, decode_cluster_kernel<false>, cp, ds.t, n_steps));
     ++launch_counter();
-    h->dec_t += n_steps;                                                // upper bound; tts_decode_status refines it
+    ds.t += n_steps;                                                    // upper bound; tts_decode_status refines it
     return 0;
 }
 
@@ -622,62 +618,66 @@ static int postnet_halo(const TtsHandle* h) { return h->cfg.postnet_layers * (h-
 
 extern "C" int tts_decode_status(TtsHandle* h, void* ws, int* t_done, int* n_finished, void* stream) {
     if (!h || !ws) return TTS_E_ARG;
-    if (!h->dec_active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
+    auto& ds = h->session;
+    if (!ds.active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
     DEV_GUARD(h);
     cudaStream_t st = (cudaStream_t)stream;
-    CK(cudaMemcpyAsync(h->h_status, h->cparams.n_finished, 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(h->h_status, ds.cp.n_finished, 4, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     const int nf = h->h_status[0];
-    if (nf >= h->dec_B) {                                 // every utterance fired: the frames run = the longest utterance
-        std::vector<int> lens(h->dec_B);
-        CK(cudaMemcpyAsync(lens.data(), h->cparams.lens, (size_t)h->dec_B * 4, cudaMemcpyDeviceToHost, st));
+    if (nf >= ds.B) {                                     // every utterance fired: the frames run = the longest utterance
+        std::vector<int> lens(ds.B);
+        CK(cudaMemcpyAsync(lens.data(), ds.cp.lens, (size_t)ds.B * 4, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
         int mx = 0; for (int v : lens) mx = std::max(mx, v);
-        h->dec_t = mx;
+        ds.t = mx;
     }
     // tts_decode_emit's frontier: a frame's postnet output is final once the postnet's halo past it is decoded, or once the session
     // has ended (every utterance stopped, or max_len reached).  Only this call moves it; tts_decode_steps does not.
-    const bool ended = nf >= h->dec_B || h->dec_t >= h->dec_T;
-    h->dec_t_status = h->dec_t;
-    h->dec_frontier = ended ? h->dec_t : std::max(0, h->dec_t - postnet_halo(h));
+    const bool ended = nf >= ds.B || ds.t >= ds.T;
+    ds.t_status = ds.t;
+    ds.frontier = ended ? ds.t : std::max(0, ds.t - postnet_halo(h));
     if (n_finished) *n_finished = nf;
-    if (t_done) *t_done = h->dec_t;
+    if (t_done) *t_done = ds.t;
     return 0;
 }
 
 extern "C" int tts_decode_set_batch(TtsHandle* h, void* ws, const int32_t* utt_ids, const int32_t* max_lens, int work_stealing, void* stream) {
     if (!h || !ws) return TTS_E_ARG;
-    if (!h->dec_active || h->dec_t != 0) FAIL(TTS_E_STATE, "tts_decode_set_batch belongs between tts_decode_begin and the first tts_decode_steps");
+    auto& ds = h->session;
+    if (!ds.active || ds.t != 0) FAIL(TTS_E_STATE, "tts_decode_set_batch belongs between tts_decode_begin and the first tts_decode_steps");
     DEV_GUARD(h);
-    const Ws L = Ws::make(h->dec_B, h->dec_S, h->dec_T);
     cudaStream_t st = (cudaStream_t)stream;
-    if (utt_ids) CK(cudaMemcpyAsync(wsp<int>(ws, L.utt_ids), utt_ids, (size_t)h->dec_B * 4, cudaMemcpyDeviceToDevice, st));
-    if (max_lens) CK(cudaMemcpyAsync(wsp<int>(ws, L.tlens), max_lens, (size_t)h->dec_B * 4, cudaMemcpyDeviceToDevice, st));
-    h->dec_ids = utt_ids != nullptr; h->dec_tlens = max_lens != nullptr; h->dec_steal = work_stealing != 0;
+    int* ids = utt_ids ? wsp<int>(ws, ds.L.utt_ids) : nullptr;
+    int* tlens = max_lens ? wsp<int>(ws, ds.L.tlens) : nullptr;
+    if (ids) CK(cudaMemcpyAsync(ids, utt_ids, (size_t)ds.B * 4, cudaMemcpyDeviceToDevice, st));
+    if (tlens) CK(cudaMemcpyAsync(tlens, max_lens, (size_t)ds.B * 4, cudaMemcpyDeviceToDevice, st));
+    ds.cp.utt_ids = ids; ds.cp.tlens = tlens;
+    ds.cp.group_queue = work_stealing ? wsp<int>(ws, ds.L.scalars) + 1 : nullptr;
     return 0;
 }
 
 extern "C" int tts_decode_set_frame(TtsHandle* h, void* ws, int t, const float* frames, void* stream) {
     if (!h || !ws || !frames) return TTS_E_ARG;
-    if (!h->dec_active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
-    if (t < 0 || t >= h->dec_t) FAIL(TTS_E_ARG, "frame index must lie in [0, frames decoded so far)");
+    const auto& ds = h->session;
+    if (!ds.active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
+    if (t < 0 || t >= ds.t) FAIL(TTS_E_ARG, "frame index must lie in [0, frames decoded so far)");
     DEV_GUARD(h);
-    const Ws L = Ws::make(h->dec_B, h->dec_S, h->dec_T);
-    CK(cudaMemcpy2DAsync(wsp<float>(ws, L.mel_before) + (size_t)t * 80, (size_t)h->dec_T * 80 * 4, frames, 80 * 4, 80 * 4, (size_t)h->dec_B,
+    CK(cudaMemcpy2DAsync(wsp<float>(ws, ds.L.mel_before) + (size_t)t * 80, (size_t)ds.T * 80 * 4, frames, 80 * 4, 80 * 4, (size_t)ds.B,
                          cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     return 0;
 }
 
 extern "C" int tts_decode_get_frame(TtsHandle* h, void* ws, int t, float* frames, float* stop_logits, void* stream) {
     if (!h || !ws || !frames) return TTS_E_ARG;
-    if (!h->dec_active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
-    if (t < 0 || t >= h->dec_t) FAIL(TTS_E_ARG, "frame index must lie in [0, frames decoded so far)");
+    const auto& ds = h->session;
+    if (!ds.active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
+    if (t < 0 || t >= ds.t) FAIL(TTS_E_ARG, "frame index must lie in [0, frames decoded so far)");
     DEV_GUARD(h);
-    const Ws L = Ws::make(h->dec_B, h->dec_S, h->dec_T);
-    CK(cudaMemcpy2DAsync(frames, 80 * 4, wsp<float>(ws, L.mel_before) + (size_t)t * 80, (size_t)h->dec_T * 80 * 4, 80 * 4, (size_t)h->dec_B,
+    CK(cudaMemcpy2DAsync(frames, 80 * 4, wsp<float>(ws, ds.L.mel_before) + (size_t)t * 80, (size_t)ds.T * 80 * 4, 80 * 4, (size_t)ds.B,
                          cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     if (stop_logits)
-        CK(cudaMemcpy2DAsync(stop_logits, 4, wsp<float>(ws, L.stop_logits) + t, (size_t)h->dec_T * 4, 4, (size_t)h->dec_B, cudaMemcpyDeviceToDevice,
+        CK(cudaMemcpy2DAsync(stop_logits, 4, wsp<float>(ws, ds.L.stop_logits) + t, (size_t)ds.T * 4, 4, (size_t)ds.B, cudaMemcpyDeviceToDevice,
                              (cudaStream_t)stream));
     return 0;
 }
@@ -685,21 +685,22 @@ extern "C" int tts_decode_get_frame(TtsHandle* h, void* ws, int t, float* frames
 extern "C" int tts_decode_end(TtsHandle* h, void* ws, int T_out, float* mel_after, int32_t* mel_lens, float* stop_logits,
                               float* mel_before, void* stream) {
     if (!h || !ws || !mel_after || T_out <= 0) return TTS_E_ARG;
-    if (!h->dec_active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
-    if (T_out > h->dec_T) FAIL(TTS_E_ARG, "T_out exceeds max_len");
+    const auto& ds = h->session;
+    if (!ds.active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
+    if (T_out > ds.T) FAIL(TTS_E_ARG, "T_out exceeds max_len");
     DEV_GUARD(h);
     cudaStream_t st = (cudaStream_t)stream;
-    const int B = h->dec_B;
-    const Ws L = Ws::make(B, h->dec_S, h->dec_T);
+    const int B = ds.B;
+    const Ws& L = ds.L;
     const int* lens = wsp<int>(ws, L.lens);
     const int n = B * T_out * 24;
-    mel_to_bf16_kernel<<<(n + 255) / 256, 256, 0, st>>>(wsp<float>(ws, L.mel_before), h->dec_T, lens, 0,
+    mel_to_bf16_kernel<<<(n + 255) / 256, 256, 0, st>>>(wsp<float>(ws, L.mel_before), ds.T, lens, 0,
                                                         wsp<bf16>(ws, L.mel16), wsp<float>(ws, L.mel32), B, T_out);
     ++launch_counter();
     CK(cudaGetLastError());
     if (stop_logits || mel_lens) {
         float* so = stop_logits ? stop_logits : wsp<float>(ws, L.y);
-        finalize_stop_kernel<<<(std::max(B * T_out, B) + 255) / 256, 256, 0, st>>>(wsp<float>(ws, L.stop_logits), h->dec_T, lens, so, mel_lens, B, T_out);
+        finalize_stop_kernel<<<(std::max(B * T_out, B) + 255) / 256, 256, 0, st>>>(wsp<float>(ws, L.stop_logits), ds.T, lens, so, mel_lens, B, T_out);
         ++launch_counter();
         CK(cudaGetLastError());
     }
@@ -733,23 +734,24 @@ extern "C" size_t tts_stream_scratch_bytes(TtsHandle* h, int B, int max_frames) 
 extern "C" int tts_decode_emit(TtsHandle* h, void* ws, void* scratch, size_t scratch_bytes, int t_begin, int t_end, float* mel_after,
                                float* stop_logits, int32_t* mel_lens, float* mel_before, void* stream) {
     if (!h || !ws || !scratch || !mel_after || !stop_logits) return TTS_E_ARG;
-    if (!h->dec_active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
-    if (h->dec_t_status < 0) FAIL(TTS_E_STATE, "tts_decode_emit needs a tts_decode_status call first");
+    const auto& ds = h->session;
+    if (!ds.active) FAIL(TTS_E_STATE, "tts_decode_begin not called");
+    if (ds.t_status < 0) FAIL(TTS_E_STATE, "tts_decode_emit needs a tts_decode_status call first");
     if (t_begin < 0 || t_end <= t_begin) FAIL(TTS_E_ARG, "frame range must be non-empty and start at >= 0");
-    if (t_end > h->dec_frontier) FAIL(TTS_E_ARG, "t_end lies past the frontier of the last tts_decode_status");
-    const int halo = postnet_halo(h), B = h->dec_B, n = t_end - t_begin;
-    const int a = std::max(0, t_begin - halo), e = std::min(t_end + halo, h->dec_t_status), W = e - a;
+    if (t_end > ds.frontier) FAIL(TTS_E_ARG, "t_end lies past the frontier of the last tts_decode_status");
+    const int halo = postnet_halo(h), B = ds.B, n = t_end - t_begin;
+    const int a = std::max(0, t_begin - halo), e = std::min(t_end + halo, ds.t_status), W = e - a;
     const StreamScratch S = StreamScratch::make(B, W);
     if (S.total > scratch_bytes) FAIL(TTS_E_ARG, "scratch too small for this window (tts_stream_scratch_bytes)");
     // the decode kernel holds CL_SIZE SMs per co-resident cluster while it runs; the postnet GEMMs take only the others
-    const int max_ctas = h->num_sms - CL_SIZE * std::min(h->cparams.ngroups, h->max_clusters);
+    const int max_ctas = h->num_sms - CL_SIZE * std::min(ds.cp.ngroups, h->max_clusters);
     if (max_ctas < 1) FAIL(TTS_E_DEVICE, "no SM left beside the decode kernel");
     DEV_GUARD(h);
     cudaStream_t st = (cudaStream_t)stream;
-    const Ws L = Ws::make(B, h->dec_S, h->dec_T);
+    const Ws& L = ds.L;
     const int nthreads = std::max(B * W * 24, B * n);
-    stream_window_kernel<<<(nthreads + 255) / 256, 256, 0, st>>>(wsp<float>(ws, L.mel_before), wsp<float>(ws, L.stop_logits), h->dec_T,
-                                                                 wsp<int>(ws, L.lens), h->dec_t_status, a, W, t_begin, n,
+    stream_window_kernel<<<(nthreads + 255) / 256, 256, 0, st>>>(wsp<float>(ws, L.mel_before), wsp<float>(ws, L.stop_logits), ds.T,
+                                                                 wsp<int>(ws, L.lens), ds.t_status, a, W, t_begin, n,
                                                                  wsp<bf16>(scratch, S.in16), wsp<float>(scratch, S.res32),
                                                                  wsp<int>(scratch, S.wlens), stop_logits, mel_lens, B);
     ++launch_counter();
@@ -966,20 +968,20 @@ extern "C" int tts_forward_align(TtsHandle* h, void* ws, void* scratch, const in
 // profiling aid: copy the per-phase globaltimer stamps of the persistent decode kernel to the host.
 extern "C" int tts_debug_phase_timestamps(TtsHandle* h, void* ws, unsigned long long* out, int n_steps, void* stream) {
     if (!h || !ws || !out || n_steps <= 0) return TTS_E_ARG;
-    if (!h->dec_active || n_steps != h->dec_T) FAIL(TTS_E_STATE, "no decode session / n_steps must equal max_len");
-    const Ws L = Ws::make(h->dec_B, h->dec_S, h->dec_T);
-    CK(cudaMemcpyAsync(out, wsp<unsigned long long>(ws, L.ts), (size_t)(n_steps + 1) * CL_TS_COLS * 8, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+    const auto& ds = h->session;
+    if (!ds.active || n_steps != ds.T) FAIL(TTS_E_STATE, "no decode session / n_steps must equal max_len");
+    CK(cudaMemcpyAsync(out, wsp<unsigned long long>(ws, ds.L.ts), (size_t)(n_steps + 1) * CL_TS_COLS * 8, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
     CK(cudaStreamSynchronize((cudaStream_t)stream));
     return 52;
 }
 
 extern "C" int tts_debug_read_dump(TtsHandle* h, void* ws, int64_t offset, int64_t n, float* out_host, void* stream) {
     if (!h || !ws || !out_host || offset < 0 || n <= 0) return TTS_E_ARG;
-    if (!h->dec_active) FAIL(TTS_E_STATE, "no decode session");
-    const Ws L = Ws::make(h->dec_B, h->dec_S, h->dec_T);
-    const size_t cap = (size_t)h->dec_B * (size_t)std::max(h->dec_S, h->dec_T) * 2048 * 2 / 4;
+    const auto& ds = h->session;
+    if (!ds.active) FAIL(TTS_E_STATE, "no decode session");
+    const size_t cap = (size_t)ds.B * (size_t)std::max(ds.S, ds.T) * 2048 * 2 / 4;
     if ((size_t)(offset + n) > cap) FAIL(TTS_E_ARG, "dump range exceeds the debug buffer");
-    CK(cudaMemcpyAsync(out_host, wsp<float>(ws, L.wide) + offset, (size_t)n * 4, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+    CK(cudaMemcpyAsync(out_host, wsp<float>(ws, ds.L.wide) + offset, (size_t)n * 4, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
     CK(cudaStreamSynchronize((cudaStream_t)stream));
     return 0;
 }
@@ -1199,26 +1201,43 @@ extern "C" size_t tts_train_workspace_bytes(TtsHandle* h, int B, int S, int T) {
     if (!h || B <= 0 || S <= 0 || T <= 0) return 0;
     return TrWs::make(nullptr, B, S, T).total;
 }
-extern "C" int tts_train_step(TtsHandle* h, void* ws, const int64_t* phonemes, const int32_t* phoneme_lens, const float* mels, const int32_t* mel_lens,
-                              int B, int S, int T, uint64_t seed, int utt_offset, double p_residual, float pos_weight, float* loss_out, void* stream) {
-    if (!h || !ws || !phonemes || !phoneme_lens || !mels || !mel_lens || !loss_out || B <= 0 || S <= 0 || T <= 0) return TTS_E_ARG;
-    if (!h->train) FAIL(TTS_E_STATE, "tts_train_begin has not been called");
-    if (S > h->cfg.max_pos || T > h->cfg.max_pos) FAIL(TTS_E_ARG, "sequence exceeds max_pos");
-    if (p_residual < 0.0 || p_residual >= 1.0) FAIL(TTS_E_ARG, "p_residual out of range");
-    DEV_GUARD(h);
+namespace {
+// context of one training call: workspace views, dropout threshold / scale, flat parameter and gradient buffers
+TrCtx train_ctx(TtsHandle* h, void* ws, int B, int S, int T, int utt_offset, double p_residual, cudaStream_t st) {
     TrCtx c;
     TtsTrain* t = h->train;
-    c.h = h; c.t = t; c.w = TrWs::make(reinterpret_cast<unsigned char*>(ws), B, S, T); c.st = (cudaStream_t)stream;
+    c.h = h; c.t = t; c.w = TrWs::make(reinterpret_cast<unsigned char*>(ws), B, S, T); c.st = st;
     c.B = B; c.S = S; c.T = T; c.seed = c.w.seed_dev; c.utt0 = utt_offset;
     c.thresh = (uint32_t)(p_residual * 4294967296.0); c.dscale = 1.0f / (float)(1.0 - p_residual);
     c.P = t->P; c.G = t->G;
-    // stage the inputs: the step itself (eager or replayed from its CUDA graph) reads workspace memory only
-    CK(cudaMemcpyAsync(c.w.plens, phoneme_lens, (size_t)B * 4, cudaMemcpyDeviceToDevice, c.st));
-    CK(cudaMemcpyAsync(c.w.mlens, mel_lens, (size_t)B * 4, cudaMemcpyDeviceToDevice, c.st));
-    CK(cudaMemcpyAsync(c.w.ph_in, phonemes, (size_t)B * S * 8, cudaMemcpyDeviceToDevice, c.st));
-    CK(cudaMemcpyAsync(c.w.mels_in, mels, (size_t)B * T * 80 * 4, cudaMemcpyDeviceToDevice, c.st));
-    set_u64_kernel<<<1, 1, 0, c.st>>>(c.w.seed_dev, seed);
+    return c;
+}
+// Checks the arguments of a training call that takes a batch, builds its context and stages the inputs: the step itself (eager
+// or replayed from its CUDA graph) reads workspace memory only.  The caller holds the device guard.
+int train_stage(TrCtx& c, TtsHandle* h, void* ws, const int64_t* phonemes, const int32_t* phoneme_lens, const float* mels, const int32_t* mel_lens,
+                int B, int S, int T, uint64_t seed, int utt_offset, double p_residual, cudaStream_t st) {
+    if (!ws || !phonemes || !phoneme_lens || !mels || !mel_lens || B <= 0 || S <= 0 || T <= 0) return TTS_E_ARG;
+    if (!h->train) FAIL(TTS_E_STATE, "tts_train_begin has not been called");
+    if (S > h->cfg.max_pos || T > h->cfg.max_pos) FAIL(TTS_E_ARG, "sequence exceeds max_pos");
+    if (p_residual < 0.0 || p_residual >= 1.0) FAIL(TTS_E_ARG, "p_residual out of range");
+    c = train_ctx(h, ws, B, S, T, utt_offset, p_residual, st);
+    CK(cudaMemcpyAsync(c.w.plens, phoneme_lens, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
+    CK(cudaMemcpyAsync(c.w.mlens, mel_lens, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
+    CK(cudaMemcpyAsync(c.w.ph_in, phonemes, (size_t)B * S * 8, cudaMemcpyDeviceToDevice, st));
+    CK(cudaMemcpyAsync(c.w.mels_in, mels, (size_t)B * T * 80 * 4, cudaMemcpyDeviceToDevice, st));
+    set_u64_kernel<<<1, 1, 0, st>>>(c.w.seed_dev, seed);
     ++launch_counter();
+    return 0;
+}
+}  // namespace
+extern "C" int tts_train_step(TtsHandle* h, void* ws, const int64_t* phonemes, const int32_t* phoneme_lens, const float* mels, const int32_t* mel_lens,
+                              int B, int S, int T, uint64_t seed, int utt_offset, double p_residual, float pos_weight, float* loss_out, void* stream) {
+    if (!h || !loss_out) return TTS_E_ARG;
+    DEV_GUARD(h);
+    TrCtx c;
+    int r = train_stage(c, h, ws, phonemes, phoneme_lens, mels, mel_lens, B, S, T, seed, utt_offset, p_residual, (cudaStream_t)stream);
+    if (r) return r;
+    TtsTrain* t = h->train;
     const TtsTrain::GraphKey key{ws, B, S, T, utt_offset, p_residual, pos_weight, loss_out, c.st};
     if (h->train_graph && t->graph_exec && key == t->graph_key) {
         CK(cudaGraphLaunch(t->graph_exec, c.st));
@@ -1234,7 +1253,7 @@ extern "C" int tts_train_step(TtsHandle* h, void* ws, const int64_t* phonemes, c
         cudaStream_t user_st = c.st;
         c.st = t->cap_stream;
         CK(cudaStreamBeginCapture(c.st, cudaStreamCaptureModeThreadLocal));
-        int r = train_forward_backward(c, loss_out, pos_weight);
+        r = train_forward_backward(c, loss_out, pos_weight);
         cudaError_t e = cudaStreamEndCapture(c.st, &graph);
         c.st = user_st;
         if (r) { if (graph) cudaGraphDestroy(graph); return r; }
@@ -1252,33 +1271,13 @@ extern "C" int tts_train_step(TtsHandle* h, void* ws, const int64_t* phonemes, c
     t->seen_key = key;
     return train_forward_backward(c, loss_out, pos_weight);
 }
-namespace {
-// context of one training call: workspace views, dropout threshold / scale, flat parameter and gradient buffers
-TrCtx train_ctx(TtsHandle* h, void* ws, int B, int S, int T, int utt_offset, double p_residual, cudaStream_t st) {
-    TrCtx c;
-    TtsTrain* t = h->train;
-    c.h = h; c.t = t; c.w = TrWs::make(reinterpret_cast<unsigned char*>(ws), B, S, T); c.st = st;
-    c.B = B; c.S = S; c.T = T; c.seed = c.w.seed_dev; c.utt0 = utt_offset;
-    c.thresh = (uint32_t)(p_residual * 4294967296.0); c.dscale = 1.0f / (float)(1.0 - p_residual);
-    c.P = t->P; c.G = t->G;
-    return c;
-}
-}  // namespace
 extern "C" int tts_train_forward(TtsHandle* h, void* ws, const int64_t* phonemes, const int32_t* phoneme_lens, const float* mels, const int32_t* mel_lens,
                                  int B, int S, int T, uint64_t seed, int utt_offset, double p_residual, void* stream) {
-    if (!h || !ws || !phonemes || !phoneme_lens || !mels || !mel_lens || B <= 0 || S <= 0 || T <= 0) return TTS_E_ARG;
-    if (!h->train) FAIL(TTS_E_STATE, "tts_train_begin has not been called");
-    if (S > h->cfg.max_pos || T > h->cfg.max_pos) FAIL(TTS_E_ARG, "sequence exceeds max_pos");
-    if (p_residual < 0.0 || p_residual >= 1.0) FAIL(TTS_E_ARG, "p_residual out of range");
+    if (!h) return TTS_E_ARG;
     DEV_GUARD(h);
-    TrCtx c = train_ctx(h, ws, B, S, T, utt_offset, p_residual, (cudaStream_t)stream);
-    CK(cudaMemcpyAsync(c.w.plens, phoneme_lens, (size_t)B * 4, cudaMemcpyDeviceToDevice, c.st));
-    CK(cudaMemcpyAsync(c.w.mlens, mel_lens, (size_t)B * 4, cudaMemcpyDeviceToDevice, c.st));
-    CK(cudaMemcpyAsync(c.w.ph_in, phonemes, (size_t)B * S * 8, cudaMemcpyDeviceToDevice, c.st));
-    CK(cudaMemcpyAsync(c.w.mels_in, mels, (size_t)B * T * 80 * 4, cudaMemcpyDeviceToDevice, c.st));
-    set_u64_kernel<<<1, 1, 0, c.st>>>(c.w.seed_dev, seed);
-    ++launch_counter();
-    return train_forward(c);
+    TrCtx c;
+    int r = train_stage(c, h, ws, phonemes, phoneme_lens, mels, mel_lens, B, S, T, seed, utt_offset, p_residual, (cudaStream_t)stream);
+    return r ? r : train_forward(c);
 }
 extern "C" int tts_train_backward(TtsHandle* h, void* ws, int B, int S, int T, int utt_offset, double p_residual, const float* d_before,
                                   const float* d_after, const float* d_stop, void* stream) {

@@ -300,14 +300,23 @@ class TransformerTTS(nn.Module):
         except Exception:
             pass
 
+    def _stage_inputs(self, phonemes, phoneme_lens, mels=None, mel_lens=None):
+        """The inputs a call has, on the module's device and contiguous: phonemes int64, lengths int32, mels fp32."""
+        inputs = ((phonemes, torch.int64), (phoneme_lens, torch.int32), (mels, torch.float32), (mel_lens, torch.int32))
+        return tuple(t.to(self.device, dt).contiguous() for t, dt in inputs if t is not None)
+
     @staticmethod
-    def _utt_offset(utt_ids, B, utt_offset):
+    def _utt_ids(utt_ids, B, utt_offset, contiguous=False):
+        """-> (offset, ids or None).  A contiguous range of utterance ids is just the offset of utterance 0; any other ids come
+        back as an int32 tensor, or raise ValueError with contiguous=True (the teacher-forced C entry points take the offset only)."""
         if utt_ids is None:
-            return int(utt_offset)
-        ids = [int(v) for v in utt_ids]
-        if ids != list(range(ids[0], ids[0] + B)):
+            return int(utt_offset), None
+        ids = torch.as_tensor([int(v) for v in utt_ids], dtype=torch.int32)
+        if ids.tolist() == list(range(int(ids[0]), int(ids[0]) + B)):
+            return int(ids[0]), None
+        if contiguous:
             raise ValueError("utt_ids must be a contiguous range (the C ABI takes the id of utterance 0)")
-        return ids[0]
+        return int(utt_offset), ids
 
     # ------------------------------------------------------------------ teacher-forced
     def forward(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_ids=None, utt_offset: int = 0
@@ -315,24 +324,28 @@ class TransformerTTS(nn.Module):
         """phonemes [B,S] i64, phoneme_lens [B], mels [B,T,80] f32, mel_lens [B]
         -> mel_before [B,T,80], mel_after [B,T,80], stop_logits [B,T]  (on the GPU, zero past mel_lens)."""
         if self.training:
-            return self._train_forward(phonemes, phoneme_lens, mels, mel_lens, seed, self._utt_offset(utt_ids, phonemes.shape[0], utt_offset))
+            return self._train_forward(phonemes, phoneme_lens, mels, mel_lens, seed,
+                                       self._utt_ids(utt_ids, phonemes.shape[0], utt_offset, contiguous=True)[0])
         with torch.no_grad():
             return self._eval_forward(phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset)
 
-    def _eval_forward(self, phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset):
+    def _teacher_forced_setup(self, phonemes, phoneme_lens, mels, mel_lens, utt_ids, utt_offset):
+        """Set-up shared by tts_forward and tts_forward_align.  -> lib, workspace, staged (ph, pl, mels, mel_lens), (B, S, T),
+        offset of utterance 0."""
         lib = self._ensure_handle()
         self.sync_weights()
-        dev = self.device
         B, S = phonemes.shape
         T = mels.shape[1]
-        ph = phonemes.to(dev, torch.int64).contiguous()
-        pl = phoneme_lens.to(dev, torch.int32).contiguous()
-        ml = mel_lens.to(dev, torch.int32).contiguous()
-        m = mels.to(dev, torch.float32).contiguous()
+        inputs = self._stage_inputs(phonemes, phoneme_lens, mels, mel_lens)
         ws = self._workspace(B, S, T)
+        return lib, ws, inputs, (B, S, T), self._utt_ids(utt_ids, B, utt_offset, contiguous=True)[0]
+
+    def _eval_forward(self, phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset):
+        lib, ws, (ph, pl, m, ml), (B, S, T), u0 = self._teacher_forced_setup(phonemes, phoneme_lens, mels, mel_lens, utt_ids, utt_offset)
+        dev = self.device
         mb = torch.empty(B, T, 80, device=dev); ma = torch.empty(B, T, 80, device=dev); st = torch.empty(B, T, device=dev)
         rc = lib.tts_forward(self._handle, ws.data_ptr(), ph.data_ptr(), pl.data_ptr(), m.data_ptr(), ml.data_ptr(), B, S, T,
-                             int(seed), self._utt_offset(utt_ids, B, utt_offset), mb.data_ptr(), ma.data_ptr(), st.data_ptr(), self._stream())
+                             int(seed), u0, mb.data_ptr(), ma.data_ptr(), st.data_ptr(), self._stream())
         self._check(rc, "tts_forward")
         return mb, ma, st
 
@@ -379,16 +392,8 @@ class TransformerTTS(nn.Module):
                        want_align, want_durations):
         if self.training:
             raise RuntimeError("alignments() / durations() are eval-mode paths: call model.eval() first")
-        lib = self._ensure_handle()
-        self.sync_weights()
+        lib, ws, (ph, pl, m, ml), (B, S, T), u0 = self._teacher_forced_setup(phonemes, phoneme_lens, mels, mel_lens, utt_ids, utt_offset)
         dev = self.device
-        B, S = phonemes.shape
-        T = mels.shape[1]
-        ph = phonemes.to(dev, torch.int64).contiguous()
-        pl = phoneme_lens.to(dev, torch.int32).contiguous()
-        ml = mel_lens.to(dev, torch.int32).contiguous()
-        m = mels.to(dev, torch.float32).contiguous()
-        ws = self._workspace(B, S, T)
         out, scratch = {}, None
         if want_align:
             out["align"] = torch.empty(bin(layer_mask).count("1"), B, 8, T, S, device=dev)
@@ -399,7 +404,7 @@ class TransformerTTS(nn.Module):
             out["focus"] = torch.empty(6, B, 8, device=dev)
         ptr = lambda k: out[k].data_ptr() if k in out else None                                          # noqa: E731
         rc = lib.tts_forward_align(self._handle, ws.data_ptr(), scratch.data_ptr() if scratch is not None else None, ph.data_ptr(),
-                                   pl.data_ptr(), m.data_ptr(), ml.data_ptr(), B, S, T, int(seed), self._utt_offset(utt_ids, B, utt_offset),
+                                   pl.data_ptr(), m.data_ptr(), ml.data_ptr(), B, S, T, int(seed), u0,
                                    layer_mask, fixed_head, None, None, None, ptr("align"), ptr("focus"), ptr("durations"), ptr("head"),
                                    self._stream())
         self._check(rc, "tts_forward_align")
@@ -430,6 +435,17 @@ class TransformerTTS(nn.Module):
         return out
 
     # ------------------------------------------------------------------ greedy AR
+    def _start_decode(self, ws, ph, pl, max_len, seed, utt_offset, ids, max_lens, work_stealing, stream):
+        """Opens a decode session in `ws` and encodes the batch: tts_decode_begin, tts_decode_set_batch when there are per-utterance
+        ids or frame budgets (device int32 tensors or None), tts_encode."""
+        lib, h, wsp = self._lib, self._handle, ws.data_ptr()
+        B, S = ph.shape
+        self._check(lib.tts_decode_begin(h, wsp, B, S, max_len, int(seed), utt_offset, stream), "tts_decode_begin")
+        if ids is not None or max_lens is not None:
+            ptr = lambda t: None if t is None else t.data_ptr()                                           # noqa: E731
+            self._check(lib.tts_decode_set_batch(h, wsp, ptr(ids), ptr(max_lens), int(work_stealing), stream), "tts_decode_set_batch")
+        self._check(lib.tts_encode(h, wsp, ph.data_ptr(), pl.data_ptr(), B, S, max_len, None, stream), "tts_encode")
+
     @torch.no_grad()
     def inference(self, phonemes, phoneme_lens, max_len: int = 800, seed: int = 0, utt_ids=None, utt_offset: int = 0,
                   return_before: bool = False, clone_outputs: bool = True, max_lens=None, sort_by_length: bool = False,
@@ -453,12 +469,7 @@ class TransformerTTS(nn.Module):
         lib = self._ensure_handle()
         self.sync_weights()
         B, S = phonemes.shape
-        ids = None
-        if utt_ids is not None:
-            ids = torch.as_tensor([int(v) for v in utt_ids], dtype=torch.int32)
-            if ids.tolist() == list(range(int(ids[0]), int(ids[0]) + B)):
-                utt_offset, ids = int(ids[0]), None                    # a contiguous range is just an offset
-        u0 = int(utt_offset)
+        u0, ids = self._utt_ids(utt_ids, B, utt_offset)
         ragged = ids is not None or max_lens is not None or sort_by_length
         ws = self._workspace(B, S, max_len)
         if not phonemes.is_cuda and not return_before and not ragged:
@@ -479,8 +490,7 @@ class TransformerTTS(nn.Module):
             return tuple(t.clone() for t in out) if clone_outputs else out
         dev = self.device
         to_host = not phonemes.is_cuda
-        ph = phonemes.to(dev, torch.int64).contiguous()
-        pl = phoneme_lens.to(dev, torch.int32).contiguous()
+        ph, pl = self._stage_inputs(phonemes, phoneme_lens)
         perm = inv = None
         mlens_d = None if max_lens is None else torch.as_tensor(max_lens).to(dev, torch.int32).clamp(1, int(max_len)).contiguous()
         ids_d = None if ids is None else ids.to(dev)
@@ -494,12 +504,8 @@ class TransformerTTS(nn.Module):
             if mlens_d is not None:
                 mlens_d = mlens_d[perm].contiguous()
         stream = self._stream()
-        self._check(lib.tts_decode_begin(self._handle, ws.data_ptr(), B, S, int(max_len), int(seed), u0, stream), "tts_decode_begin")
-        if ragged:
-            steal = ragged if work_stealing is None else bool(work_stealing)
-            self._check(lib.tts_decode_set_batch(self._handle, ws.data_ptr(), ids_d.data_ptr() if ids_d is not None else None,
-                                                 mlens_d.data_ptr() if mlens_d is not None else None, int(steal), stream), "tts_decode_set_batch")
-        self._check(lib.tts_encode(self._handle, ws.data_ptr(), ph.data_ptr(), pl.data_ptr(), B, S, int(max_len), None, stream), "tts_encode")
+        # a ragged batch always has ids_d or mlens_d here; work stealing is on for it unless the caller says otherwise
+        self._start_decode(ws, ph, pl, int(max_len), seed, u0, ids_d, mlens_d, work_stealing is None or bool(work_stealing), stream)
         td, nf = C.c_int(0), C.c_int(0)
         chunk = int(max_len)                               # one launch: every cluster stops itself on the device
         if self.profile_events:
@@ -549,16 +555,11 @@ class TransformerTTS(nn.Module):
         self.sync_weights()
         B, S = phonemes.shape
         max_len = int(max_len)
-        ids = None
-        if utt_ids is not None:
-            ids = torch.as_tensor([int(v) for v in utt_ids], dtype=torch.int32)
-            if ids.tolist() == list(range(int(ids[0]), int(ids[0]) + B)):
-                utt_offset, ids = int(ids[0]), None
+        u0, ids = self._utt_ids(utt_ids, B, utt_offset)
         sched = StreamSchedule(chunk_frames, postnet_halo(self.cfg), max_len)
         dev = self.device
         to_host = not phonemes.is_cuda
-        ph = phonemes.to(dev, torch.int64).contiguous()
-        pl = phoneme_lens.to(dev, torch.int32).contiguous()
+        ph, pl = self._stage_inputs(phonemes, phoneme_lens)
         mlens_d = None if max_lens is None else torch.as_tensor(max_lens).to(dev, torch.int32).clamp(1, max_len).contiguous()
         ids_d = None if ids is None else ids.to(dev)
         ws = self._workspace(B, S, max_len)
@@ -568,11 +569,7 @@ class TransformerTTS(nn.Module):
         side, cur = self._side_stream, torch.cuda.current_stream(dev)
         stream, side_ptr = self._stream(), C.c_void_p(side.cuda_stream)
         h, wsp = self._handle, ws.data_ptr()
-        self._check(lib.tts_decode_begin(h, wsp, B, S, max_len, int(seed), int(utt_offset), stream), "tts_decode_begin")
-        if ids_d is not None or mlens_d is not None:
-            self._check(lib.tts_decode_set_batch(h, wsp, ids_d.data_ptr() if ids_d is not None else None,
-                                                 mlens_d.data_ptr() if mlens_d is not None else None, 0, stream), "tts_decode_set_batch")
-        self._check(lib.tts_encode(h, wsp, ph.data_ptr(), pl.data_ptr(), B, S, max_len, None, stream), "tts_encode")
+        self._start_decode(ws, ph, pl, max_len, seed, u0, ids_d, mlens_d, False, stream)
         nbytes = lib.tts_stream_scratch_bytes(h, B, sched.max_emit_frames())
         with torch.cuda.stream(side):
             scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev)
@@ -634,8 +631,7 @@ class TransformerTTS(nn.Module):
         B, S = phonemes.shape
         T = int(T or S)
         ws = self._workspace(B, S, T)
-        ph = phonemes.to(dev, torch.int64).contiguous()
-        pl = phoneme_lens.to(dev, torch.int32).contiguous()
+        ph, pl = self._stage_inputs(phonemes, phoneme_lens)
         mem = torch.empty(B, S, 512, device=dev)
         self._check(lib.tts_encode(self._handle, ws.data_ptr(), ph.data_ptr(), pl.data_ptr(), B, S, T, mem.data_ptr(), self._stream()), "tts_encode")
         return mem

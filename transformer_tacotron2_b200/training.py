@@ -85,43 +85,39 @@ class Trainer:
         dist.all_reduce(self._tick, op=dist.ReduceOp.SUM, group=self.group)
 
     # ------------------------------------------------------------------ one step
-    def _workspace(self, B, S, T):
+    def _stage(self, phonemes, phoneme_lens, mels, mel_lens):
+        """Moves a batch to the device, into self._in (the library's asynchronous copies read from it), records its shape and
+        returns the workspace for that shape."""
+        B, S = phonemes.shape
+        T = mels.shape[1]
+        self._in = self.model._stage_inputs(phonemes, phoneme_lens, mels, mel_lens)
         if self._ws_key != (B, S, T):
             n = self._lib.tts_train_workspace_bytes(self._h, B, S, T)
             self._ws = None
             self._ws = torch.empty(n, dtype=torch.uint8, device=self.model.device)
             self._ws_key = (B, S, T)
+        self._shape = (B, S, T)
         return self._ws
 
     def forward_backward(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_offset: int = 0) -> torch.Tensor:
         """Train-mode forward + loss + backward.  Returns the loss (1-element device tensor); gradients are in flat_grads."""
-        m, dev = self.model, self.model.device
-        B, S = phonemes.shape
-        T = mels.shape[1]
-        self._in = (phonemes.to(dev, torch.int64).contiguous(), phoneme_lens.to(dev, torch.int32).contiguous(),
-                    mels.to(dev, torch.float32).contiguous(), mel_lens.to(dev, torch.int32).contiguous())
-        ph, pl, me, ml = self._in
-        ws = self._workspace(B, S, T)
+        m = self.model
+        ws = self._stage(phonemes, phoneme_lens, mels, mel_lens)
+        (ph, pl, me, ml), (B, S, T) = self._in, self._shape
         rc = self._lib.tts_train_step(self._h, ws.data_ptr(), ph.data_ptr(), pl.data_ptr(), me.data_ptr(), ml.data_ptr(), B, S, T, int(seed),
                                       int(utt_offset), self.p_residual, self.pos_weight, self._loss.data_ptr(), m._stream())
         m._check(rc, "tts_train_step")
-        self._shape = (B, S, T)
         return self._loss
 
     # ------------------------------------------------------------------ autograd bridge (model.train(); model(...); loss.backward())
     def forward_only(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_offset: int = 0):
         """Train-mode forward alone; the activations stay in the workspace for backward_from().  -> (mel_before, mel_after, stop)."""
-        m, dev = self.model, self.model.device
-        B, S = phonemes.shape
-        T = mels.shape[1]
-        self._in = (phonemes.to(dev, torch.int64).contiguous(), phoneme_lens.to(dev, torch.int32).contiguous(),
-                    mels.to(dev, torch.float32).contiguous(), mel_lens.to(dev, torch.int32).contiguous())
-        ph, pl, me, ml = self._in
-        ws = self._workspace(B, S, T)
+        m = self.model
+        ws = self._stage(phonemes, phoneme_lens, mels, mel_lens)
+        (ph, pl, me, ml), (B, S, T) = self._in, self._shape
         rc = self._lib.tts_train_forward(self._h, ws.data_ptr(), ph.data_ptr(), pl.data_ptr(), me.data_ptr(), ml.data_ptr(), B, S, T, int(seed),
                                          int(utt_offset), self.p_residual, m._stream())
         m._check(rc, "tts_train_forward")
-        self._shape = (B, S, T)
         self._fwd_args = (int(utt_offset),)
         return self.outputs()
 
