@@ -39,12 +39,19 @@ extern "C" {
 typedef struct TtsHandle TtsHandle;
 
 /* oracle/transformer_tts.py:TTSConfig (SURVEY.md section 5 "Config / flags").  Only the base model
- * (d_model 512, 8 heads, d_ff 2048, 80 mels, prenet 256, kernel 5) is accepted. */
+ * (d_model 512, 8 heads, d_ff 2048, 80 mels, prenet 256, kernel 5) is accepted.
+ * Multi-speaker models (ESPnet Transformer-TTS, spk_embed_integration_type "add"): n_speakers > 0 adds a speaker-ID table
+ * "speaker_embed.weight" [n_speakers][512] (n_speakers <= 65536), spk_embed_dim > 0 an x-vector projection "spk_proj.weight"
+ * [512][spk_embed_dim] + "spk_proj.bias" [512] (spk_embed_dim <= 1024).  The speaker vector
+ *     cond[b] = speaker_embed[sids[b]] + spk_proj(spembs[b] / max(||spembs[b]||, 1e-12))
+ * is added to every row of the encoder output before the decoder reads it as memory.  struct_size may also be
+ * offsetof(TtsConfig, n_speakers) (callers built before these fields existed): an unconditioned model. */
 typedef struct TtsConfig {
     uint32_t struct_size;
     int32_t n_vocab, d_model, n_heads, n_enc_layers, n_dec_layers, d_ff, n_mels, d_prenet;
     int32_t enc_conv_layers, conv_kernel, postnet_channels, postnet_layers, max_pos;
     float ln_eps, bn_eps;
+    int32_t n_speakers, spk_embed_dim;
 } TtsConfig;
 
 /* ---- lifetime ------------------------------------------------------------------------------ */
@@ -82,6 +89,14 @@ size_t tts_workspace_bytes(TtsHandle* h, int B, int S, int T);
  * memory_out: optional fp32 [B][S][512] copy of the encoder output (may be NULL). */
 int tts_encode(TtsHandle* h, void* ws, const int64_t* phonemes, const int32_t* phoneme_lens,
                int B, int S, int T, float* memory_out, void* stream);
+/* Speaker conditioning of a multi-speaker handle (TtsConfig.n_speakers / spk_embed_dim): stage the batch's speakers in `ws`
+ * (cudaMemcpyAsync of sids int32 [B], given iff n_speakers > 0, and spembs fp32 [B][spk_embed_dim], given iff spk_embed_dim > 0;
+ * device memory).  The next tts_encode, tts_forward or tts_forward_align on the same ws with the same B consumes the staged
+ * speakers; on a conditioned handle those calls return TTS_E_STATE without a matching tts_set_conditioning, so a batch can never
+ * silently reuse the previous batch's voices.  In a decode session call it after tts_decode_begin / tts_decode_set_batch and
+ * before tts_encode.  An id outside [0, n_speakers) contributes a zero vector.  TTS_E_STATE on an unconditioned handle.
+ * tts_infer_host returns TTS_E_STATE on a conditioned handle.  The encoder of a conditioned handle issues one launch more. */
+int tts_set_conditioning(TtsHandle* h, void* ws, int B, const int32_t* sids, const float* spembs, void* stream);
 /* Reset the AR state (KV cache cursor, lengths, stop flags).  utt_offset = global id of utterance 0
  * (dropout masks are keyed by global utterance id so a sharded batch reproduces the unsharded one). */
 int tts_decode_begin(TtsHandle* h, void* ws, int B, int S, int max_len, uint64_t seed, int utt_offset, void* stream);
@@ -191,6 +206,12 @@ size_t tts_train_workspace_bytes(TtsHandle* h, int B, int S, int T);
 /* Train-mode forward (batch-statistics BatchNorm, Philox dropout at every site), loss, full backward.  All pointers
  * are DEVICE pointers.  Afterwards the gradient of every parameter is in the flat gradient buffer (tts_train_grads),
  * loss_out[0] holds the scalar loss, and BatchNorm running statistics have been updated. */
+/* The training counterpart of tts_set_conditioning, for the training workspace: the next tts_train_step or tts_train_forward on
+ * it with the same B consumes the staged speakers (TTS_E_STATE without them on a conditioned handle).  The inputs are copied
+ * into the workspace, so a step replayed from its CUDA graph reads each step's new speakers.  The gradients of speaker_embed,
+ * spk_proj.weight and spk_proj.bias land in the flat gradient buffer like every other parameter's (spembs get none); a
+ * conditioned step issues three launches more than an unconditioned one. */
+int tts_train_set_conditioning(TtsHandle* h, void* workspace, int B, const int32_t* sids, const float* spembs, void* stream);
 int tts_train_step(TtsHandle* h, void* workspace, const int64_t* phonemes, const int32_t* phoneme_lens, const float* mels,
                    const int32_t* mel_lens, int B, int S, int T, uint64_t seed, int utt_offset, double p_residual,
                    float pos_weight, float* loss_out, void* stream);
@@ -256,6 +277,19 @@ int tts_k_cross_align(const void* Q, int ldq, const void* K, const int32_t* qlen
                       int B, int H, int Lq, int Lk, float* P, float* rowmax, int16_t* argmax, void* stream);
 /* LayerNorm over rows of 512: fp32 in -> bf16 out. */
 int tts_k_layernorm(const float* X, const float* gamma, const float* beta, void* Y_bf16, int M, float eps, void* stream);
+/* Speaker conditioning (speaker.cuh), launched as the library launches it.  One CTA per utterance: nhat [B][D] = spembs[b] /
+ * max(||spembs[b]||, 1e-12), cond [B][512] = table[sids[b]] (zero for an id outside [0, n_speakers)) + W [512][D] . nhat[b] + bias.
+ * table may be NULL (no speaker-ID term), W / bias / spembs / nhat are NULL iff D = 0; fp32, device memory. */
+int tts_k_speaker_cond(const int32_t* sids, const float* spembs, int B, int n_speakers, int D, const float* table, const float* W,
+                       const float* bias, float* cond, float* nhat, void* stream);
+/* LayerNorm over rows of 512 plus a per-utterance row: Y[m] = bf16(LN(X[m]) * gamma + beta + cond[m / S]), summed in fp32. */
+int tts_k_layernorm_cond(const float* X, const float* gamma, const float* beta, const float* cond, void* Y_bf16, int M, int S, float eps,
+                         void* stream);
+/* Its backward: dcond [B][512] = sum_{s < plens[b]} dmem[b * S + s] (dmem fp32 [B * S][512]), then dE[sids[b]] += dcond[b],
+ * dW[n][k] += sum_b dcond[b][n] nhat[b][k], dbias += sum_b dcond[b]; every element summed in ascending b by one thread (no
+ * atomics: bit-identical from run to run).  dE may be NULL; dW / dbias / nhat are NULL iff D = 0. */
+int tts_k_speaker_cond_bwd(const float* dmem, const int32_t* plens, const int32_t* sids, const float* nhat, int B, int S, int n_speakers,
+                           int D, float* dcond, float* dE, float* dW, float* dbias, void* stream);
 /* Keep-bits of a p = 0.5 dropout site: out[t][b][c] (uint8) for t < T, b < B, c < C. */
 int tts_k_philox_bits(uint64_t seed, int site, int T, int B, int C, int utt_offset, uint8_t* out, void* stream);
 

@@ -15,7 +15,7 @@ class TtsConfig(C.Structure):
     _fields_ = [("struct_size", C.c_uint32)] + [(n, C.c_int32) for n in (
         "n_vocab", "d_model", "n_heads", "n_enc_layers", "n_dec_layers", "d_ff", "n_mels", "d_prenet",
         "enc_conv_layers", "conv_kernel", "postnet_channels", "postnet_layers", "max_pos")] + [
-        ("ln_eps", C.c_float), ("bn_eps", C.c_float)]
+        ("ln_eps", C.c_float), ("bn_eps", C.c_float), ("n_speakers", C.c_int32), ("spk_embed_dim", C.c_int32)]
 
 
 _P, _I, _I64, _U64, _SZ = C.c_void_p, C.c_int, C.c_int64, C.c_uint64, C.c_size_t
@@ -32,6 +32,7 @@ SIGNATURES = {
     "tts_set_option": (_I, [_P, C.c_char_p, _I64]),
     "tts_workspace_bytes": (_SZ, [_P, _I, _I, _I]),
     "tts_encode": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P]),
+    "tts_set_conditioning": (_I, [_P, _P, _I, _P, _P, _P]),
     "tts_decode_begin": (_I, [_P, _P, _I, _I, _I, _U64, _I, _P]),
     "tts_decode_steps": (_I, [_P, _P, _I, _P]),
     "tts_decode_status": (_I, [_P, _P, C.POINTER(_I), C.POINTER(_I), _P]),
@@ -52,6 +53,7 @@ SIGNATURES = {
     "tts_train_begin": (_I, [_P]),
     "tts_train_end": (_I, [_P]),
     "tts_train_workspace_bytes": (_SZ, [_P, _I, _I, _I]),
+    "tts_train_set_conditioning": (_I, [_P, _P, _I, _P, _P, _P]),
     "tts_train_step": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _U64, _I, C.c_double, C.c_float, _P, _P]),
     "tts_train_outputs": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _P]),
     "tts_train_grads": (_I, [_P, C.POINTER(_P), C.POINTER(_I64)]),
@@ -73,6 +75,9 @@ SIGNATURES = {
     "tts_k_attention_bwd": (_I, [_P] * 11 + [_I, _I, _I, _I, _I, _P]),
     "tts_k_cross_align": (_I, [_P, _I, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P]),
     "tts_k_layernorm": (_I, [_P, _P, _P, _P, _I, C.c_float, _P]),
+    "tts_k_speaker_cond": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P]),
+    "tts_k_layernorm_cond": (_I, [_P, _P, _P, _P, _P, _I, _I, C.c_float, _P]),
+    "tts_k_speaker_cond_bwd": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
     "tts_k_philox_bits": (_I, [_U64, _I, _I, _I, _I, _I, _P, _P]),
     "tts_k_wgrad": (_I, [_P, _I, _I, _P, _I, _I, _I, _I, _I, _P, _P, _P]),
     "tts_k_dgrad": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _I, _P, _P, _I, _P, _P]),

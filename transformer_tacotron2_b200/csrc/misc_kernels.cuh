@@ -20,8 +20,12 @@ __global__ void embed_kernel(const int64_t* __restrict__ ph, const int* __restri
 }
 
 // LayerNorm over rows of 512 (fp32 in, bf16 and/or fp32 out); one warp per row, two-pass statistics.
+// kCond: the row of utterance m / S of cond fp32 [B][512] is added to the affine output in fp32, before the rounding
+// (speaker conditioning of the encoder memory, speaker.cuh); the <false> instantiation never reads cond.
+template <bool kCond>
 __global__ void layernorm512_kernel(const float* __restrict__ x, const float* __restrict__ g, const float* __restrict__ bta,
-                                    bf16* __restrict__ out_bf16, float* __restrict__ out_f32, int M, float eps) {
+                                    bf16* __restrict__ out_bf16, float* __restrict__ out_f32, int M, float eps,
+                                    const float* __restrict__ cond, int S) {
     const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (row >= M) return;
     float v[16];
@@ -43,8 +47,12 @@ __global__ void layernorm512_kernel(const float* __restrict__ x, const float* __
     for (int i = 0; i < 4; ++i) {
         const int c = i * 128 + lane * 4;
         const float4 g4 = *reinterpret_cast<const float4*>(g + c), b4 = *reinterpret_cast<const float4*>(bta + c);
-        const float o0 = (v[i * 4] - mean) * rstd * g4.x + b4.x, o1 = (v[i * 4 + 1] - mean) * rstd * g4.y + b4.y;
-        const float o2 = (v[i * 4 + 2] - mean) * rstd * g4.z + b4.z, o3 = (v[i * 4 + 3] - mean) * rstd * g4.w + b4.w;
+        float o0 = (v[i * 4] - mean) * rstd * g4.x + b4.x, o1 = (v[i * 4 + 1] - mean) * rstd * g4.y + b4.y;
+        float o2 = (v[i * 4 + 2] - mean) * rstd * g4.z + b4.z, o3 = (v[i * 4 + 3] - mean) * rstd * g4.w + b4.w;
+        if constexpr (kCond) {
+            const float4 c4 = *reinterpret_cast<const float4*>(cond + (size_t)(row / S) * kDModel + c);
+            o0 += c4.x; o1 += c4.y; o2 += c4.z; o3 += c4.w;
+        }
         if (out_bf16) *reinterpret_cast<uint2*>(out_bf16 + (size_t)row * kDModel + c) = make_uint2(pack_bf16x2(o0, o1), pack_bf16x2(o2, o3));
         if (out_f32) *reinterpret_cast<float4*>(out_f32 + (size_t)row * kDModel + c) = make_float4(o0, o1, o2, o3);
     }

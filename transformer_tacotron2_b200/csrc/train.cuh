@@ -51,6 +51,7 @@ struct TtsTrain {
     bf16* wpack = nullptr;
     std::vector<TrMat> mats;
     size_t enc_alpha = 0, dec_alpha = 0;
+    size_t spk_table = 0, spk_w = 0, spk_b = 0;                      // speaker conditioning (fp32, read directly from P; no operand copies)
     int embed = 0;
     TrConv enc_conv[3], post_conv[5];
     TrLin enc_proj, fc1, fc2, dproj, ckv, head;
@@ -109,9 +110,16 @@ struct TrWs {
     bf16 *dsub, *dwide, *dqkv, *dctx, *dkv, *dhead, *dcv, *dcv2;
     int *plens, *mlens;
     int64_t* ph_in; float* mels_in; uint64_t* seed_dev;     // staged inputs: a captured step only ever reads workspace memory
-    static TrWs make(unsigned char* base, int B, int S, int T) {
+    // speaker conditioning (cond_dim >= 0, as Ws::make): staged sids / spembs, cond [B][512], normalised spembs, dcond [B][512].
+    // First in the workspace, so that tts_train_set_conditioning finds it from B alone; an unconditioned layout is unchanged.
+    int* sids = nullptr; float *spembs = nullptr, *cond = nullptr, *nhat = nullptr, *dcond = nullptr;
+    static TrWs make(unsigned char* base, int B, int S, int T, int cond_dim = -1) {
         TrWs w; size_t o = 0;
         auto take = [&](size_t bytes) { size_t r = o; o = align_up(o + bytes, 1024); return base + r; };
+        if (cond_dim >= 0) {
+            w.sids = (int*)take((size_t)B * 4); w.spembs = (float*)take((size_t)B * cond_dim * 4 + 4);
+            w.cond = (float*)take((size_t)B * 512 * 4); w.nhat = (float*)take((size_t)B * cond_dim * 4 + 4); w.dcond = (float*)take((size_t)B * 512 * 4);
+        }
         const size_t Me = (size_t)B * S, Md = (size_t)B * T, Mx = Me > Md ? Me : Md;
         w.Mep = (int)((Me + 63) / 64 * 64); w.Mdp = (int)((Md + 63) / 64 * 64);
         for (auto& p : w.e) p = (bf16*)take(Me * 512 * 2);
@@ -225,6 +233,8 @@ int train_build(TtsHandle* h) {
     }
     for (int i = 0; i < 5; ++i) t->post_conv[i] = conv("postnet.convs." + std::to_string(i), i == 0 ? 80 : 512, i == 4 ? 80 : 512);
     pad4();
+    if (c.n_speakers > 0) { t->spk_table = add("speaker_embed.weight", (size_t)c.n_speakers * D); pad4(); }
+    if (c.spk_embed_dim > 0) { t->spk_w = add("spk_proj.weight", (size_t)D * c.spk_embed_dim); t->spk_b = add("spk_proj.bias", D); pad4(); }
 
     CK(cudaMalloc(&t->P, t->n * 4)); CK(cudaMalloc(&t->G, t->n * 4)); CK(cudaMalloc(&t->M1, t->n * 4)); CK(cudaMalloc(&t->V2, t->n * 4));
     CK(cudaMalloc(&t->RS, t->nrs * 4)); CK(cudaMalloc(&t->wpack, t->wpack_elems * 2));
@@ -378,6 +388,9 @@ int train_forward(TrCtx& c) {
     const int* plens = w.plens; const int* mlens = w.mlens;
     const int64_t* ph = w.ph_in; const float* mels = w.mels_in;
     // ================================================================ forward (train mode)
+    if (w.cond)
+        TRL(launch_speaker_cond(w.sids, w.spembs, B, h->cfg.n_speakers, h->cfg.spk_embed_dim, h->cfg.n_speakers > 0 ? c.P + t->spk_table : nullptr,
+                                h->cfg.spk_embed_dim > 0 ? c.P + t->spk_w : nullptr, c.P + t->spk_b, w.cond, w.nhat, st));
     embed_kernel<<<(Me + 3) / 4, 256, 0, st>>>(ph, plens, t->mats[t->embed].fwd, w.e[0], B, S, h->cfg.n_vocab);
     ++launch_counter();
     for (int i = 0; i < 3; ++i) {
@@ -402,9 +415,10 @@ int train_forward(TrCtx& c) {
         TRL(launch_gemm_tc(p, st));
         p = tr_fwd(c, a.hdn, 2048, Me, S, L.w2); tr_dropw(c, p, SITE_ENC_LAYER0 + 2 * l + 1); p.resid_bf16 = a.x1; p.ldr = 512; p.out_f32 = a.y2; p.ldo = 512;
         TRL(launch_gemm_tc(p, st));
-        TRL(layernorm(a.y2, c.P + L.ln2g, c.P + L.ln2b, w.xe[l + 1], nullptr, Me, eps, st));
+        if (l == 5 && w.cond) TRL(launch_layernorm_cond(a.y2, c.P + L.ln2g, c.P + L.ln2b, w.xe[l + 1], nullptr, Me, eps, w.cond, S, st));
+        else TRL(layernorm(a.y2, c.P + L.ln2g, c.P + L.ln2b, w.xe[l + 1], nullptr, Me, eps, st));
     }
-    const bf16* mem = w.xe[6];
+    const bf16* mem = w.xe[6];                                          // (+ cond[b], added by the last LayerNorm when conditioned)
     {
         GemmParams p = tr_fwd(c, mem, 512, Me, S, t->ckv); p.out_bf16 = w.kvmem; p.ldo = 6144;
         TRL(launch_gemm_tc(p, st));
@@ -545,6 +559,10 @@ int train_backward(TrCtx& c) {
         GemmParams p = tr_dgrad(c, w.dkv, 6144, 6144, Me, S, t->ckv.mat); p.out_f32 = w.dx; p.ldo = 512;
         TRL(launch_gemm_tc(p, st));
     }
+    if (w.cond)   // memory = LN(y2) + cond[b]: dcond is the memory gradient summed over the valid rows (it is zero at padded keys)
+        TRL(launch_speaker_cond_bwd(w.dx, plens, w.sids, w.nhat, B, S, h->cfg.n_speakers, h->cfg.spk_embed_dim, w.dcond,
+                                    h->cfg.n_speakers > 0 ? c.G + t->spk_table : nullptr, h->cfg.spk_embed_dim > 0 ? c.G + t->spk_w : nullptr,
+                                    c.G + t->spk_b, st));
     for (int l = 5; l >= 0; --l) {
         const TrEnc& L = t->enc[l]; auto& a = w.el[l];
         int r;

@@ -22,6 +22,7 @@
 #include "train_kernels.cuh"
 #include "wgrad_tc.cuh"
 #include "align.cuh"
+#include "speaker.cuh"
 
 using namespace tts;
 
@@ -33,11 +34,20 @@ struct Ws {
     size_t total = 0;
     size_t self_kv, cross_kv, mel_before, stop_logits, lens, finished, scalars, ts, utt_ids, tlens;
     size_t x, x2, wide, a, y, mel16, mel32, ph, plens, mlens;         // sequence-parallel activations
+    size_t sids, spembs, cond, nhat;                                  // speaker conditioning (cond_dim >= 0 only)
     int Tpad, Spad, nblk_self, nblk_cross;
+    bool has_cond = false;
     size_t self_kv_bytes, cross_kv_bytes;
-    static Ws make(int B, int S, int T) {
+    // cond_dim >= 0: the handle is speaker-conditioned with x-vectors of cond_dim floats (0: speaker ids only).  Its region comes
+    // first, so that tts_set_conditioning finds it from B alone; an unconditioned layout is unchanged.
+    static Ws make(int B, int S, int T, int cond_dim = -1) {
         Ws w; size_t o = 0;
         auto take = [&](size_t bytes) { size_t r = o; o = align_up(o + bytes); return r; };
+        if (cond_dim >= 0) {
+            w.has_cond = true;
+            w.sids = take((size_t)B * 4); w.spembs = take((size_t)B * cond_dim * 4 + 4);
+            w.cond = take((size_t)B * kDModel * 4); w.nhat = take((size_t)B * cond_dim * 4 + 4);
+        }
         const size_t P = (size_t)B * kHeads;
         const size_t M = (size_t)B * (size_t)(S > T ? S : T);
         w.Tpad = (T + 15) / 16 * 16; w.Spad = (S + 15) / 16 * 16;
@@ -90,6 +100,10 @@ struct TtsHandle {
     float *pre_b1, *pre_b2, *pre_bp, *head_b;
     bf16* post_w[5] = {}; float* post_b[5] = {};
     float* pe = nullptr;
+    float *spk_table = nullptr, *spk_w = nullptr, *spk_b = nullptr;  // fp32 speaker-ID table [n_speakers][512], x-vector projection [512][D] + bias
+    // conditioning staged by tts_set_conditioning / tts_train_set_conditioning into (ws, B); the next call on that workspace that
+    // encodes consumes it, so a forgotten call can never reuse the previous batch's voices
+    struct CondRecord { void* ws = nullptr; int B = 0; } cond_inf, cond_train;
     // ---- decode session: set up by tts_decode_begin, ended by the next tts_decode_begin or tts_finalize_weights
     struct DecodeSession {
         bool active = false; int B = 0, S = 0, T = 0, t = 0;          // T = max_len; t: frames decoded (upper bound until tts_decode_status)
@@ -100,6 +114,10 @@ struct TtsHandle {
     TtsTrain* train = nullptr;                                        // training state (train.cuh), built by tts_train_begin
     int train_graph = 1;                                              // replay the train step from a CUDA graph (option "train_graph")
 };
+
+static bool conditioned(const TtsHandle* h) { return h->cfg.n_speakers > 0 || h->cfg.spk_embed_dim > 0; }
+// the inference workspace layout of this handle (with the conditioning region iff the handle is conditioned)
+static Ws ws_layout(const TtsHandle* h, int B, int S, int T) { return Ws::make(B, S, T, conditioned(h) ? h->cfg.spk_embed_dim : -1); }
 
 #define CK(call)                                                                                     \
     do {                                                                                             \
@@ -128,7 +146,14 @@ extern "C" unsigned long long tts_launch_count(void) { return launch_counter(); 
 extern "C" const char* tts_last_error_string(TtsHandle* h) { return h ? h->err.c_str() : "null handle"; }
 
 extern "C" int tts_create(const TtsConfig* cfg, int device, TtsHandle** out) {
-    if (!cfg || !out || cfg->struct_size != sizeof(TtsConfig)) return TTS_E_ARG;
+    // the size before n_speakers (callers built against the unconditioned ABI) means an unconditioned model
+    if (!cfg || !out || (cfg->struct_size != sizeof(TtsConfig) && cfg->struct_size != offsetof(TtsConfig, n_speakers))) return TTS_E_ARG;
+    TtsConfig c;
+    memset(&c, 0, sizeof(c));
+    memcpy(&c, cfg, cfg->struct_size);
+    c.struct_size = sizeof(TtsConfig);
+    cfg = &c;
+    if (cfg->n_speakers < 0 || cfg->n_speakers > kSpkMaxSpeakers || cfg->spk_embed_dim < 0 || cfg->spk_embed_dim > kSpkMaxDim) return TTS_E_ARG;
     if (cfg->d_model != 512 || cfg->n_heads != 8 || cfg->d_ff != 2048 || cfg->n_mels != 80 || cfg->d_prenet != 256 ||
         cfg->conv_kernel != 5 || cfg->n_enc_layers != 6 || cfg->n_dec_layers != 6 || cfg->enc_conv_layers != 3 ||
         cfg->postnet_layers != 5 || cfg->postnet_channels != 512 || cfg->max_pos < 1 || cfg->n_vocab < 1 ||
@@ -345,6 +370,12 @@ extern "C" int tts_finalize_weights(TtsHandle* h) {
         bind(&h->head_w, pack_rowmajor(ar, w.data(), 81, D, 1, 128, D, nullptr));
         bind(&h->head_b, pack_f32(ar, b.data(), 81, 128));
     }
+    h->spk_table = h->spk_w = h->spk_b = nullptr;                       // speaker conditioning, kept fp32 (speaker.cuh)
+    if (c.n_speakers > 0) { GET(e, "speaker_embed.weight", (size_t)c.n_speakers * D); bind(&h->spk_table, pack_f32(ar, e, (size_t)c.n_speakers * D)); }
+    if (c.spk_embed_dim > 0) {
+        GET(w, "spk_proj.weight", (size_t)D * c.spk_embed_dim); GET(b, "spk_proj.bias", (size_t)D);
+        bind(&h->spk_w, pack_f32(ar, w, (size_t)D * c.spk_embed_dim)); bind(&h->spk_b, pack_f32(ar, b, D));
+    }
     if (!h->pe) {   // P4 sinusoid table, fp32 rounded from float64 (same definition as oracle.sinusoid_table).  Its own allocation,
                     // made once per handle: a captured training graph and a live decode session keep its address across re-finalisation
         std::vector<float> pe((size_t)c.max_pos * D);
@@ -412,7 +443,7 @@ extern "C" int tts_finalize_weights(TtsHandle* h) {
 
 extern "C" size_t tts_workspace_bytes(TtsHandle* h, int B, int S, int T) {
     if (!h || B <= 0 || S <= 0 || T <= 0) return 0;
-    return Ws::make(B, S, T).total;
+    return ws_layout(h, B, S, T).total;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -437,17 +468,21 @@ AttnParams ap_packed(const bf16* Q, int ldq, const bf16* K, int ldk, const bf16*
     return a;
 }
 cudaError_t layernorm(const float* x, const float* g, const float* b, bf16* o16, float* o32, int M, float eps, cudaStream_t st) {
-    layernorm512_kernel<<<(M + 7) / 8, 256, 0, st>>>(x, g, b, o16, o32, M, eps);
+    layernorm512_kernel<false><<<(M + 7) / 8, 256, 0, st>>>(x, g, b, o16, o32, M, eps, nullptr, 0);
     ++launch_counter();
     return cudaGetLastError();
 }
 }  // namespace
 
-// Encoder (C1-C4) + hoisted cross-K/V projection.  Result: memory in ws.x (bf16 [B*S][512]).
+// Encoder (C1-C4) + hoisted cross-K/V projection.  Result: memory in ws.x (bf16 [B*S][512]).  A conditioned layout adds the speaker
+// vector of every utterance (speaker.cuh, from the inputs staged by tts_set_conditioning) inside the last LayerNorm.
 static int run_encoder(TtsHandle* h, void* ws, const Ws& L, const int64_t* ph, const int* plens, int B, int S, bool v_blocked, cudaStream_t st) {
     const int M = B * S;
     bf16 *x = wsp<bf16>(ws, L.x), *x2 = wsp<bf16>(ws, L.x2), *wide = wsp<bf16>(ws, L.wide), *a = wsp<bf16>(ws, L.a);
     float* y = wsp<float>(ws, L.y);
+    if (L.has_cond)
+        CK(launch_speaker_cond(wsp<int>(ws, L.sids), wsp<float>(ws, L.spembs), B, h->cfg.n_speakers, h->cfg.spk_embed_dim, h->spk_table, h->spk_w,
+                               h->spk_b, wsp<float>(ws, L.cond), wsp<float>(ws, L.nhat), st));
     embed_kernel<<<(M + 3) / 4, 256, 0, st>>>(ph, plens, h->embed, x, B, S, h->cfg.n_vocab);
     ++launch_counter();
     CK(cudaGetLastError());
@@ -476,7 +511,8 @@ static int run_encoder(TtsHandle* h, void* ws, const Ws& L, const int64_t* ph, c
         CK(launch_gemm_tc(p, st));
         p = gp(wide, 2048, W.w2, 2048, M, 512, 2048); p.bias = W.b2; p.resid_bf16 = x; p.ldr = 512; p.out_f32 = y; p.ldo = 512;
         CK(launch_gemm_tc(p, st));
-        CK(layernorm(y, W.ln2g, W.ln2b, x, nullptr, M, h->cfg.ln_eps, st));
+        if (l == 5 && L.has_cond) CK(launch_layernorm_cond(y, W.ln2g, W.ln2b, x, nullptr, M, h->cfg.ln_eps, wsp<float>(ws, L.cond), S, st));
+        else CK(layernorm(y, W.ln2g, W.ln2b, x, nullptr, M, h->cfg.ln_eps, st));
     }
     if (x != wsp<bf16>(ws, L.x)) {                                     // keep memory in ws.x
         CK(cudaMemcpyAsync(wsp<bf16>(ws, L.x), x, (size_t)M * 512 * 2, cudaMemcpyDeviceToDevice, st));
@@ -514,14 +550,44 @@ static int run_postnet(TtsHandle* h, void* ws, const Ws& L, const int* mlens, in
 }
 
 // ------------------------------------------------------------------------------------------------
+// Consumes the conditioning record of a conditioned handle: it must name this workspace and batch size.
+static int take_conditioning(TtsHandle* h, TtsHandle::CondRecord& rec, void* ws, int B, const char* setter) {
+    if (!conditioned(h)) return 0;
+    if (rec.ws != ws || rec.B != B) FAIL(TTS_E_STATE, std::string("speaker-conditioned model: ") + setter + " must stage this batch's speakers first");
+    rec = TtsHandle::CondRecord();
+    return 0;
+}
+// Copies sids int32 [B] / spembs fp32 [B][spk_embed_dim] (device) into the conditioning region at the start of ws.
+static int stage_conditioning(TtsHandle* h, void* ws, int B, const int32_t* sids, const float* spembs, size_t sids_off, size_t spembs_off,
+                              cudaStream_t st) {
+    if (!ws || B <= 0) return TTS_E_ARG;
+    if (!conditioned(h)) FAIL(TTS_E_STATE, "the model has no speaker conditioning (n_speakers = spk_embed_dim = 0)");
+    if (!sids != !(h->cfg.n_speakers > 0)) FAIL(TTS_E_ARG, "sids must be given exactly when n_speakers > 0");
+    if (!spembs != !(h->cfg.spk_embed_dim > 0)) FAIL(TTS_E_ARG, "spembs must be given exactly when spk_embed_dim > 0");
+    if (sids) CK(cudaMemcpyAsync(wsp<int>(ws, sids_off), sids, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
+    if (spembs) CK(cudaMemcpyAsync(wsp<float>(ws, spembs_off), spembs, (size_t)B * h->cfg.spk_embed_dim * 4, cudaMemcpyDeviceToDevice, st));
+    return 0;
+}
+
+extern "C" int tts_set_conditioning(TtsHandle* h, void* ws, int B, const int32_t* sids, const float* spembs, void* stream) {
+    if (!h) return TTS_E_ARG;
+    DEV_GUARD(h);
+    const Ws L = Ws::make(B, 1, 1, h->cfg.spk_embed_dim);            // the region's offsets depend on B only
+    int r = stage_conditioning(h, ws, B, sids, spembs, L.sids, L.spembs, (cudaStream_t)stream);
+    if (r) return r;
+    h->cond_inf = {ws, B};
+    return 0;
+}
+
 extern "C" int tts_encode(TtsHandle* h, void* ws, const int64_t* phonemes, const int32_t* phoneme_lens, int B, int S, int T,
                           float* memory_out, void* stream) {
     if (!h || !ws || !phonemes || !phoneme_lens || B <= 0 || S <= 0 || T <= 0) return TTS_E_ARG;
     if (!h->finalized) FAIL(TTS_E_STATE, "weights not finalised");
     if (S > h->cfg.max_pos) FAIL(TTS_E_ARG, "S exceeds max_pos");
     DEV_GUARD(h);
+    if (int r = take_conditioning(h, h->cond_inf, ws, B, "tts_set_conditioning")) return r;
     cudaStream_t st = (cudaStream_t)stream;
-    const Ws L = Ws::make(B, S, T);
+    const Ws L = ws_layout(h, B, S, T);
     // the decode phases read the key-padding lengths from the workspace copy
     CK(cudaMemcpyAsync(wsp<int>(ws, L.plens), phoneme_lens, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
     int r = run_encoder(h, ws, L, phonemes, wsp<int>(ws, L.plens), B, S, true, st);
@@ -543,7 +609,7 @@ extern "C" int tts_decode_begin(TtsHandle* h, void* ws, int B, int S, int max_le
     cudaStream_t st = (cudaStream_t)stream;
     auto& ds = h->session;
     ds.active = true; ds.B = B; ds.S = S; ds.T = max_len; ds.t = 0; ds.t_status = -1; ds.frontier = 0;
-    ds.L = Ws::make(B, S, max_len);
+    ds.L = ws_layout(h, B, S, max_len);
     const Ws& L = ds.L;
     init_decode_state_kernel<<<(std::max(B, 4) + 255) / 256, 256, 0, st>>>(wsp<int>(ws, L.lens), wsp<int>(ws, L.finished),
                                                                           wsp<int>(ws, L.scalars), B, max_len);
@@ -776,6 +842,7 @@ extern "C" int tts_infer_host(TtsHandle* h, void* ws, const int64_t* phonemes, c
     if (!h->finalized) FAIL(TTS_E_STATE, "weights not finalised");
     if (S > h->cfg.max_pos) FAIL(TTS_E_ARG, "S exceeds max_pos");              // checked before any copy or launch
     if (max_len > h->cfg.max_pos) FAIL(TTS_E_ARG, "max_len exceeds max_pos");
+    if (conditioned(h)) FAIL(TTS_E_STATE, "speaker-conditioned model: use the device path (tts_set_conditioning, tts_encode, tts_decode_*)");
     DEV_GUARD(h);
     cudaStream_t st = (cudaStream_t)stream;
     const Ws L = Ws::make(B, S, max_len);
@@ -902,7 +969,8 @@ extern "C" int tts_forward(TtsHandle* h, void* ws, const int64_t* phonemes, cons
     if (!h->finalized) FAIL(TTS_E_STATE, "weights not finalised");
     if (S > h->cfg.max_pos || T > h->cfg.max_pos) FAIL(TTS_E_ARG, "sequence exceeds max_pos");
     DEV_GUARD(h);
-    return run_teacher_forced(h, ws, Ws::make(B, S, T), phonemes, phoneme_lens, mels, mel_lens, B, S, T, seed, utt_offset, mel_before,
+    if (int r = take_conditioning(h, h->cond_inf, ws, B, "tts_set_conditioning")) return r;
+    return run_teacher_forced(h, ws, ws_layout(h, B, S, T), phonemes, phoneme_lens, mels, mel_lens, B, S, T, seed, utt_offset, mel_before,
                               mel_after, stop_logits, nullptr, (cudaStream_t)stream);
 }
 
@@ -942,10 +1010,11 @@ extern "C" int tts_forward_align(TtsHandle* h, void* ws, void* scratch, const in
     const bool stats = focus || durations || head;
     if (stats && !scratch) FAIL(TTS_E_ARG, "focus / durations / head need the scratch of tts_align_scratch_bytes");
     DEV_GUARD(h);
+    if (int r = take_conditioning(h, h->cond_inf, ws, B, "tts_set_conditioning")) return r;
     cudaStream_t st = (cudaStream_t)stream;
     const AlignScratch A = AlignScratch::make(B, T);
     AlignSink sink{layer_mask, align, stats ? wsp<float>(scratch, A.rowmax) : nullptr, stats ? wsp<int16_t>(scratch, A.argmax) : nullptr};
-    int r = run_teacher_forced(h, ws, Ws::make(B, S, T), phonemes, phoneme_lens, mels, mel_lens, B, S, T, seed, utt_offset, mel_before,
+    int r = run_teacher_forced(h, ws, ws_layout(h, B, S, T), phonemes, phoneme_lens, mels, mel_lens, B, S, T, seed, utt_offset, mel_before,
                                mel_after, stop_logits, (align || stats) ? &sink : nullptr, st);
     if (r) return r;
     float* f = focus ? focus : wsp<float>(scratch, A.focus);
@@ -1092,6 +1161,25 @@ extern "C" int tts_k_layernorm(const float* X, const float* gamma, const float* 
     if (!X || !gamma || !beta || !Y || M <= 0) return TTS_E_ARG;
     return (int)layernorm(X, gamma, beta, (bf16*)Y, nullptr, M, eps, (cudaStream_t)stream);
 }
+extern "C" int tts_k_speaker_cond(const int32_t* sids, const float* spembs, int B, int n_speakers, int D, const float* table, const float* W,
+                                  const float* bias, float* cond, float* nhat, void* stream) {
+    if (!cond || B <= 0 || n_speakers < 0 || D < 0 || D > kSpkMaxDim || (!table && !W) || (table && (!sids || n_speakers == 0)) ||
+        (!W != (D == 0)) || (W && (!bias || !spembs || !nhat)))
+        return TTS_E_ARG;
+    return (int)launch_speaker_cond(sids, spembs, B, n_speakers, D, table, W, bias, cond, nhat, (cudaStream_t)stream);
+}
+extern "C" int tts_k_layernorm_cond(const float* X, const float* gamma, const float* beta, const float* cond, void* Y, int M, int S, float eps,
+                                    void* stream) {
+    if (!X || !gamma || !beta || !cond || !Y || M <= 0 || S <= 0) return TTS_E_ARG;
+    return (int)launch_layernorm_cond(X, gamma, beta, (bf16*)Y, nullptr, M, eps, cond, S, (cudaStream_t)stream);
+}
+extern "C" int tts_k_speaker_cond_bwd(const float* dmem, const int32_t* plens, const int32_t* sids, const float* nhat, int B, int S, int n_speakers,
+                                      int D, float* dcond, float* dE, float* dW, float* dbias, void* stream) {
+    if (!dmem || !plens || !dcond || B <= 0 || S <= 0 || n_speakers < 0 || D < 0 || (!dE && !dW) || (dE && (!sids || n_speakers == 0)) ||
+        (!dW != (D == 0)) || (dW && (!dbias || !nhat)))
+        return TTS_E_ARG;
+    return (int)launch_speaker_cond_bwd(dmem, plens, sids, nhat, B, S, n_speakers, D, dcond, dE, dW, dbias, (cudaStream_t)stream);
+}
 extern "C" int tts_k_philox_bits(uint64_t seed, int site, int T, int B, int C, int utt_offset, uint8_t* out, void* stream) {
     if (!out || T <= 0 || B <= 0 || C <= 0) return TTS_E_ARG;
     const int n = T * B * C;
@@ -1199,14 +1287,14 @@ extern "C" int tts_train_begin(TtsHandle* h) {
 extern "C" int tts_train_end(TtsHandle* h) { if (!h) return TTS_E_ARG; DeviceGuard dev_guard_(h->device); return train_free(h); }
 extern "C" size_t tts_train_workspace_bytes(TtsHandle* h, int B, int S, int T) {
     if (!h || B <= 0 || S <= 0 || T <= 0) return 0;
-    return TrWs::make(nullptr, B, S, T).total;
+    return TrWs::make(nullptr, B, S, T, conditioned(h) ? h->cfg.spk_embed_dim : -1).total;
 }
 namespace {
 // context of one training call: workspace views, dropout threshold / scale, flat parameter and gradient buffers
 TrCtx train_ctx(TtsHandle* h, void* ws, int B, int S, int T, int utt_offset, double p_residual, cudaStream_t st) {
     TrCtx c;
     TtsTrain* t = h->train;
-    c.h = h; c.t = t; c.w = TrWs::make(reinterpret_cast<unsigned char*>(ws), B, S, T); c.st = st;
+    c.h = h; c.t = t; c.w = TrWs::make(reinterpret_cast<unsigned char*>(ws), B, S, T, conditioned(h) ? h->cfg.spk_embed_dim : -1); c.st = st;
     c.B = B; c.S = S; c.T = T; c.seed = c.w.seed_dev; c.utt0 = utt_offset;
     c.thresh = (uint32_t)(p_residual * 4294967296.0); c.dscale = 1.0f / (float)(1.0 - p_residual);
     c.P = t->P; c.G = t->G;
@@ -1220,6 +1308,7 @@ int train_stage(TrCtx& c, TtsHandle* h, void* ws, const int64_t* phonemes, const
     if (!h->train) FAIL(TTS_E_STATE, "tts_train_begin has not been called");
     if (S > h->cfg.max_pos || T > h->cfg.max_pos) FAIL(TTS_E_ARG, "sequence exceeds max_pos");
     if (p_residual < 0.0 || p_residual >= 1.0) FAIL(TTS_E_ARG, "p_residual out of range");
+    if (int r = take_conditioning(h, h->cond_train, ws, B, "tts_train_set_conditioning")) return r;
     c = train_ctx(h, ws, B, S, T, utt_offset, p_residual, st);
     CK(cudaMemcpyAsync(c.w.plens, phoneme_lens, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
     CK(cudaMemcpyAsync(c.w.mlens, mel_lens, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
@@ -1230,6 +1319,16 @@ int train_stage(TrCtx& c, TtsHandle* h, void* ws, const int64_t* phonemes, const
     return 0;
 }
 }  // namespace
+extern "C" int tts_train_set_conditioning(TtsHandle* h, void* ws, int B, const int32_t* sids, const float* spembs, void* stream) {
+    if (!h) return TTS_E_ARG;
+    if (!h->train) FAIL(TTS_E_STATE, "tts_train_begin has not been called");
+    DEV_GUARD(h);
+    const TrWs w = TrWs::make(nullptr, B, 1, 1, h->cfg.spk_embed_dim);  // the region's offsets depend on B only
+    int r = stage_conditioning(h, ws, B, sids, spembs, (size_t)w.sids, (size_t)w.spembs, (cudaStream_t)stream);
+    if (r) return r;
+    h->cond_train = {ws, B};
+    return 0;
+}
 extern "C" int tts_train_step(TtsHandle* h, void* ws, const int64_t* phonemes, const int32_t* phoneme_lens, const float* mels, const int32_t* mel_lens,
                               int B, int S, int T, uint64_t seed, int utt_offset, double p_residual, float pos_weight, float* loss_out, void* stream) {
     if (!h || !loss_out) return TTS_E_ARG;
@@ -1305,7 +1404,7 @@ extern "C" int tts_train_write(TtsHandle* h, int which, int64_t offset, int64_t 
 }
 extern "C" int tts_train_outputs(TtsHandle* h, void* ws, int B, int S, int T, float* mel_before, float* mel_after, float* stop_logits, void* stream) {
     if (!h || !ws || !h->train) return TTS_E_ARG;
-    TrWs w = TrWs::make(reinterpret_cast<unsigned char*>(ws), B, S, T);
+    TrWs w = TrWs::make(reinterpret_cast<unsigned char*>(ws), B, S, T, conditioned(h) ? h->cfg.spk_embed_dim : -1);
     cudaStream_t st = (cudaStream_t)stream;
     if (mel_before) CK(cudaMemcpyAsync(mel_before, w.mel_before, (size_t)B * T * 80 * 4, cudaMemcpyDeviceToDevice, st));
     if (mel_after) CK(cudaMemcpyAsync(mel_after, w.mel_after, (size_t)B * T * 80 * 4, cudaMemcpyDeviceToDevice, st));

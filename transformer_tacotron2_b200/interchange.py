@@ -6,7 +6,12 @@ mel-spectrograms to vocoders in the layout they expect.
 Only POST-LayerNorm checkpoints can be imported (the oracle pins post-LN without final norms, SURVEY.md 8-P P1): a checkpoint that
 carries `encoder.after_norm` / `decoder.after_norm` was trained with `normalize_before=True`, its arithmetic differs, and the import
 refuses it instead of producing a model that silently computes something else.  The same holds for reduction factors != 1 and for
-layer counts / widths other than the base model's."""
+layer counts / widths other than the base model's.
+
+Multi-speaker checkpoints (VCTK, LibriTTS, ...) carry a speaker-ID table `sid_emb.weight` and / or an x-vector projection
+`projection.{weight,bias}`; they map to `speaker_embed.weight` / `spk_proj.*` of a model built with TTSConfig(n_speakers=...,
+spk_embed_dim=...).  Only spk_embed_integration_type "add" is supported; language ids (`lid_emb`) and global style tokens (`gst`)
+are refused."""
 from __future__ import annotations
 
 import re
@@ -79,10 +84,20 @@ def _map_key(k: str) -> Optional[str]:
     return ""
 
 
-def from_espnet_state_dict(src: Mapping[str, torch.Tensor], reference: Mapping[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
+_SPEAKER = {"sid_emb.weight": "speaker_embed.weight", "projection.weight": "spk_proj.weight", "projection.bias": "spk_proj.bias"}
+
+
+def from_espnet_state_dict(src: Mapping[str, torch.Tensor], reference: Mapping[str, torch.Tensor],
+                           spk_embed_integration_type: Optional[str] = None) -> Dict[str, torch.Tensor]:
     """Translate an ESPnet-style Transformer-TTS `state_dict` (optionally prefixed `tts.`) into this module's keys.
-    `reference` = `TransformerTTS().state_dict()`: every target key must be produced with the reference's shape, and
-    nothing the source contains may be left over.  Raises InterchangeError on anything that does not fit."""
+    `reference` = `TransformerTTS(cfg).state_dict()`: every target key must be produced with the reference's shape, and
+    nothing the source contains may be left over.  Raises InterchangeError on anything that does not fit.
+
+    A checkpoint with an x-vector projection (`projection.*`) needs spk_embed_integration_type="add", the value the ESPnet
+    model was trained with: the weight shapes cannot tell "add" from "concat", and only "add" is this model's arithmetic."""
+    if spk_embed_integration_type not in (None, "add"):
+        raise InterchangeError(f"spk_embed_integration_type={spk_embed_integration_type!r} is not supported: only 'add' (the speaker "
+                               "vector added to the encoder output) is this model's arithmetic")
     out: Dict[str, torch.Tensor] = {}
     unknown = []
     for k, v in src.items():
@@ -90,7 +105,14 @@ def from_espnet_state_dict(src: Mapping[str, torch.Tensor], reference: Mapping[s
         if "after_norm" in k:
             raise InterchangeError("checkpoint was trained with normalize_before=True (pre-LayerNorm + final norm): only post-LayerNorm "
                                    "Transformer-TTS checkpoints are arithmetic-compatible with this model")
-        t = _map_key(k)
+        if k.startswith("lid_emb."):
+            raise InterchangeError("checkpoint has a language-ID embedding (lid_emb): multi-lingual models are not supported")
+        if k.startswith("gst."):
+            raise InterchangeError("checkpoint has global style tokens (gst): style-token conditioning is not supported")
+        if k.startswith("projection.") and spk_embed_integration_type != "add":
+            raise InterchangeError("checkpoint has an x-vector projection (projection.*): pass spk_embed_integration_type='add' if it was "
+                                   "trained with the speaker vector added to the encoder output ('concat' is not supported)")
+        t = _SPEAKER.get(k) or _map_key(k)
         if t is None:
             continue
         if t == "":
@@ -149,6 +171,8 @@ def to_espnet_state_dict(sd: Mapping[str, torch.Tensor]) -> Dict[str, torch.Tens
         k2 = re.sub(r"^stop_linear\.", "prob_out.", k2)
         k2 = re.sub(r"^postnet\.convs\.(\d+)\.conv\.", r"postnet.postnet.\1.0.", k2)
         k2 = re.sub(r"^postnet\.convs\.(\d+)\.bn\.", r"postnet.postnet.\1.1.", k2)
+        k2 = re.sub(r"^speaker_embed\.", "sid_emb.", k2)
+        k2 = re.sub(r"^spk_proj\.", "projection.", k2)
         inv[k2] = v
     return inv
 

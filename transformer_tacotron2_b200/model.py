@@ -35,6 +35,8 @@ class TTSConfig:
     max_pos: int = 2048
     ln_eps: float = 1e-5
     bn_eps: float = 1e-5
+    n_speakers: int = 0          # > 0: speaker-ID table speaker_embed [n_speakers, 512] (ESPnet sid_emb)
+    spk_embed_dim: int = 0       # > 0: x-vector projection spk_proj [512, spk_embed_dim] (ESPnet projection, integration "add")
 
     def to_dict(self):
         return asdict(self)
@@ -152,8 +154,8 @@ class _TrainForwardFn(torch.autograd.Function):
     The module's parameters ride along as inputs so that autograd routes the flat gradient buffer back to them."""
 
     @staticmethod
-    def forward(ctx, model, trainer, phonemes, phoneme_lens, mels, mel_lens, seed, utt_offset, *params):
-        mb, ma, st = trainer.forward_only(phonemes, phoneme_lens, mels, mel_lens, seed, utt_offset)
+    def forward(ctx, model, trainer, phonemes, phoneme_lens, mels, mel_lens, seed, utt_offset, sids, spembs, *params):
+        mb, ma, st = trainer.forward_only(phonemes, phoneme_lens, mels, mel_lens, seed, utt_offset, sids=sids, spembs=spembs)
         ctx.model, ctx.trainer = model, trainer
         ctx.names = [n for n, _ in model.named_parameters()]
         ctx.pinfo = [(p.shape, p.device, p.dtype) for p in params]
@@ -170,7 +172,7 @@ class _TrainForwardFn(torch.autograd.Function):
         tr.backward_from(z(g_mb, (B, T, 80)) * mask[..., None], z(g_ma, (B, T, 80)) * mask[..., None], z(g_st, (B, T)) * mask)
         grads = tr.grads()                                                                               # name -> host tensor
         out = [grads[n].to(dev, dt).view(shape) for n, (shape, dev, dt) in zip(ctx.names, ctx.pinfo)]
-        return (None,) * 8 + tuple(out)
+        return (None,) * 10 + tuple(out)
 
 
 class TransformerTTS(nn.Module):
@@ -191,6 +193,12 @@ class TransformerTTS(nn.Module):
         self.mel_linear = nn.Linear(c.d_model, c.n_mels)
         self.stop_linear = nn.Linear(c.d_model, 1)
         self.postnet = _Postnet(c)
+        # created after every other sub-module: the base parameters, their state_dict order and their seeded initial values
+        # are those of the unconditioned model
+        if c.n_speakers > 0:
+            self.speaker_embed = nn.Embedding(c.n_speakers, c.d_model)
+        if c.spk_embed_dim > 0:
+            self.spk_proj = nn.Linear(c.spk_embed_dim, c.d_model)
         self._device_index = device
         self._lib = None
         self._handle = C.c_void_p()
@@ -217,7 +225,7 @@ class TransformerTTS(nn.Module):
             c = self.cfg
             cc = _lib.TtsConfig(C.sizeof(_lib.TtsConfig), c.n_vocab, c.d_model, c.n_heads, c.n_enc_layers, c.n_dec_layers,
                                 c.d_ff, c.n_mels, c.d_prenet, c.enc_conv_layers, c.conv_kernel, c.postnet_channels,
-                                c.postnet_layers, c.max_pos, c.ln_eps, c.bn_eps)
+                                c.postnet_layers, c.max_pos, c.ln_eps, c.bn_eps, c.n_speakers, c.spk_embed_dim)
             rc = self._lib.tts_create(C.byref(cc), self._device_index, C.byref(self._handle))
             if rc != 0:
                 raise _lib.TtsError(f"tts_create failed ({rc}): no sm_100 device {self._device_index}?")
@@ -305,6 +313,49 @@ class TransformerTTS(nn.Module):
         inputs = ((phonemes, torch.int64), (phoneme_lens, torch.int32), (mels, torch.float32), (mel_lens, torch.int32))
         return tuple(t.to(self.device, dt).contiguous() for t, dt in inputs if t is not None)
 
+    @property
+    def conditioned(self) -> bool:
+        """True for a multi-speaker model (n_speakers > 0 or spk_embed_dim > 0)."""
+        return self.cfg.n_speakers > 0 or self.cfg.spk_embed_dim > 0
+
+    def _speaker_inputs(self, sids, spembs, B):
+        """Checks sids [B] (integers in [0, n_speakers)) and spembs [B, spk_embed_dim] (floating) against the config and returns
+        them staged on the device as int32 / fp32 (None for the absent one), or None for an unconditioned model.  ValueError when a
+        conditioned model lacks one it needs, an unconditioned model gets one, or a shape, dtype or id is wrong."""
+        c = self.cfg
+        if not self.conditioned:
+            if sids is not None or spembs is not None:
+                raise ValueError("sids / spembs given to a model without speaker conditioning (n_speakers = spk_embed_dim = 0)")
+            return None
+        out = []
+        for name, t, need, shape in (("sids", sids, c.n_speakers > 0, (B,)), ("spembs", spembs, c.spk_embed_dim > 0, (B, c.spk_embed_dim))):
+            if t is None:
+                if need:
+                    raise ValueError(f"this multi-speaker model needs {name} (n_speakers = {c.n_speakers}, spk_embed_dim = {c.spk_embed_dim})")
+                out.append(None)
+                continue
+            if not need:
+                raise ValueError(f"{name} given, but the model has no {'speaker-ID table' if name == 'sids' else 'x-vector projection'}")
+            t = torch.as_tensor(t)
+            if tuple(t.shape) != shape:
+                raise ValueError(f"{name} must have shape {shape}, got {tuple(t.shape)}")
+            if name == "sids":
+                if t.is_floating_point() or t.is_complex() or t.dtype == torch.bool:
+                    raise ValueError(f"sids must be an integer tensor, got {t.dtype}")
+                lo, hi = int(t.min()), int(t.max())
+                if lo < 0 or hi >= c.n_speakers:
+                    raise ValueError(f"sids must lie in [0, {c.n_speakers}), got values in [{lo}, {hi}]")
+            elif not t.is_floating_point():
+                raise ValueError(f"spembs must be a floating-point tensor, got {t.dtype}")
+            out.append(t)
+        return tuple(None if t is None else t.to(self.device, dt).contiguous() for t, dt in zip(out, (torch.int32, torch.float32)))
+
+    def _stage_speakers(self, ws, spk, B, stream):
+        """tts_set_conditioning for a conditioned model (spk from _speaker_inputs); nothing for an unconditioned one."""
+        if spk is not None:
+            ptr = lambda t: None if t is None else t.data_ptr()                                           # noqa: E731
+            self._check(self._lib.tts_set_conditioning(self._handle, ws.data_ptr(), B, ptr(spk[0]), ptr(spk[1]), stream), "tts_set_conditioning")
+
     @staticmethod
     def _utt_ids(utt_ids, B, utt_offset, contiguous=False):
         """-> (offset, ids or None).  A contiguous range of utterance ids is just the offset of utterance 0; any other ids come
@@ -319,29 +370,35 @@ class TransformerTTS(nn.Module):
         return int(utt_offset), ids
 
     # ------------------------------------------------------------------ teacher-forced
-    def forward(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_ids=None, utt_offset: int = 0
+    def forward(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_ids=None, utt_offset: int = 0, sids=None, spembs=None
                 ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
         """phonemes [B,S] i64, phoneme_lens [B], mels [B,T,80] f32, mel_lens [B]
-        -> mel_before [B,T,80], mel_after [B,T,80], stop_logits [B,T]  (on the GPU, zero past mel_lens)."""
+        -> mel_before [B,T,80], mel_after [B,T,80], stop_logits [B,T]  (on the GPU, zero past mel_lens).
+        Multi-speaker models take sids [B] (speaker ids, n_speakers > 0) and / or spembs [B, spk_embed_dim] (x-vectors, spk_embed_dim
+        > 0); every path of the module takes them the same way.  spembs are inputs: they get no gradient."""
         if self.training:
             return self._train_forward(phonemes, phoneme_lens, mels, mel_lens, seed,
-                                       self._utt_ids(utt_ids, phonemes.shape[0], utt_offset, contiguous=True)[0])
+                                       self._utt_ids(utt_ids, phonemes.shape[0], utt_offset, contiguous=True)[0], sids, spembs)
         with torch.no_grad():
-            return self._eval_forward(phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset)
+            return self._eval_forward(phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset, sids, spembs)
 
-    def _teacher_forced_setup(self, phonemes, phoneme_lens, mels, mel_lens, utt_ids, utt_offset):
-        """Set-up shared by tts_forward and tts_forward_align.  -> lib, workspace, staged (ph, pl, mels, mel_lens), (B, S, T),
-        offset of utterance 0."""
+    def _teacher_forced_setup(self, phonemes, phoneme_lens, mels, mel_lens, utt_ids, utt_offset, sids, spembs):
+        """Set-up shared by tts_forward and tts_forward_align (the batch's speakers staged last).  -> lib, workspace, staged (ph, pl,
+        mels, mel_lens), (B, S, T), offset of utterance 0."""
         lib = self._ensure_handle()
-        self.sync_weights()
         B, S = phonemes.shape
+        spk = self._speaker_inputs(sids, spembs, B)
+        self.sync_weights()
         T = mels.shape[1]
         inputs = self._stage_inputs(phonemes, phoneme_lens, mels, mel_lens)
         ws = self._workspace(B, S, T)
-        return lib, ws, inputs, (B, S, T), self._utt_ids(utt_ids, B, utt_offset, contiguous=True)[0]
+        u0 = self._utt_ids(utt_ids, B, utt_offset, contiguous=True)[0]
+        self._stage_speakers(ws, spk, B, self._stream())
+        return lib, ws, inputs, (B, S, T), u0
 
-    def _eval_forward(self, phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset):
-        lib, ws, (ph, pl, m, ml), (B, S, T), u0 = self._teacher_forced_setup(phonemes, phoneme_lens, mels, mel_lens, utt_ids, utt_offset)
+    def _eval_forward(self, phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset, sids, spembs):
+        lib, ws, (ph, pl, m, ml), (B, S, T), u0 = self._teacher_forced_setup(phonemes, phoneme_lens, mels, mel_lens, utt_ids, utt_offset,
+                                                                              sids, spembs)
         dev = self.device
         mb = torch.empty(B, T, 80, device=dev); ma = torch.empty(B, T, 80, device=dev); st = torch.empty(B, T, device=dev)
         rc = lib.tts_forward(self._handle, ws.data_ptr(), ph.data_ptr(), pl.data_ptr(), m.data_ptr(), ml.data_ptr(), B, S, T,
@@ -351,8 +408,8 @@ class TransformerTTS(nn.Module):
 
     # ------------------------------------------------------------------ cross-attention alignments / durations
     @torch.no_grad()
-    def alignments(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_ids=None, utt_offset: int = 0, layers=None
-                   ) -> torch.Tensor:
+    def alignments(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_ids=None, utt_offset: int = 0, layers=None,
+                   sids=None, spembs=None) -> torch.Tensor:
         """Encoder-decoder attention of the teacher-forced forward (eval mode): [n_layers, B, 8, T, S] fp32, P[l, b, h, t, s] =
         softmax_s(q_t . k_s / 8) of decoder layer layers[l] (default: all six, ascending), zero at frames t >= mel_lens[b] and
         phonemes s >= phoneme_lens[b].  Same inputs as forward(); CUDA tensors in -> CUDA tensor out, CPU in -> CPU out.
@@ -361,12 +418,12 @@ class TransformerTTS(nn.Module):
         `model.alignments(ph, pl, mb, lens)` with the same seed -- the teacher-forced decoder then sees exactly the frames the
         AR decoder fed back (shifted right behind the zero go-frame, same prenet dropout masks)."""
         ls, mask = self._align_layers(layers)
-        out = self._forward_align(phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset, mask, -1, True, False)
+        out = self._forward_align(phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset, mask, -1, True, False, sids, spembs)
         return out["align"] if phonemes.is_cuda else out["align"].cpu()
 
     @torch.no_grad()
     def durations(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_ids=None, utt_offset: int = 0, layers=None,
-                  head: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+                  head: Optional[int] = None, sids=None, spembs=None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
         """FastSpeech duration targets from the teacher-forced cross-attention (Ren et al., 2019, section 3.3; ESPnet's
         DurationCalculator), computed on the GPU without forming P in memory.
         -> durations [B, S] int32 (frames t < mel_lens[b] whose most-attended phoneme is s; sums to mel_lens[b]),
@@ -377,7 +434,7 @@ class TransformerTTS(nn.Module):
         fixed = -1 if head is None else int(head)
         if fixed != -1 and not (0 <= fixed < 48 and fixed // 8 in ls):
             raise ValueError("head must be layer * 8 + h of a selected layer")
-        out = self._forward_align(phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset, mask, fixed, False, True)
+        out = self._forward_align(phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset, mask, fixed, False, True, sids, spembs)
         res = (out["durations"], out["head"], out["focus"])
         return res if phonemes.is_cuda else tuple(t.cpu() for t in res)
 
@@ -389,10 +446,11 @@ class TransformerTTS(nn.Module):
         return ls, sum(1 << v for v in ls)
 
     def _forward_align(self, phonemes, phoneme_lens, mels, mel_lens, seed, utt_ids, utt_offset, layer_mask, fixed_head,
-                       want_align, want_durations):
+                       want_align, want_durations, sids, spembs):
         if self.training:
             raise RuntimeError("alignments() / durations() are eval-mode paths: call model.eval() first")
-        lib, ws, (ph, pl, m, ml), (B, S, T), u0 = self._teacher_forced_setup(phonemes, phoneme_lens, mels, mel_lens, utt_ids, utt_offset)
+        lib, ws, (ph, pl, m, ml), (B, S, T), u0 = self._teacher_forced_setup(phonemes, phoneme_lens, mels, mel_lens, utt_ids, utt_offset,
+                                                                              sids, spembs)
         dev = self.device
         out, scratch = {}, None
         if want_align:
@@ -410,7 +468,7 @@ class TransformerTTS(nn.Module):
         self._check(rc, "tts_forward_align")
         return out
 
-    def _train_forward(self, phonemes, phoneme_lens, mels, mel_lens, seed, utt_offset):
+    def _train_forward(self, phonemes, phoneme_lens, mels, mel_lens, seed, utt_offset, sids, spembs):
         """Train-mode forward with autograd: `model.train(); out = model(...); loss_fn(*out).backward(); optimiser.step()` works on
         the module exactly as on the oracle (oracle/transformer_tts.py: forward in .train() mode).  Arithmetic: the library's
         training forward / backward (tts_train_forward / tts_train_backward); gradients are copied into the (host) parameters'
@@ -425,7 +483,8 @@ class TransformerTTS(nn.Module):
             elif self._ag_version != self._param_version():          # an optimiser (or the user) changed the module's tensors
                 tr.write_parameters(self._raw_state_dict())
                 self._ag_version = self._param_version()
-        out = _TrainForwardFn.apply(self, tr, phonemes, phoneme_lens, mels, mel_lens, int(seed), int(utt_offset), *list(self.parameters()))
+        out = _TrainForwardFn.apply(self, tr, phonemes, phoneme_lens, mels, mel_lens, int(seed), int(utt_offset), sids, spembs,
+                                    *list(self.parameters()))
         with torch.no_grad():                                        # BatchNorm running statistics moved in the forward: mirror them
             sd = self._raw_state_dict()
             for k, v in tr.buffers().items():
@@ -435,21 +494,22 @@ class TransformerTTS(nn.Module):
         return out
 
     # ------------------------------------------------------------------ greedy AR
-    def _start_decode(self, ws, ph, pl, max_len, seed, utt_offset, ids, max_lens, work_stealing, stream):
+    def _start_decode(self, ws, ph, pl, max_len, seed, utt_offset, ids, max_lens, work_stealing, spk, stream):
         """Opens a decode session in `ws` and encodes the batch: tts_decode_begin, tts_decode_set_batch when there are per-utterance
-        ids or frame budgets (device int32 tensors or None), tts_encode."""
+        ids or frame budgets (device int32 tensors or None), tts_set_conditioning for a multi-speaker model, tts_encode."""
         lib, h, wsp = self._lib, self._handle, ws.data_ptr()
         B, S = ph.shape
         self._check(lib.tts_decode_begin(h, wsp, B, S, max_len, int(seed), utt_offset, stream), "tts_decode_begin")
         if ids is not None or max_lens is not None:
             ptr = lambda t: None if t is None else t.data_ptr()                                           # noqa: E731
             self._check(lib.tts_decode_set_batch(h, wsp, ptr(ids), ptr(max_lens), int(work_stealing), stream), "tts_decode_set_batch")
+        self._stage_speakers(ws, spk, B, stream)
         self._check(lib.tts_encode(h, wsp, ph.data_ptr(), pl.data_ptr(), B, S, max_len, None, stream), "tts_encode")
 
     @torch.no_grad()
     def inference(self, phonemes, phoneme_lens, max_len: int = 800, seed: int = 0, utt_ids=None, utt_offset: int = 0,
                   return_before: bool = False, clone_outputs: bool = True, max_lens=None, sort_by_length: bool = False,
-                  work_stealing: Optional[bool] = None):
+                  work_stealing: Optional[bool] = None, sids=None, spembs=None):
         """-> mel_after [B,Tout,80], mel_lens [B] i32, stop_logits [B,Tout].
 
         CPU tensors in -> the whole call runs through tts_infer_host (H2D, encoder, decode loop,
@@ -465,14 +525,18 @@ class TransformerTTS(nn.Module):
         the latest); `sort_by_length=True` decodes the batch sorted by budget / phoneme length, so that the utterances sharing
         a cluster group stop together, and returns the results in the caller's order -- bit-identical to the unsorted call;
         `work_stealing` lets a cluster whose group has stopped take the next group from a device-side queue (default: on
-        whenever max_lens or sort_by_length is used)."""
+        whenever max_lens or sort_by_length is used).
+
+        Multi-speaker models: sids / spembs as in forward(); every utterance of a batch may have its own voice.  CPU inputs of such
+        a model run through the device pipeline (tts_infer_host takes no speakers)."""
         lib = self._ensure_handle()
-        self.sync_weights()
         B, S = phonemes.shape
+        spk = self._speaker_inputs(sids, spembs, B)
+        self.sync_weights()
         u0, ids = self._utt_ids(utt_ids, B, utt_offset)
         ragged = ids is not None or max_lens is not None or sort_by_length
         ws = self._workspace(B, S, max_len)
-        if not phonemes.is_cuda and not return_before and not ragged:
+        if not phonemes.is_cuda and not return_before and not ragged and spk is None:
             ph = phonemes.to(torch.int64).contiguous()
             pl = phoneme_lens.to(torch.int32).contiguous()
             key = (B, int(max_len))
@@ -503,9 +567,11 @@ class TransformerTTS(nn.Module):
             ph, pl, ids_d = ph[perm].contiguous(), pl[perm].contiguous(), ids_d[perm].contiguous()
             if mlens_d is not None:
                 mlens_d = mlens_d[perm].contiguous()
+            if spk is not None:
+                spk = tuple(None if t is None else t[perm].contiguous() for t in spk)
         stream = self._stream()
         # a ragged batch always has ids_d or mlens_d here; work stealing is on for it unless the caller says otherwise
-        self._start_decode(ws, ph, pl, int(max_len), seed, u0, ids_d, mlens_d, work_stealing is None or bool(work_stealing), stream)
+        self._start_decode(ws, ph, pl, int(max_len), seed, u0, ids_d, mlens_d, work_stealing is None or bool(work_stealing), spk, stream)
         td, nf = C.c_int(0), C.c_int(0)
         chunk = int(max_len)                               # one launch: every cluster stops itself on the device
         if self.profile_events:
@@ -536,7 +602,7 @@ class TransformerTTS(nn.Module):
 
     @torch.no_grad()
     def inference_stream(self, phonemes, phoneme_lens, max_len: int = 800, seed: int = 0, chunk_frames: int = 50, utt_ids=None,
-                         utt_offset: int = 0, max_lens=None):
+                         utt_offset: int = 0, max_lens=None, sids=None, spembs=None):
         """Greedy AR like inference(), yielding StreamChunk(start, mel_after, stop_logits, n_valid, finished) while the decoder keeps
         running.  The chunks cover consecutive frame ranges; concatenated along time they are exactly inference()'s mel_after and
         stop_logits, and their n_valid sum to its mel_lens.  CUDA inputs give CUDA chunks (ready when yielded), CPU inputs CPU chunks.
@@ -550,10 +616,12 @@ class TransformerTTS(nn.Module):
         The stream's decode session lives in the module's workspace until the generator is exhausted or closed.  Any other call
         on the module that runs in between (inference(), forward(), alignments(), encode(), another stream) takes that workspace
         over; the open generator then raises RuntimeError on its next step instead of yielding frames of the other call.  Serve
-        concurrent requests from one module by batching them, or give each open stream its own module."""
+        concurrent requests from one module by batching them, or give each open stream its own module.  sids / spembs of a
+        multi-speaker model as in inference()."""
         lib = self._ensure_handle()
-        self.sync_weights()
         B, S = phonemes.shape
+        spk = self._speaker_inputs(sids, spembs, B)
+        self.sync_weights()
         max_len = int(max_len)
         u0, ids = self._utt_ids(utt_ids, B, utt_offset)
         sched = StreamSchedule(chunk_frames, postnet_halo(self.cfg), max_len)
@@ -569,7 +637,7 @@ class TransformerTTS(nn.Module):
         side, cur = self._side_stream, torch.cuda.current_stream(dev)
         stream, side_ptr = self._stream(), C.c_void_p(side.cuda_stream)
         h, wsp = self._handle, ws.data_ptr()
-        self._start_decode(ws, ph, pl, max_len, seed, u0, ids_d, mlens_d, False, stream)
+        self._start_decode(ws, ph, pl, max_len, seed, u0, ids_d, mlens_d, False, spk, stream)
         nbytes = lib.tts_stream_scratch_bytes(h, B, sched.max_emit_frames())
         with torch.cuda.stream(side):
             scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev)
@@ -623,15 +691,18 @@ class TransformerTTS(nn.Module):
         return out[:n_steps, :n].clone()
 
     @torch.no_grad()
-    def encode(self, phonemes, phoneme_lens, T: Optional[int] = None) -> torch.Tensor:
-        """Encoder output ("memory") [B,S,512] fp32 on the GPU (bf16 values widened)."""
+    def encode(self, phonemes, phoneme_lens, T: Optional[int] = None, sids=None, spembs=None) -> torch.Tensor:
+        """Encoder output ("memory") [B,S,512] fp32 on the GPU (bf16 values widened); a multi-speaker model adds each utterance's
+        speaker vector (sids / spembs as in forward()) to all S rows."""
         lib = self._ensure_handle()
-        self.sync_weights()
         dev = self.device
         B, S = phonemes.shape
+        spk = self._speaker_inputs(sids, spembs, B)
+        self.sync_weights()
         T = int(T or S)
         ws = self._workspace(B, S, T)
         ph, pl = self._stage_inputs(phonemes, phoneme_lens)
+        self._stage_speakers(ws, spk, B, self._stream())
         mem = torch.empty(B, S, 512, device=dev)
         self._check(lib.tts_encode(self._handle, ws.data_ptr(), ph.data_ptr(), pl.data_ptr(), B, S, T, mem.data_ptr(), self._stream()), "tts_encode")
         return mem

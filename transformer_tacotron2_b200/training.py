@@ -85,11 +85,13 @@ class Trainer:
         dist.all_reduce(self._tick, op=dist.ReduceOp.SUM, group=self.group)
 
     # ------------------------------------------------------------------ one step
-    def _stage(self, phonemes, phoneme_lens, mels, mel_lens):
+    def _stage(self, phonemes, phoneme_lens, mels, mel_lens, sids=None, spembs=None):
         """Moves a batch to the device, into self._in (the library's asynchronous copies read from it), records its shape and
-        returns the workspace for that shape."""
+        returns the workspace for that shape.  A multi-speaker model's sids / spembs (as TransformerTTS.forward takes them) are
+        staged into the workspace with tts_train_set_conditioning; the next training call consumes them."""
         B, S = phonemes.shape
         T = mels.shape[1]
+        spk = self.model._speaker_inputs(sids, spembs, B)
         self._in = self.model._stage_inputs(phonemes, phoneme_lens, mels, mel_lens)
         if self._ws_key != (B, S, T):
             n = self._lib.tts_train_workspace_bytes(self._h, B, S, T)
@@ -97,12 +99,18 @@ class Trainer:
             self._ws = torch.empty(n, dtype=torch.uint8, device=self.model.device)
             self._ws_key = (B, S, T)
         self._shape = (B, S, T)
+        if spk is not None:
+            ptr = lambda t: None if t is None else t.data_ptr()                                           # noqa: E731
+            self.model._check(self._lib.tts_train_set_conditioning(self._h, self._ws.data_ptr(), B, ptr(spk[0]), ptr(spk[1]),
+                                                                   self.model._stream()), "tts_train_set_conditioning")
+        self._spk = spk
         return self._ws
 
-    def forward_backward(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_offset: int = 0) -> torch.Tensor:
+    def forward_backward(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_offset: int = 0, sids=None, spembs=None
+                         ) -> torch.Tensor:
         """Train-mode forward + loss + backward.  Returns the loss (1-element device tensor); gradients are in flat_grads."""
         m = self.model
-        ws = self._stage(phonemes, phoneme_lens, mels, mel_lens)
+        ws = self._stage(phonemes, phoneme_lens, mels, mel_lens, sids, spembs)
         (ph, pl, me, ml), (B, S, T) = self._in, self._shape
         rc = self._lib.tts_train_step(self._h, ws.data_ptr(), ph.data_ptr(), pl.data_ptr(), me.data_ptr(), ml.data_ptr(), B, S, T, int(seed),
                                       int(utt_offset), self.p_residual, self.pos_weight, self._loss.data_ptr(), m._stream())
@@ -110,10 +118,10 @@ class Trainer:
         return self._loss
 
     # ------------------------------------------------------------------ autograd bridge (model.train(); model(...); loss.backward())
-    def forward_only(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_offset: int = 0):
+    def forward_only(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_offset: int = 0, sids=None, spembs=None):
         """Train-mode forward alone; the activations stay in the workspace for backward_from().  -> (mel_before, mel_after, stop)."""
         m = self.model
-        ws = self._stage(phonemes, phoneme_lens, mels, mel_lens)
+        ws = self._stage(phonemes, phoneme_lens, mels, mel_lens, sids, spembs)
         (ph, pl, me, ml), (B, S, T) = self._in, self._shape
         rc = self._lib.tts_train_forward(self._h, ws.data_ptr(), ph.data_ptr(), pl.data_ptr(), me.data_ptr(), ml.data_ptr(), B, S, T, int(seed),
                                          int(utt_offset), self.p_residual, m._stream())
@@ -163,8 +171,8 @@ class Trainer:
         m._check(self._lib.tts_train_repack(self._h, m._stream()), "tts_train_repack")
         m._host_stale = True
 
-    def step(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_offset: int = 0) -> torch.Tensor:
-        loss = self.forward_backward(phonemes, phoneme_lens, mels, mel_lens, seed, utt_offset)
+    def step(self, phonemes, phoneme_lens, mels, mel_lens, seed: int = 0, utt_offset: int = 0, sids=None, spembs=None) -> torch.Tensor:
+        loss = self.forward_backward(phonemes, phoneme_lens, mels, mel_lens, seed, utt_offset, sids, spembs)
         if self._peers:
             self.adam_step_peers()
         else:
