@@ -259,12 +259,42 @@ int tts_k_gemm(const void* A_bf16, const void* W_bf16, const float* bias, float*
 /* conv1d(k=5, pad=2) over [B][T][Cin] with W [5][Cout][Cin] bf16 -> fp32 [B][T][Cout]; rows t >= lens[b] zeroed. */
 int tts_k_conv5(const void* X_bf16, const void* W_bf16, const float* bias, const int32_t* lens, float* Y,
                 int B, int T, int Cin, int Cout, int act, void* stream);
+/* The sequence GEMM / conv with every epilogue field exposed, validated and launched through the library's own launcher
+ * (gemm_tc.cuh, epilogue gemm_epilogue.cuh).  C[m][n] = epi(sum_tap sum_k A[b*T + t + tap - taps/2][k] W[tap][n][k]) for
+ * m = b*T + t, rows outside [0, T) of the utterance read as zero; W has taps * round_up(N, 128) rows of ldw bf16.  epi, in
+ * this order: + bias[n]; + alpha * pe[t][n] (pe row stride 512, alpha read from alpha_ptr if set); word dropout (dropw_site
+ * >= 0: keep iff Philox word >= dropw_thresh, kept values * dropw_scale); + resid_bf16 / resid_f32 [m][ldr]; act (0 none,
+ * 1 relu, 2 tanh); p = 0.5 bit dropout (drop_site >= 0, seed or *seed_ptr, utterance id utt_offset + b); zero rows t >=
+ * lens[b].  Output: out_f32 / out_bf16 [m][ldo] (scatter 0), the cross-K/V caches (scatter 1: out_bf16 [N/1024][2][B][8]
+ * [Lpad][64], Lpad a multiple of 16; scatter 3: the decode kernel's 64-row blocks, Lpad a multiple of 64; both N % 1024 == 0
+ * and B * T == M), or the heads (scatter 2: N = 81, out_f32 [M][80] mel, out2_f32 [M] stop logit).  max_ctas caps the
+ * persistent grid (0 = one CTA per SM).  TTS_E_ARG for any layout the kernel cannot handle.  struct_size = sizeof. */
+typedef struct TtsKGemm {
+    uint32_t struct_size;
+    const void* A; int32_t lda;
+    const void* W; int32_t ldw;
+    int32_t M, N, K, taps, T;
+    const float* bias; int32_t act;
+    const void* resid_bf16; const float* resid_f32; int32_t ldr;
+    const float* pe; float alpha; const float* alpha_ptr;
+    const int32_t* lens;
+    int32_t drop_site; uint64_t seed; const uint64_t* seed_ptr; int32_t utt_offset;
+    int32_t dropw_site; uint32_t dropw_thresh; float dropw_scale;
+    float* out_f32; void* out_bf16; int32_t ldo;
+    int32_t scatter; float* out2_f32; int32_t B; int32_t Lpad; int32_t max_ctas;
+} TtsKGemm;
+int tts_k_gemm_epi(const TtsKGemm* args, void* stream);
 /* Attention core: Q [B][Lq][H*64], K/V [B][Lk][H*64] bf16 -> O [B][Lq][H*64] bf16. */
 int tts_k_attention(const void* Q, const void* K, const void* V, void* O, const int32_t* klens,
                     int B, int H, int Lq, int Lk, int causal, void* stream);
 /* Attention core with the per-row log-sum-exp kept for the backward pass: lse [B][H][Lq] fp32 (log2 domain). */
 int tts_k_attention_lse(const void* Q, const void* K, const void* V, void* O, float* lse, const int32_t* klens,
                         int B, int H, int Lq, int Lk, int causal, void* stream);
+/* Attention core with explicit element strides, as the library calls it on packed QKV rows and on the cross-K/V cache:
+ * strides = {q_bs, q_hs, q_rs, k_bs, k_hs, k_rs, v_bs, v_hs, v_rs, o_bs, o_hs, o_rs} (batch, head, row; multiples of 8),
+ * bases 16-byte aligned; lse [B][H][Lq] may be NULL.  Head h of row r reads the 64 elements at base + b bs + h hs + r rs. */
+int tts_k_attention_strided(const void* Q, const void* K, const void* V, void* O, float* lse, const int32_t* klens,
+                            const int64_t* strides, int B, int H, int Lq, int Lk, int causal, void* stream);
 /* Attention backward (training path): Q/K/V/O/dO as above + lse -> dQ/dK/dV bf16 in the same layouts.
  * scratch: fp32 [B*Lq*H*64 + B*H*Lq] device buffer. */
 int tts_k_attention_bwd(const void* Q, const void* K, const void* V, const void* O, const void* dO, const float* lse,

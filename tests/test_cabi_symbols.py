@@ -190,3 +190,41 @@ def test_decode_weight_stream_matches_kernel_addressing():
     W = rng.standard_normal((256, 80)).astype(np.float32)
     stream = _pack(lib, W, np.arange(32), 0, 4, 1)
     assert not _read_fragment_block(stream, 2 * 1024, 0, 1)[:2].any()                     # k = 2 * 32 + 16 = 80: padding
+
+
+def test_sequence_test_entry_points_validate_on_the_host():
+    """tts_k_gemm_epi and tts_k_attention_strided refuse layouts their kernels cannot handle before any device work (the
+    addresses below are never dereferenced)."""
+    import pytest
+    import torch
+    if torch.cuda.is_available():
+        pytest.skip("GPU present: tests/test_gpu_seq_kernels.py checks the same with real buffers")
+    from transformer_tacotron2_b200 import _lib
+    lib = _lib.load()
+    fake = 1 << 20
+
+    def gemm(**kw):
+        a = _lib.TtsKGemm()
+        a.struct_size = C.sizeof(_lib.TtsKGemm)
+        base = dict(A=fake, lda=512, W=fake, ldw=512, M=74, N=6144, K=512, taps=1, T=37, bias=fake, drop_site=-1, dropw_site=-1,
+                    scatter=1, out_bf16=fake, B=2, Lpad=48)
+        for k, v in dict(base, **kw).items():
+            setattr(a, k, v)
+        return lib.tts_k_gemm_epi(C.byref(a), None)
+    assert gemm(struct_size=8) == -1
+    assert gemm(Lpad=40) == -1                          # row-major cache: Lpad a multiple of 16
+    assert gemm(Lpad=32) == -1                          # Lpad < T
+    assert gemm(N=5632) == -1                           # cross K/V: N a multiple of 1024
+    assert gemm(scatter=3) == -1                        # blocked cache: Lpad a multiple of 64
+    assert gemm(B=3) == -1                              # B * T != M
+    assert gemm(T=36) == -1                             # M % T
+    assert gemm(scatter=2, N=80, out_f32=fake, out2_f32=fake) == -1      # heads: N = 81
+    assert gemm(scatter=0, N=512, ldo=500) == -1        # ldo < N
+    assert gemm(scatter=0, N=1024, ldo=1024, pe=fake) == -1              # pe rows are 512 wide
+    assert gemm(bias=fake + 2) == -1                    # not even element-aligned
+    assert gemm(lda=500) == -1                          # TMA row stride: a multiple of 8 elements
+    assert gemm(taps=3) == -1
+    st = (C.c_int64 * 12)(*([64 * 1536, 64, 1536] * 3 + [64 * 512, 64, 516]))
+    assert lib.tts_k_attention_strided(fake, fake, fake, fake, None, None, st, 2, 8, 64, 64, 0, None) == -1
+    st = (C.c_int64 * 12)(*([64 * 1536, 64, 1536] * 3 + [64 * 512, 64, 512]))
+    assert lib.tts_k_attention_strided(fake + 2, fake, fake, fake, None, None, st, 2, 8, 64, 64, 0, None) == -1

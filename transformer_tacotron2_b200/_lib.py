@@ -18,6 +18,22 @@ class TtsConfig(C.Structure):
         ("ln_eps", C.c_float), ("bn_eps", C.c_float), ("n_speakers", C.c_int32), ("spk_embed_dim", C.c_int32)]
 
 
+class TtsKGemm(C.Structure):
+    """include/tts_b200.h TtsKGemm: every field of the sequence GEMM's launch (tts_k_gemm_epi)."""
+    _fields_ = [
+        ("struct_size", C.c_uint32),
+        ("A", C.c_void_p), ("lda", C.c_int32), ("W", C.c_void_p), ("ldw", C.c_int32),
+        ("M", C.c_int32), ("N", C.c_int32), ("K", C.c_int32), ("taps", C.c_int32), ("T", C.c_int32),
+        ("bias", C.c_void_p), ("act", C.c_int32),
+        ("resid_bf16", C.c_void_p), ("resid_f32", C.c_void_p), ("ldr", C.c_int32),
+        ("pe", C.c_void_p), ("alpha", C.c_float), ("alpha_ptr", C.c_void_p),
+        ("lens", C.c_void_p),
+        ("drop_site", C.c_int32), ("seed", C.c_uint64), ("seed_ptr", C.c_void_p), ("utt_offset", C.c_int32),
+        ("dropw_site", C.c_int32), ("dropw_thresh", C.c_uint32), ("dropw_scale", C.c_float),
+        ("out_f32", C.c_void_p), ("out_bf16", C.c_void_p), ("ldo", C.c_int32),
+        ("scatter", C.c_int32), ("out2_f32", C.c_void_p), ("B", C.c_int32), ("Lpad", C.c_int32), ("max_ctas", C.c_int32)]
+
+
 _P, _I, _I64, _U64, _SZ = C.c_void_p, C.c_int, C.c_int64, C.c_uint64, C.c_size_t
 
 # name -> (restype, argtypes); every symbol include/tts_b200.h declares
@@ -70,6 +86,8 @@ SIGNATURES = {
     "tts_train_backward": (_I, [_P, _P, _I, _I, _I, _I, C.c_double, _P, _P, _P, _P]),
     "tts_k_gemm": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "tts_k_conv5": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
+    "tts_k_gemm_epi": (_I, [C.POINTER(TtsKGemm), _P]),
+    "tts_k_attention_strided": (_I, [_P] * 7 + [_I, _I, _I, _I, _I, _P]),
     "tts_k_attention": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "tts_k_attention_lse": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "tts_k_attention_bwd": (_I, [_P] * 11 + [_I, _I, _I, _I, _I, _P]),

@@ -3,7 +3,9 @@
 // epi order: + bias, + alpha * pe, word dropout, + residual, activation, bit dropout, length mask
 // used by the encoder, the cross-K/V projection, the teacher-forced decoder and the postnet
 // (SURVEY.md 8(a) rows a3, a4, a10).  gemm_store is the scalar (pair-wise) form of the epilogue; the kernel uses
-// a 16-byte vectorised form of the same arithmetic where the output is a plain matrix.
+// a 16-byte vectorised form of the same arithmetic where the output is a plain matrix with 16-byte aligned rows.  The two
+// forms give bit-identical results (tests/test_gpu_seq_kernels.py); the scalar form handles any layout, so it also takes the
+// scatters, the columns past the last full 32-column chunk and every misaligned operand.
 #pragma once
 #include "common.cuh"
 #include "philox.cuh"
@@ -44,18 +46,19 @@ TTS_D void gemm_store(const GemmParams& p, int m, int n, float v0, float v1) {
     const bool has1 = (n + 1) < p.N;
     const int b = m / p.T, t = m - b * p.T;
     const uint64_t seed = p.seed_ptr ? *p.seed_ptr : p.seed;
-    if (p.bias) { v0 += p.bias[n]; if (has1) v1 += p.bias[n + 1]; }
-    if (p.pe) {
+    // + 0 without a bias, as the vector form adds (a -0 accumulator leaves both forms as +0)
+    v0 += p.bias ? p.bias[n] : 0.f; v1 += p.bias && has1 ? p.bias[n + 1] : 0.f;
+    if (p.pe) {                                      // explicit FMA / multiply below: both forms round alike whatever nvcc contracts
         const float alpha = p.alpha_ptr ? *p.alpha_ptr : p.alpha;
-        v0 += alpha * p.pe[(size_t)t * kDModel + n];
-        if (has1) v1 += alpha * p.pe[(size_t)t * kDModel + n + 1];
+        v0 = __fmaf_rn(alpha, p.pe[(size_t)t * kDModel + n], v0);
+        if (has1) v1 = __fmaf_rn(alpha, p.pe[(size_t)t * kDModel + n + 1], v1);
     }
     if (p.dropw_site >= 0) {                         // n even: words n % 4 and n % 4 + 1 of chunk n / 4
         const uint4 w = philox4x32_10(make_uint4((uint32_t)p.dropw_site, (uint32_t)t, (uint32_t)(p.utt_offset + b), (uint32_t)(n >> 2)),
                                       (uint32_t)seed, (uint32_t)(seed >> 32));
         const uint32_t w0 = (n & 2) ? w.z : w.x, w1 = (n & 2) ? w.w : w.y;
-        v0 = w0 >= p.dropw_thresh ? v0 * p.dropw_scale : 0.f;
-        v1 = w1 >= p.dropw_thresh ? v1 * p.dropw_scale : 0.f;
+        v0 = w0 >= p.dropw_thresh ? __fmul_rn(v0, p.dropw_scale) : 0.f;
+        v1 = w1 >= p.dropw_thresh ? __fmul_rn(v1, p.dropw_scale) : 0.f;
     }
     if (p.resid_bf16) {
         v0 += __bfloat162float(p.resid_bf16[(size_t)m * p.ldr + n]);
@@ -102,10 +105,11 @@ TTS_D void gemm_store(const GemmParams& p, int m, int n, float v0, float v1) {
         if (has1) p.out_f32[(size_t)m * p.ldo + n + 1] = v1;
     }
     if (p.out_bf16) {
-        if (has1 && ((p.ldo & 1) == 0)) *reinterpret_cast<uint32_t*>(p.out_bf16 + (size_t)m * p.ldo + n) = pack_bf16x2(v0, v1);
+        bf16* o = p.out_bf16 + (size_t)m * p.ldo + n;
+        if (has1 && (reinterpret_cast<uintptr_t>(o) & 3) == 0) *reinterpret_cast<uint32_t*>(o) = pack_bf16x2(v0, v1);
         else {
-            p.out_bf16[(size_t)m * p.ldo + n] = __float2bfloat16(v0);
-            if (has1) p.out_bf16[(size_t)m * p.ldo + n + 1] = __float2bfloat16(v1);
+            o[0] = __float2bfloat16(v0);
+            if (has1) o[1] = __float2bfloat16(v1);
         }
     }
 }

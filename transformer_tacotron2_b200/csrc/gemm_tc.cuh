@@ -29,6 +29,7 @@ struct GemmTcParams {
     alignas(64) CUtensorMap tm_w;     // bf16 {K (inner), taps * Nw}, box {64, 128}, SWIZZLE_128B
     alignas(64) CUtensorMap tm_out;   // output {N (inner), T, B}: fp32 box {32, 32, 1} / bf16 box {64, 32, 1}, SWIZZLE_128B (TMA store)
     int tma_out;                      // 0 = direct stores, 1 = fp32 via TMA store, 2 = bf16 via TMA store
+    int vec_ok;                       // the 16-byte vector form may run: ldo, ldr multiples of 8 and every operand base 16-byte aligned
     GemmParams g;                     // shapes + epilogue (A / W pointers unused here)
     int Tl;                           // rows per A-tensor slab: T for convs (taps > 1), M for plain GEMMs
     int tiles_per_utt;                // ceil(Tl / 128)
@@ -152,8 +153,11 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gemm_tc_kernel(const __grid_con
         if (g.bias) {
             const int bc = n0 + chalf * (TC_BN / 2) + lane * 4;
             if (lane * 4 >= TC_BN / 2) { /* this lane's columns belong to the other warp */ }
-            else if (bc + 3 < g.N) bq = __ldg(reinterpret_cast<const float4*>(g.bias + bc));
-            else { if (bc < g.N) bq.x = g.bias[bc]; if (bc + 1 < g.N) bq.y = g.bias[bc + 1]; if (bc + 2 < g.N) bq.z = g.bias[bc + 2]; }
+            else if (bc + 3 < g.N && (reinterpret_cast<uintptr_t>(g.bias) & 15) == 0) bq = __ldg(reinterpret_cast<const float4*>(g.bias + bc));
+            else {
+                if (bc < g.N) bq.x = g.bias[bc]; if (bc + 1 < g.N) bq.y = g.bias[bc + 1];
+                if (bc + 2 < g.N) bq.z = g.bias[bc + 2]; if (bc + 3 < g.N) bq.w = g.bias[bc + 3];
+            }
         }
         tc_mbar_wait(&tmem_full[acc], (j >> 1) & 1);
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -174,7 +178,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gemm_tc_kernel(const __grid_con
             {
                 const int nb0 = n0 + c0;
                 const bool rvalid = t < p.Tl && m < g.M;
-                const bool vec = g.scatter == SC_NONE && nb0 + 32 <= g.N && (g.ldo & 7) == 0 && (g.ldr & 7) == 0;      // warp-uniform
+                const bool vec = g.scatter == SC_NONE && nb0 + 32 <= g.N && p.vec_ok;      // warp-uniform
                 if (!vec) {
                     if (rvalid) {
 #pragma unroll
@@ -201,7 +205,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gemm_tc_kernel(const __grid_con
 #pragma unroll
                             for (int j = 0; j < 32; j += 4) {
                                 const float4 pv = __ldg(reinterpret_cast<const float4*>(g.pe + (size_t)tt * kDModel + nb0 + j));
-                                f[j] += alpha * pv.x; f[j + 1] += alpha * pv.y; f[j + 2] += alpha * pv.z; f[j + 3] += alpha * pv.w;
+                                f[j] = __fmaf_rn(alpha, pv.x, f[j]); f[j + 1] = __fmaf_rn(alpha, pv.y, f[j + 1]); f[j + 2] = __fmaf_rn(alpha, pv.z, f[j + 2]); f[j + 3] = __fmaf_rn(alpha, pv.w, f[j + 3]);
                             }
                         }
                         if (g.dropw_site >= 0) {             // word dropout (P12): 4 consecutive columns = one Philox call
@@ -209,10 +213,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gemm_tc_kernel(const __grid_con
                             for (int j = 0; j < 32; j += 4) {
                                 const uint4 w4 = philox4x32_10(make_uint4((uint32_t)g.dropw_site, (uint32_t)tt, (uint32_t)(g.utt_offset + bb), (uint32_t)((nb0 + j) >> 2)),
                                                                (uint32_t)seed, (uint32_t)(seed >> 32));
-                                f[j] = w4.x >= g.dropw_thresh ? f[j] * g.dropw_scale : 0.f;
-                                f[j + 1] = w4.y >= g.dropw_thresh ? f[j + 1] * g.dropw_scale : 0.f;
-                                f[j + 2] = w4.z >= g.dropw_thresh ? f[j + 2] * g.dropw_scale : 0.f;
-                                f[j + 3] = w4.w >= g.dropw_thresh ? f[j + 3] * g.dropw_scale : 0.f;
+                                f[j] = w4.x >= g.dropw_thresh ? __fmul_rn(f[j], g.dropw_scale) : 0.f;
+                                f[j + 1] = w4.y >= g.dropw_thresh ? __fmul_rn(f[j + 1], g.dropw_scale) : 0.f;
+                                f[j + 2] = w4.z >= g.dropw_thresh ? __fmul_rn(f[j + 2], g.dropw_scale) : 0.f;
+                                f[j + 3] = w4.w >= g.dropw_thresh ? __fmul_rn(f[j + 3], g.dropw_scale) : 0.f;
                             }
                         }
                         if (g.resid_bf16) {
@@ -365,12 +369,17 @@ inline cudaError_t launch_gemm_tc(const GemmParams& g, cudaStream_t stream) {
                 CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
             return cudaErrorInvalidValue;
     }
+    // the vector form stores 16 bytes to out_* and loads 16 bytes from resid_* / pe at every 8th column: a view offset by a
+    // few bytes (a caller's output slice, say) takes the scalar form instead, which makes no alignment assumption
+    const auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
+    p.vec_ok = (g.ldo & 7) == 0 && (g.ldr & 7) == 0 && al16(g.out_f32) && al16(g.out_bf16) && al16(g.resid_bf16) && al16(g.resid_f32) &&
+               al16(g.pe);
     p.tma_out = 0;
     if (g.scatter == SC_NONE && (g.out_f32 != nullptr) != (g.out_bf16 != nullptr)) {
         const bool f32 = g.out_f32 != nullptr;
         const size_t es = f32 ? 4 : 2;
         void* base = f32 ? (void*)g.out_f32 : (void*)g.out_bf16;
-        if (((size_t)g.ldo * es) % 16 == 0 && (reinterpret_cast<uintptr_t>(base) & 15) == 0 && (g.ldo & 7) == 0 && (g.ldr & 7) == 0) {
+        if (p.vec_ok) {                                  // the TMA store is part of the vector form (ldo * es is a multiple of 16)
             const cuuint64_t dims[3] = {(cuuint64_t)g.N, (cuuint64_t)p.Tl, (cuuint64_t)nb};
             const cuuint64_t strides[2] = {(cuuint64_t)g.ldo * es, (cuuint64_t)g.ldo * es * p.Tl};
             const cuuint32_t box[3] = {f32 ? 32u : 64u, 32, 1};

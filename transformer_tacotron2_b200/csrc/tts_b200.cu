@@ -1086,6 +1086,55 @@ extern "C" int tts_k_conv5(const void* X, const void* W, const float* bias, cons
     p.taps = 5; p.T = T; p.bias = bias; p.act = act; p.lens = lens; p.out_f32 = Y; p.ldo = Cout;
     return (int)launch_gemm_tc(p, (cudaStream_t)stream);
 }
+extern "C" int tts_k_gemm_epi(const TtsKGemm* a, void* stream) {
+    if (!a || a->struct_size != sizeof(TtsKGemm)) return TTS_E_ARG;
+    const auto al = [](const void* q, uintptr_t n) { return (reinterpret_cast<uintptr_t>(q) & (n - 1)) == 0; };
+    if (!a->A || !a->W || a->M <= 0 || a->N <= 0 || a->K <= 0 || a->T <= 0 || (a->M % a->T) || (a->K % 8) || (a->taps != 1 && a->taps != 5) ||
+        a->lda < a->K || a->ldw < a->K || (a->lda % 8) || (a->ldw % 8) || !al(a->A, 16) || !al(a->W, 16) || a->act < 0 || a->act > 2 ||
+        a->max_ctas < 0 || a->scatter < SC_NONE || a->scatter > SC_CROSS_KV_VT)
+        return TTS_E_ARG;
+    // operands the kernel reads or writes element-wise must at least be aligned to their element
+    if (!al(a->bias, 4) || !al(a->resid_bf16, 2) || !al(a->resid_f32, 4) || !al(a->pe, 4) || !al(a->alpha_ptr, 4) || !al(a->lens, 4) ||
+        !al(a->seed_ptr, 8) || !al(a->out_f32, 4) || !al(a->out_bf16, 2) || !al(a->out2_f32, 4))
+        return TTS_E_ARG;
+    if ((a->resid_bf16 || a->resid_f32) && a->ldr < a->N) return TTS_E_ARG;
+    if (a->pe && a->N > kDModel) return TTS_E_ARG;
+    if (a->scatter == SC_NONE && (!(a->out_f32 || a->out_bf16) || a->ldo < a->N)) return TTS_E_ARG;
+    if (a->scatter == SC_CROSS_KV || a->scatter == SC_CROSS_KV_VT) {
+        const int q = a->scatter == SC_CROSS_KV ? 16 : KV_BLOCK_ROWS;
+        if (!a->out_bf16 || !al(a->out_bf16, 16) || (a->N % 1024) || a->B <= 0 || a->B * a->T != a->M || a->Lpad < a->T || (a->Lpad % q))
+            return TTS_E_ARG;
+    }
+    if (a->scatter == SC_HEAD && (a->N != 81 || !a->out_f32 || !a->out2_f32)) return TTS_E_ARG;
+    GemmParams p = gp((const bf16*)a->A, a->lda, (const bf16*)a->W, a->ldw, a->M, a->N, a->K);
+    p.taps = a->taps; p.T = a->T;
+    p.bias = a->bias; p.act = a->act;
+    p.resid_bf16 = (const bf16*)a->resid_bf16; p.resid_f32 = a->resid_f32; p.ldr = a->ldr;
+    p.pe = a->pe; p.alpha = a->alpha; p.alpha_ptr = a->alpha_ptr;
+    p.lens = a->lens;
+    p.drop_site = a->drop_site; p.seed = a->seed; p.seed_ptr = a->seed_ptr; p.utt_offset = a->utt_offset;
+    p.dropw_site = a->dropw_site; p.dropw_thresh = a->dropw_thresh; p.dropw_scale = a->dropw_scale;
+    p.out_f32 = a->out_f32; p.out_bf16 = (bf16*)a->out_bf16; p.ldo = a->ldo;
+    p.scatter = a->scatter; p.out2_f32 = a->out2_f32; p.B = a->scatter == SC_NONE || a->scatter == SC_HEAD ? 1 : a->B; p.Lpad = a->Lpad;
+    p.max_ctas = a->max_ctas;
+    return (int)launch_gemm_tc(p, (cudaStream_t)stream);
+}
+extern "C" int tts_k_attention_strided(const void* Q, const void* K, const void* V, void* O, float* lse, const int32_t* klens,
+                                       const int64_t* s, int B, int H, int Lq, int Lk, int causal, void* stream) {
+    if (!Q || !K || !V || !O || !s || B <= 0 || H <= 0 || Lq <= 0 || Lk <= 0) return TTS_E_ARG;
+    for (int i = 0; i < 12; ++i)
+        if (s[i] < 0 || (s[i] % 8)) return TTS_E_ARG;
+    for (const void* q : {Q, K, V, (const void*)O})
+        if (reinterpret_cast<uintptr_t>(q) & 15) return TTS_E_ARG;
+    if (reinterpret_cast<uintptr_t>(lse) & 3) return TTS_E_ARG;
+    AttnParams a; memset(&a, 0, sizeof(a));
+    a.Q = (const bf16*)Q; a.K = (const bf16*)K; a.V = (const bf16*)V; a.O = (bf16*)O;
+    a.q_bs = s[0]; a.q_hs = s[1]; a.q_rs = s[2]; a.k_bs = s[3]; a.k_hs = s[4]; a.k_rs = s[5];
+    a.v_bs = s[6]; a.v_hs = s[7]; a.v_rs = s[8]; a.o_bs = s[9]; a.o_hs = s[10]; a.o_rs = s[11];
+    a.B = B; a.H = H; a.Lq = Lq; a.Lk = Lk; a.klens = klens; a.causal = causal; a.lse = lse;
+    a.scale_log2 = 0.125f * kLog2e;
+    return (int)launch_flash_attn_tc(a, (cudaStream_t)stream);
+}
 extern "C" int tts_k_attention(const void* Q, const void* K, const void* V, void* O, const int32_t* klens, int B, int H, int Lq,
                                int Lk, int causal, void* stream) {
     if (!Q || !K || !V || !O || B <= 0 || H <= 0 || Lq <= 0 || Lk <= 0) return TTS_E_ARG;
